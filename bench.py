@@ -8,7 +8,8 @@ equivalent on 1 B200"; 8 GPUs x 512 = the 4096 scenarios of configs[4]).  Scenar
 that every (scenario, step, vehicle) search record is fixed; one bench "step" =
 one pass of the hot path over all records of the rank.  Both arms plan the SAME
 records: they come from the same seeds, are rolled out by bit-identical planners
-(GPU library / C oracle) and are shared through a cache under build/.
+(GPU library / C oracle) and are shared through a per-user cache in the temporary
+directory (never in the source tree, which may be read-only).
 
   value     : records already resident in HBM, search kernel timed with CUDA
               events on the library's stream, L2 flushed between steps.
@@ -28,6 +29,10 @@ records: they come from the same seeds, are rolled out by bit-identical planners
 over the ranks (strong scaling).  `--optimizer sampled` times the sampled optimizer
 (MonteCarloTreeSearch) on the same records.  `--config explorative` runs BASELINE
 configs[2] (8 priority permutations per time step, sharded over the GPUs) closed loop.
+`--dump-outputs DIR` writes what the timed search returned in its last step as DIR/<field>.npy
+(float64; a fixed sample of searches when all of them exceed 60 MB; with several GPUs DIR/rank<r>/
+per rank, 60 MB over all ranks), so that two builds can be compared output for output on the same
+records.
 """
 from __future__ import annotations
 
@@ -36,6 +41,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -47,6 +53,30 @@ import numpy as np  # noqa: E402
 BLOCK = 8            # scenarios per record-cache file (the unit of generation and of sharding)
 LAT_SCENARIOS = 8    # scenarios whose time steps are replayed for the per-time-step latency (= block 0)
 L2_NOTE = "GPU arm: flushed between timed steps (256 MiB write); CPU arm: not applicable"
+DUMP_LIMIT = 60_000_000   # array bytes --dump-outputs writes over all ranks: under 64 MB with the .npy headers
+
+
+def records_version() -> str:
+    """Digest of what the rolled-out records depend on: the scenario generator, the record layout, both rollout
+    planners (CUDA library, C oracle), the map and this file's rollout.  The cache is keyed on it, so a cached block
+    is only read by the version of the project that wrote it."""
+    import glob
+    import hashlib
+    files = [os.path.join(ROOT, "bench.py")]
+    for pat in ("p-dmpc_b200/*.py", "p-dmpc_b200/data/*", "p-dmpc_b200/csrc/*.cu", "p-dmpc_b200/csrc/*.cuh",
+                "p-dmpc_b200/csrc/*.h", "include/*.h", "oracle/pdmpc_oracle.[ch]"):
+        files += sorted(glob.glob(os.path.join(ROOT, pat)))
+    h = hashlib.sha256()
+    for f in files:
+        h.update(os.path.relpath(f, ROOT).encode())
+        with open(f, "rb") as fh:
+            h.update(fh.read())
+    return h.hexdigest()[:16]
+
+
+# per user (the owner is checked before use) and per version, outside the source tree, which may be read-only
+RECORD_CACHE_ROOT = os.path.join(tempfile.gettempdir(), f"pdmpc_bench_records_{os.getuid()}")
+RECORD_CACHE = os.path.join(RECORD_CACHE_ROOT, records_version())
 
 
 def parse_args():
@@ -68,13 +98,17 @@ def parse_args():
     ap.add_argument("--sim-steps", type=int, default=35)
     ap.add_argument("--vehicles", type=int, default=20)
     ap.add_argument("--mpa", default="triple_speed")
-    ap.add_argument("--no-cache", action="store_true", help="do not read/write the record cache under build/")
+    ap.add_argument("--no-cache", action="store_true", help=f"do not read/write the record cache ({RECORD_CACHE})")
     ap.add_argument("--cpu-sample", type=int, default=0, help="searches in the CPU sample (0 = auto)")
     ap.add_argument("--pipeline-chunks", type=int, default=0,
                     help="chunks of the e2e call's copy/search pipeline (0 = library default, 1 = off)")
     ap.add_argument("--permutations", type=int, default=8, help="--config explorative: priority permutations per time step")
     ap.add_argument("--mcts-expansions", type=int, default=250, help="--optimizer sampled: n_expansions_max")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<field>.npy (float64, under 64 MB)")
     a = ap.parse_args()
+    if a.dump_outputs and (a.impl != "ours" or a.config != "road"):
+        ap.error("--dump-outputs covers the timed search of the GPU arm (--impl ours, --config road)")
     for v in (a.scenarios, a.scenarios_total):
         if v % BLOCK:
             ap.error(f"scenario counts must be multiples of {BLOCK}")
@@ -142,8 +176,7 @@ class ClockSampler:
 
 # ---------------------------------------------------------------------------- records
 def block_path(args, block: int) -> str:
-    return os.path.join(ROOT, "build", "bench_records",
-                        f"{args.mpa}_{args.vehicles}v_{args.sim_steps}t_block{block:04d}.npz")
+    return os.path.join(RECORD_CACHE, f"{args.mpa}_{args.vehicles}v_{args.sim_steps}t_block{block:04d}.npz")
 
 
 def _roll_block(job):
@@ -205,11 +238,15 @@ def rank_blocks(args, rank: int, world: int):
 
 def get_records(args, blocks, kind: str, dev: int, workers: int):
     """Flat batch of every search record of `blocks` (+ level structure and one-call inputs of block 0 when
-    it is among them).  Missing blocks are rolled out by `workers` processes and cached under build/."""
+    it is among them).  Missing blocks are rolled out by `workers` processes and cached in RECORD_CACHE."""
     import pickle
     import multiprocessing as mp
     from pdmpc_b200.records import SearchBatch
-    import tempfile
+    if not args.no_cache:
+        os.makedirs(RECORD_CACHE_ROOT, mode=0o700, exist_ok=True)
+        if os.stat(RECORD_CACHE_ROOT).st_uid != os.getuid():   # the cache holds pickles: read only our own
+            raise SystemExit(f"{RECORD_CACHE_ROOT} belongs to another user; run with --no-cache")
+        os.makedirs(RECORD_CACHE, mode=0o700, exist_ok=True)
     tmpdir = tempfile.mkdtemp(prefix="pdmpc_gen_") if args.no_cache else None
     path = (lambda b: os.path.join(tmpdir, f"block{b:04d}.npz")) if tmpdir else (lambda b: block_path(args, b))
     todo = [b for b in blocks if not os.path.exists(path(b)) or
@@ -232,6 +269,39 @@ def get_records(args, blocks, kind: str, dev: int, workers: int):
         import shutil
         shutil.rmtree(tmpdir, ignore_errors=True)
     return batch, levels, timesteps
+
+
+def dump_outputs(res, out_dir: str, limit: int) -> None:
+    """The BatchResult of the timed path (what pdmpc_fetch_staged hands a caller), one DIR/<field>.npy per field, in
+    float64: every integer field is exact in it, the 64-bit pop-order hash is split into two 32-bit halves.  When all
+    searches do not fit in `limit` bytes, a fixed sample of them (seed 0, ascending; DIR/rows.npy lists it) is written.
+    An exhausted search has no plan: its poses and costs are NaN and are written as 0 (is_exhausted marks those rows).
+    Any other value that is not finite is a wrong result and raises."""
+    import dataclasses
+    exhausted = res.is_exhausted.astype(bool)
+    fields = {}
+    for f in dataclasses.fields(res):
+        a = getattr(res, f.name)
+        if not isinstance(a, np.ndarray):
+            continue
+        if a.dtype == np.uint64:
+            fields[f.name + "_hi"] = (a >> np.uint64(32)).astype(np.float64)
+            fields[f.name + "_lo"] = (a & np.uint64(0xFFFFFFFF)).astype(np.float64)
+        else:
+            a = a.astype(np.float64)          # a copy: the caller's result stays as the library returned it
+            a[exhausted] = np.nan_to_num(a[exhausted], nan=0.0, posinf=np.inf, neginf=-np.inf)
+            if not np.isfinite(a).all():
+                bad = np.argwhere(~np.isfinite(a))[0]
+                raise RuntimeError(f"--dump-outputs: {f.name} is not finite at {tuple(bad)}")
+            fields[f.name] = a
+    n = res.status.size
+    row_bytes = 8 * (1 + sum(a[:1].size for a in fields.values()))    # + the row index itself
+    m = min(n, limit // row_bytes)
+    rows = np.arange(n) if m == n else np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
+    for name, a in fields.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a[rows])
 
 
 def workload_config(args, world: int, n: int, Hp: int) -> dict:
@@ -472,6 +542,10 @@ def main():
     barrier()
     clocks = sampler.stop()
     res = planner.fetch()
+    if args.dump_outputs:
+        # each rank holds its own records: with several GPUs, DIR/rank<r>/ per rank, the byte budget split evenly
+        dump_outputs(res, args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}"),
+                     DUMP_LIMIT // world)
     stats = planner.stats()
     shape = int(stats.shape)
     ms_step = float(np.mean(kernel_ms))
@@ -668,7 +742,7 @@ def main():
                                            "(profiles/search_kernel_traffic.json), 4 issue slots/clk/SM"}
         line = {
             "metric": "vehicle-plans/sec", "value": value, "unit": "plans/s", "n_gpus": world,
-            "steps": args.steps, "warmup": max(args.warmup, 3), "ms_per_step": total_ms / args.steps,
+            "steps": len(kernel_ms), "warmup": max(args.warmup, 3), "ms_per_step": total_ms / len(kernel_ms),
             "higher_is_better": True, "scaling": "strong" if args.scenarios_total else "weak",
             "vs_baseline": None, "dtype": "f64", "data": "synthetic",
             "config": workload_config(args, world, n, Hp),

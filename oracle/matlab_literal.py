@@ -157,24 +157,12 @@ class Info:
     tree: Optional[Tree] = None
 
 
-class _HeapqLikeStd:
-    """Fallback when oracle/_ref is absent: the oracle's restated libstdc++ heap."""
-
-    def __init__(self):
-        self.q = oracle_py.OraclePQ()
-
-    def push(self, ids, vals):
-        for i, v in zip(np.atleast_1d(ids), np.atleast_1d(vals)):
-            self.q.push(int(i), float(v))
-
-    def pop(self):
-        return self.q.pop()
-
-
 def _new_pq(use_reference_pq: bool):
+    """The reference's own queue source, or (where it is not built) its restatement on libstdc++'s
+    std::priority_queue (StdPQ); neither shares code with the C oracle's heap."""
     if use_reference_pq:
         return oracle_py.ReferencePQ()
-    return _HeapqLikeStd()
+    return oracle_py.StdPQ()
 
 
 def do_graph_search(it, mpa, checker: int, trig: str = "spec", use_reference_pq: bool = True) -> Info:

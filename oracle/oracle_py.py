@@ -1,6 +1,7 @@
-"""ctypes binding of the CPU oracle (oracle/libpdmpc_oracle.so) and of the
+"""ctypes binding of the CPU oracle (oracle/libpdmpc_oracle.so), of the
 reference's own priority queue compiled against stub MEX headers
-(oracle/_ref/libpq_ref.so).
+(oracle/_ref/libpq_ref.so) and of the same queue on libstdc++'s
+std::priority_queue (oracle/libpq_std.so).
 
 TEST INFRASTRUCTURE: import only from tests/, __graft_entry__.smoke() and
 bench.py's cpu_baseline / --impl reference legs.  Never from p-dmpc_b200/.
@@ -8,6 +9,7 @@ bench.py's cpu_baseline / --impl reference legs.  Never from p-dmpc_b200/.
 from __future__ import annotations
 
 import ctypes as C
+import functools
 import os
 import subprocess
 import sys
@@ -24,18 +26,32 @@ from pdmpc_b200.records import BatchResult, SearchBatch  # noqa: E402
 
 ORACLE_LIB = os.path.join(_HERE, "libpdmpc_oracle.so")
 PQ_REF_LIB = os.path.join(_HERE, "_ref", "libpq_ref.so")
+PQ_STD_LIB = os.path.join(_HERE, "libpq_std.so")
 
 _p_f64 = C.POINTER(C.c_double)
 _p_i64 = C.POINTER(C.c_int64)
 
 
 def build(force: bool = False) -> None:
-    """make -C oracle (oracle .so; reference PQ .so when /root/reference exists)."""
+    """make -C oracle: the oracle .so, the std::priority_queue .so and, when the reference checkout is given
+    (oracle/Makefile REFERENCE=...), the reference's own PQ .so."""
     if force or not os.path.exists(ORACLE_LIB) or \
             os.path.getmtime(ORACLE_LIB) < os.path.getmtime(os.path.join(_HERE, "pdmpc_oracle.c")):
         subprocess.run(["make", "-C", _HERE, "libpdmpc_oracle.so"], check=True, capture_output=True)
+    if force or not os.path.exists(PQ_STD_LIB) or \
+            os.path.getmtime(PQ_STD_LIB) < os.path.getmtime(os.path.join(_HERE, "pq_std_driver.cpp")):
+        subprocess.run(["make", "-C", _HERE, "libpq_std.so"], check=True, capture_output=True)
     if not os.path.exists(PQ_REF_LIB) or force:
         subprocess.run(["make", "-C", _HERE, "ref"], check=True, capture_output=True)
+
+
+@functools.lru_cache(maxsize=None)
+def have_reference_pq() -> bool:
+    """True when the reference's priority-queue MEX is built (oracle/_ref/libpq_ref.so).  It is built from the
+    reference checkout (oracle/Makefile, REFERENCE=...), which is not part of this repository; without it the
+    tests drive the matrix-form restatement with StdPQ instead."""
+    build()
+    return os.path.exists(PQ_REF_LIB)
 
 
 _LIB = None
@@ -190,6 +206,48 @@ class ReferencePQ:
 
     def size(self) -> int:
         return int(ReferencePQ._lib.pq_ref_size(self.obj))
+
+
+class StdPQ:
+    """The reference's queue on libstdc++'s std::priority_queue (oracle/pq_std_driver.cpp): shares no code with
+    OraclePQ.  Same interface as ReferencePQ."""
+
+    _lib = None
+
+    def __init__(self):
+        if StdPQ._lib is None:
+            build()
+            L = C.CDLL(PQ_STD_LIB)
+            L.pq_std_new.restype = C.c_void_p
+            L.pq_std_free.argtypes = [C.c_void_p]
+            L.pq_std_free.restype = None
+            L.pq_std_push.argtypes = [C.c_void_p, _p_f64, _p_f64, C.c_int64]
+            L.pq_std_push.restype = None
+            L.pq_std_pop.argtypes = [C.c_void_p, _p_f64]
+            L.pq_std_pop.restype = C.c_int64
+            L.pq_std_size.argtypes = [C.c_void_p]
+            L.pq_std_size.restype = C.c_int64
+            StdPQ._lib = L
+        self.obj = StdPQ._lib.pq_std_new()
+
+    def push(self, ids, vals):
+        ids = np.ascontiguousarray(np.atleast_1d(ids), dtype=np.float64)
+        vals = np.ascontiguousarray(np.atleast_1d(vals), dtype=np.float64)
+        StdPQ._lib.pq_std_push(self.obj, ids.ctypes.data_as(_p_f64), vals.ctypes.data_as(_p_f64), int(ids.size))
+
+    def pop(self):
+        v = C.c_double()
+        i = StdPQ._lib.pq_std_pop(self.obj, C.byref(v))
+        return int(i), v.value
+
+    def size(self) -> int:
+        return int(StdPQ._lib.pq_std_size(self.obj))
+
+    def __del__(self):
+        try:
+            StdPQ._lib.pq_std_free(self.obj)
+        except Exception:
+            pass
 
 
 def plan_batch(mpa, batch: SearchBatch, n_threads: int = 1, hash_valid_pops_only: bool = False) -> BatchResult:

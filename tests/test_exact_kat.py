@@ -173,6 +173,7 @@ def emulate_costs(mpa, x0, y0, trims, ref, v_ref, dt):
 
 def test_expand_node_costs_against_emulated_ieee_arithmetic():
     rng = np.random.default_rng(3)
+    use_reference_pq = oracle_py.have_reference_pq()
     for Hp, dt in ((3, 0.2), (4, 0.2), (3, 0.25)):
         mpa = literal_mpa(Hp, dt)
         iters = []
@@ -191,7 +192,7 @@ def test_expand_node_costs_against_emulated_ieee_arithmetic():
             assert np.array_equal(h.view(np.uint64), res.h_path[i].view(np.uint64)), (Hp, dt, i)
             assert (x, y) == (res.y_predicted[i, -1, 0], res.y_predicted[i, -1, 1])
             # the matrix-form restatement follows the same arithmetic
-            info = ml.do_graph_search(it, mpa, CHECKER_SAT)
+            info = ml.do_graph_search(it, mpa, CHECKER_SAT, use_reference_pq=use_reference_pq)
             g2 = np.array([info.tree.g[j - 1] for j in info.tree_path])      # node ids are 1-based
             h2 = np.array([info.tree.h[j - 1] for j in info.tree_path])
             assert np.array_equal(g2.view(np.uint64), g.view(np.uint64)) and np.array_equal(h2.view(np.uint64), h.view(np.uint64))

@@ -1,6 +1,7 @@
 """The single-thread heap of the lane-per-search kernel (p-dmpc_b200/csrc/pdmpc_heap_serial.h,
 compiled here as host code) against the reference's unmodified priority-queue MEX source
-(oracle/_ref/libpq_ref.so) and the oracle's literal libstdc++ restatement: identical pop
+(oracle/_ref/libpq_ref.so, when built), the same queue on libstdc++'s std::priority_queue and
+the oracle's literal libstdc++ restatement: identical pop
 sequences on tie-dense push/pop mixes, including the early-stop pop."""
 import ctypes as C
 import os
@@ -32,14 +33,11 @@ def hs():
     return L
 
 
-HAVE_REF_PQ = os.path.exists(oracle_py.PQ_REF_LIB) or os.path.exists("/root/reference")
-
-
 @pytest.mark.parametrize("seed", range(12))
 def test_serial_heap_matches_reference_and_oracle(hs, seed):
     rng = np.random.default_rng(1000 + seed)
-    refs = [oracle_py.OraclePQ()]
-    if HAVE_REF_PQ:
+    refs = [oracle_py.OraclePQ(), oracle_py.StdPQ()]
+    if oracle_py.have_reference_pq():
         refs.append(oracle_py.ReferencePQ())
     q = hs.hs_new()
     next_id = 1
@@ -67,7 +65,7 @@ def test_serial_heap_matches_reference_and_oracle(hs, seed):
                 ids = np.arange(next_id, next_id + m)
                 next_id += m
                 for r in refs:
-                    if isinstance(r, oracle_py.ReferencePQ):
+                    if isinstance(r, (oracle_py.ReferencePQ, oracle_py.StdPQ)):
                         r.push(ids, vals)
                     else:
                         for i, v in zip(ids, vals):

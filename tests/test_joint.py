@@ -180,8 +180,9 @@ def test_joint_errors_are_loud(planner):
 def test_joint_oracle_against_matrix_form_restatement():
     """Second, independent restatement of the joint search (oracle/matlab_literal.py: nV x nNodes arrays,
     successor ids through trim_tuple / cartprod with the radix offsets, the reference's own priority-queue
-    source): same pop sequence length, node count, trims, poses and joint costs as the C oracle."""
+    source when built): same pop sequence length, node count, trims, poses and joint costs as the C oracle."""
     from oracle import matlab_literal as ml
+    use_reference_pq = oracle_py.have_reference_pq()
     mpa6 = get_mpa("single_speed", non_convex=False)
     mpa3 = get_mpa("single_speed", Hp=3, non_convex=False)     # three vehicles: 12^3 children per expansion
     blocked = crossing_pair(mpa6, 0.35)
@@ -193,7 +194,7 @@ def test_joint_oracle_against_matrix_form_restatement():
         nV = len(rows)
         batch = SearchBatch.from_iters(rows, Hp, CHECKER_SAT, mpa.dt_seconds)
         ref = oracle_py.joint_plan_batch(mpa, batch, nV)
-        info = ml.do_joint_graph_search(rows, mpa)
+        info = ml.do_joint_graph_search(rows, mpa, use_reference_pq=use_reference_pq)
         assert info.is_exhausted == bool(ref.is_exhausted[0])
         assert info.n_expanded == int(ref.n_expanded[0]) and len(info.pops) == int(ref.n_pops[0])
         h = 0xcbf29ce484222325

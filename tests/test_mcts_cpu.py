@@ -2,8 +2,6 @@
 matrix-form restatement that uses numpy's independent MT19937, the reference's
 own priority-queue source (when built) and MATLAB-style `children` bookkeeping;
 hand-countable cases; the random stream against numpy's RandomState."""
-import os
-
 import numpy as np
 import pytest
 
@@ -14,8 +12,6 @@ from helpers import load_golden, rect, straight_iter
 from test_oracle_cpu import _iters_from_batch
 from pdmpc_b200.mpa import get_mpa
 from pdmpc_b200.records import CHECKER_INTERX, CHECKER_SAT, SearchBatch
-
-HAVE_REF_PQ = os.path.exists(oracle_py.PQ_REF_LIB) or os.path.isdir("/root/reference")
 
 
 @pytest.mark.parametrize("seed", [1, 2, 42, 5489, 2**31 + 7])
@@ -40,7 +36,7 @@ def _compare_with_literal(mpa, batch, picks, seeds, nmax):
     assert (got.status == 0).all()
     for i in picks:
         info = ml.do_mcts(_iters_from_batch(batch, i), mpa, batch.checker, int(seeds[i]), nmax,
-                          use_reference_pq=HAVE_REF_PQ)
+                          use_reference_pq=oracle_py.have_reference_pq())
         assert info.is_exhausted == bool(got.is_exhausted[i]), i
         assert info.n_expanded == got.n_expanded[i] and info.n_traversals == got.n_pops[i], i
         assert _fnv(info.pops) == int(got.pop_hash[i]), i

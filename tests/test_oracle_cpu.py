@@ -2,7 +2,8 @@
 
   * the reference's own known-answer tests (tests/unittests/hlc/intersect_unittest.m:8-54)
   * the heap restatement against the reference's UNMODIFIED priority-queue source
-    compiled here (oracle/_ref/libpq_ref.so) + this container's libstdc++
+    compiled here (oracle/_ref/libpq_ref.so) + this container's libstdc++, and against
+    the same queue on libstdc++'s std::priority_queue (oracle/libpq_std.so)
   * the C oracle against the second, matrix-form restatement (oracle/matlab_literal.py)
   * both against the committed golden fixtures (tests/golden, tools/make_golden.py)
 """
@@ -18,7 +19,6 @@ from helpers import GOLDEN_CASES, GOLDEN_DIR, load_golden, rect
 
 HEX = np.array([[-7.0749, -2.8728, 9.8889, 21.3024, 15.3469, 7.9387],
                 [-6.4707, -12.1152, -24.4428, -3.0950, 19.3838, 18.7030]])
-HAVE_REF_PQ = os.path.exists(oracle_py.PQ_REF_LIB) or os.path.exists("/root/reference")
 
 
 @pytest.fixture(scope="module")
@@ -46,11 +46,23 @@ def test_kat_intersect_lanelets(impl, lanelet1):
 
 
 # ---- priority queue: oracle heap == reference MEX + libstdc++ ----------------------
-@pytest.mark.skipif(not HAVE_REF_PQ, reason="oracle/_ref not built and /root/reference absent")
 @pytest.mark.parametrize("seed", range(6))
 def test_pq_matches_reference_mex(seed):
+    if not oracle_py.have_reference_pq():
+        pytest.skip("needs the reference's priority-queue source (oracle/Makefile REFERENCE=<reference checkout>)")
+    _pq_script_matches(seed, oracle_py.ReferencePQ())
+
+
+@pytest.mark.parametrize("seed", range(6))
+def test_pq_matches_std_priority_queue(seed):
+    """The same scripts against the queue on libstdc++'s std::priority_queue, which shares no code with the
+    oracle's heap and is the matrix-form restatement's queue where the reference's source is not built."""
+    _pq_script_matches(seed, oracle_py.StdPQ())
+
+
+def _pq_script_matches(seed, ref):
     rng = np.random.default_rng(seed)
-    ref, mine = oracle_py.ReferencePQ(), oracle_py.OraclePQ()
+    mine = oracle_py.OraclePQ()
     assert ref.pop()[0] == -1 and mine.pop()[0] == -1        # empty -> -1 (mex.cpp:87-94)
     next_id = 1
     for _ in range(400):
@@ -174,7 +186,7 @@ def test_matrix_form_reproduces_golden_subset(name):
     order = np.argsort(exp.n_pops)
     pick = set(order[:3].tolist() + order[-2:].tolist() + np.flatnonzero(exp.is_exhausted)[:2].tolist())
     for i in sorted(pick):
-        info = ml.do_graph_search(_iters_from_batch(batch, i), mpa, batch.checker, use_reference_pq=HAVE_REF_PQ)
+        info = ml.do_graph_search(_iters_from_batch(batch, i), mpa, batch.checker, use_reference_pq=oracle_py.have_reference_pq())
         assert info.is_exhausted == bool(exp.is_exhausted[i])
         assert info.n_expanded == exp.n_expanded[i] and len(info.pops) == exp.n_pops[i]
         h = 0xcbf29ce484222325
@@ -195,7 +207,7 @@ def test_libm_trig_changes_no_discrete_result():
     order = np.argsort(exp.n_pops)
     for i in order[:4].tolist() + order[-1:].tolist():
         info = ml.do_graph_search(_iters_from_batch(batch, i), mpa, batch.checker, trig="libm",
-                                  use_reference_pq=HAVE_REF_PQ)
+                                  use_reference_pq=oracle_py.have_reference_pq())
         assert info.is_exhausted == bool(exp.is_exhausted[i])
         if not info.is_exhausted:
             assert info.predicted_trims == exp.trims[i, 1:].tolist()

@@ -12,6 +12,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
+from bench import RECORD_CACHE  # noqa: E402
 from pdmpc_b200 import capi  # noqa: E402
 if os.environ.get('PDMPC_LIB'):
     capi.LIB_PATH = os.environ['PDMPC_LIB']
@@ -19,7 +20,7 @@ if os.environ.get('PDMPC_LIB'):
 from pdmpc_b200.mpa import get_mpa  # noqa: E402
 from pdmpc_b200.records import BatchResult, SearchBatch  # noqa: E402
 
-files = sorted(glob.glob(sys.argv[1] if len(sys.argv) > 1 else "build/bench_records/triple_speed_20v_35t_block00*.npz"))[:64]
+files = sorted(glob.glob(sys.argv[1] if len(sys.argv) > 1 else os.path.join(RECORD_CACHE, "triple_speed_20v_35t_block00*.npz")))[:64]
 mpa = get_mpa("triple_speed", non_convex=True)
 batch = SearchBatch.concat([SearchBatch.load(f) for f in files])
 p = capi.Planner(0)

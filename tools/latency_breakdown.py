@@ -10,12 +10,13 @@ import time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import numpy as np  # noqa: E402
+from bench import RECORD_CACHE  # noqa: E402
 from pdmpc_b200 import capi  # noqa: E402
 from pdmpc_b200.mpa import get_mpa  # noqa: E402
 from pdmpc_b200.records import BatchResult  # noqa: E402
 
 mpa = get_mpa("triple_speed", non_convex=True)
-ts = pickle.load(open(os.path.join(ROOT, "build/bench_records/triple_speed_20v_35t_block0000.npz.ts.pkl"), "rb"))
+ts = pickle.load(open(os.path.join(RECORD_CACHE, "triple_speed_20v_35t_block0000.npz.ts.pkl"), "rb"))
 p = capi.Planner(0)
 p.upload_mpa(mpa)
 p.set_cta_queue(True)

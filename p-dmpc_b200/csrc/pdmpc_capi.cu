@@ -93,26 +93,134 @@ using CtaMDepsSmemT = CtaSmem<kCtaMHeap, kCtaMPts, kCtaCheckers, kCtaMastersDeps
 static_assert(sizeof(CtaSmemT) <= kSmemLimit && sizeof(CtaDepsSmemT) <= kSmemLimit && sizeof(CtaMSmemT) <= kSmemLimit &&
               sizeof(CtaMDepsSmemT) <= kSmemLimit, "CTA shapes must fit one SM");
 
-struct DBuf {
+// Buffer that grows on demand and frees its memory with the handle: device memory, or pinned host memory for staging.
+template <bool kPinned>
+struct Buf {
     void *p = nullptr;
     size_t cap = 0;
+    Buf() = default;
+    Buf(const Buf &) = delete;
+    Buf &operator=(const Buf &) = delete;
+    ~Buf() { drop(); }
     cudaError_t reserve(size_t bytes) {
         if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-        size_t want = bytes + bytes / 8 + 256;
-        cudaError_t e = cudaMalloc(&p, want);
+        drop();
+        const size_t want = kPinned ? bytes + bytes / 4 + 4096 : bytes + bytes / 8 + 256;
+        cudaError_t e = kPinned ? cudaHostAlloc(&p, want, cudaHostAllocDefault) : cudaMalloc(&p, want);
         if (e == cudaSuccess) cap = want;
+        else p = nullptr;
         return e;
     }
-    void release() {
-        if (p) cudaFree(p);
+    template <class T> T *as() const { return reinterpret_cast<T *>(p); }
+
+  private:
+    void drop() {
+        if (p) kPinned ? cudaFreeHost(p) : cudaFree(p);
         p = nullptr;
         cap = 0;
     }
-    template <class T> T *as() const { return reinterpret_cast<T *>(p); }
 };
+using DBuf = Buf<false>;
+using PinnedBuf = Buf<true>;
+
+// Launch shapes of the search.  The values are those of pdmpc_set_variant and pdmpc_stats.shape.
+enum Shape {
+    kShapeAuto = 0,
+    kShapeLatency = 1,   // one search per one-warp CTA (search_kernel): every checker, pop traces, dependencies
+    kShapeTile2 = 2,     // two searches per warp (search_tile_kernel<16>): InterX batches, the throughput shape
+    kShapeTile4 = 3,     // four searches per warp (search_tile_kernel<8>)
+    kShapeCta = 4,       // one CTA per search, or several masters per CTA (pdmpc_cta.cuh)
+    kShapeCtaValid = 5,  // the same with the valid-only queue
+};
+
+// The input arrays of a batch, in the order of their device buffers (pdmpc_handle::b_in) and of the packed staging block.
+enum InArray {
+    kInX0, kInY0, kInYaw0, kInTrim0, kInRefX, kInRefY, kInVRef, kInSlotPtr, kInPolyPtr, kInVertX, kInVertY,
+    kInLanePtr, kInLaneX, kInLaneY, kInOrder, kNumIn
+};
+constexpr size_t kInElem[kNumIn] = {sizeof(double), sizeof(double), sizeof(double), sizeof(int),
+                                    sizeof(double), sizeof(double), sizeof(double), sizeof(int),
+                                    sizeof(int),    sizeof(double), sizeof(double), sizeof(int),
+                                    sizeof(double), sizeof(double), sizeof(int)};
+
+// Element ranges [lo, hi) of the input arrays that belong to searches [s0, s1).  p, v and l are the obstacle polygons,
+// vertices and lanelet points before s0 and s1 (the CSR offsets there); the offset arrays take one entry more.
+// The whole batch is the range [0, n) with p, v, l = 0 and the totals.
+struct InRange {
+    size_t lo[kNumIn], hi[kNumIn];
+};
+static InRange in_range(int Hp, int s0, int s1, int p0, int p1, int v0, int v1, int l0, int l1) {
+    const size_t H = (size_t)Hp;
+    return {{(size_t)s0, (size_t)s0, (size_t)s0, (size_t)s0, s0 * H, s0 * H, s0 * H, s0 * (H + 1), (size_t)p0,
+             (size_t)v0, (size_t)v0, (size_t)2 * s0, (size_t)l0, (size_t)l0, (size_t)s0},
+            {(size_t)s1, (size_t)s1, (size_t)s1, (size_t)s1, s1 * H, s1 * H, s1 * H, s1 * (H + 1) + 1, (size_t)p1 + 1,
+             (size_t)v1, (size_t)v1, (size_t)2 * s1 + 1, (size_t)l1, (size_t)l1, (size_t)s1}};
+}
+
+// The caller's input arrays; the work order comes from the host library.
+static void in_sources(const pdmpc_batch_in *in, const int *order, const void *src[kNumIn]) {
+    const void *s[kNumIn] = {in->x0,       in->y0,     in->yaw0,   in->trim0,    in->ref_x,  in->ref_y,  in->v_ref, in->slot_ptr,
+                             in->poly_ptr, in->vert_x, in->vert_y, in->lane_ptr, in->lane_x, in->lane_y, order};
+    std::copy(s, s + kNumIn, src);
+}
+
+// Names the staged input arrays `d` in b; a single search runs without a work order.
+static void set_batch(BatchDev &b, int n, int checker, double dt, const void *const d[kNumIn]) {
+    b.n = n; b.checker = checker; b.dt = dt;
+    b.x0 = (const double *)d[kInX0]; b.y0 = (const double *)d[kInY0]; b.yaw0 = (const double *)d[kInYaw0];
+    b.trim0 = (const int *)d[kInTrim0];
+    b.ref_x = (const double *)d[kInRefX]; b.ref_y = (const double *)d[kInRefY]; b.v_ref = (const double *)d[kInVRef];
+    b.slot_ptr = (const int *)d[kInSlotPtr]; b.poly_ptr = (const int *)d[kInPolyPtr];
+    b.vert_x = (const double *)d[kInVertX]; b.vert_y = (const double *)d[kInVertY];
+    b.lane_ptr = (const int *)d[kInLanePtr]; b.lane_x = (const double *)d[kInLaneX]; b.lane_y = (const double *)d[kInLaneY];
+    b.order = n > 1 ? (const int *)d[kInOrder] : nullptr;
+}
+
+// Work order of searches [s0, s1) into order[0, s1 - s0): the searches with the most obstacle polygons first (they are
+// the ones most likely to run long / exhaust, so the tail of a launch is made of short searches).  A stable counting
+// sort; false if slot_ptr decreases.
+static bool heavy_first_order(const int *slot_ptr, int Hp, int s0, int s1, int *order) {
+    auto key = [&](int i) { return slot_ptr[(size_t)(i + 1) * (Hp + 1)] - slot_ptr[(size_t)i * (Hp + 1)]; };
+    int kmax = 0;
+    for (int i = s0; i < s1; ++i) {
+        if (key(i) < 0) return false;
+        kmax = std::max(kmax, key(i));
+    }
+    std::vector<int> cnt(kmax + 2, 0);
+    for (int i = s0; i < s1; ++i) cnt[kmax - key(i) + 1]++;
+    for (int k = 0; k <= kmax; ++k) cnt[k + 1] += cnt[k];
+    for (int i = s0; i < s1; ++i) order[cnt[kmax - key(i)]++] = i;
+    return true;
+}
+
+// The result fields in the order of pdmpc_batch_out and of the output block (d_out_pack); the counter block follows them.
+constexpr int kNumOut = 13;
+constexpr size_t kCounterBytes = 16 * sizeof(unsigned long long);
+struct OutFields {
+    size_t bytes[kNumOut];   // per search
+    void *dst[kNumOut];      // the caller's arrays (null: not wanted)
+};
+static OutFields out_fields(int Hp, const pdmpc_batch_out *o = nullptr) {
+    const size_t H = (size_t)Hp, S = PDMPC_AREA_STRIDE;
+    OutFields f = {{sizeof(int), 1, sizeof(int), sizeof(int), sizeof(uint64_t), (H + 1) * sizeof(int),
+                    (H + 1) * sizeof(int), H * 3 * sizeof(double), (H + 1) * sizeof(double), (H + 1) * sizeof(double),
+                    H * sizeof(int), H * S * sizeof(double), H * S * sizeof(double)},
+                   {}};
+    if (o) {
+        void *d[kNumOut] = {o->status, o->is_exhausted, o->n_expanded, o->n_pops,     o->pop_hash, o->trims, o->tree_path,
+                            o->y_predicted, o->g_path,  o->h_path,     o->shape_npts, o->shape_x,  o->shape_y};
+        std::copy(d, d + kNumOut, f.dst);
+    }
+    return f;
+}
+
+// The arena slots from `slot` on: a launch that runs beside others gets slots of its own.
+static ArenaDev arena_from(const ArenaDev &a, size_t slot) {
+    ArenaDev x = a;
+    const size_t off = slot * (size_t)a.cap;
+    x.a += off; x.b += off; x.cs += off; x.heap += off;
+    return x;
+}
 
 }  // namespace
 
@@ -128,8 +236,7 @@ struct pdmpc_handle {
     int esc_short_list = -1;          // lists up to this long run with one master per CTA (-1: 3 per SM)
     DBuf esc;                         // [0] count, [1] producers done, [4..] escalated search indices
     DBuf esc_rows;                    // pipeline: packed output rows of the escalated searches
-    void *pin_esc = nullptr;
-    size_t pin_esc_cap = 0;
+    PinnedBuf pin_esc;
 
     bool cta_valid_only = false;      // pdmpc_set_cta_queue: the CTA shape runs its valid-only queue (shape 5) whenever it is chosen
     bool cta_ok = false;              // the CTA-per-search kernel is launchable (shared memory opt-in granted)
@@ -138,8 +245,7 @@ struct pdmpc_handle {
     DBuf j_veh, j_node, j_heap;       // centralized (joint) search arena
     DBuf d_deps, d_done, d_depx, d_depy, d_depn;
     bool lat_deps_ok = false;
-    void *pin_deps = nullptr;
-    size_t pin_deps_cap = 0;
+    PinnedBuf pin_deps;
     DepsDev deps{};
     bool deps_staged = false;
     std::vector<int> topo_order;      // work order override for the next pdmpc_stage_batch (time-step calls)
@@ -149,8 +255,7 @@ struct pdmpc_handle {
     std::vector<double> chunk_host_ms;   // host time at which chunk c's launch was enqueued (pdmpc_get_pipeline_timeline)
     int chunks_last = 0;
     cudaEvent_t ev_fork = nullptr;
-    void *pin_order = nullptr;
-    size_t pin_order_cap = 0;
+    PinnedBuf pin_order;
     DBuf wc_chunks;
     int pipeline_chunks = 0;          // 0 = auto, 1 = off (tuning/test knob, pdmpc_set_pipeline_chunks)
     cudaStream_t stream = nullptr;
@@ -169,19 +274,16 @@ struct pdmpc_handle {
     // staged batch
     bool staged = false;
     BatchDev batch{};
-    int n_polys = 0, n_verts = 0, n_lane = 0;
-    DBuf b_x0, b_y0, b_yaw0, b_trim0, b_refx, b_refy, b_vref, b_slot, b_poly, b_vx, b_vy, b_plx, b_ply, b_plxy, b_llxy,
-        b_lane, b_lx, b_ly, b_llx, b_lly, b_order, b_seed;
+    DBuf b_in[kNumIn];                // input arrays of a batch staged one by one (large batches, the pipeline)
+    DBuf b_plx, b_ply, b_plxy, b_llx, b_lly, b_llxy, b_seed;
 
     // small batches (one computation level of a time step): every input array in ONE pinned
     // staging buffer -> one H2D copy; every output array in one device block -> one D2H copy
     DBuf d_in_pack, d_out_pack;
-    void *pin_in = nullptr, *pin_out = nullptr;
-    size_t pin_in_cap = 0, pin_out_cap = 0;
+    PinnedBuf pin_in, pin_out;
     cudaEvent_t ev_pack = nullptr;    // completion of the last packed H2D (the pinned buffer is reused)
     bool pack_in_flight = false;
-    bool out_packed = false;
-    size_t out_off[14] = {};          // byte offsets of the output arrays (+ counters) inside d_out_pack
+    size_t out_off[kNumOut + 1] = {}; // byte offsets of the output arrays (+ counters) inside d_out_pack
     size_t out_bytes = 0;
 
     // outputs
@@ -214,8 +316,7 @@ struct pdmpc_handle {
     DBuf t_ids, t_n;
 
     pdmpc_stats stats{};
-    bool timing_pending_h2d = false, timing_pending_kernel = false, timing_pending_d2h = false,
-         unused_ = false;
+    bool timing_pending_h2d = false, timing_pending_kernel = false, timing_pending_d2h = false;
 };
 
 static thread_local std::string g_create_error;
@@ -325,51 +426,17 @@ int pdmpc_destroy(pdmpc_handle *h) {
     if (!h) return PDMPC_OK;
     cudaSetDevice(h->device);
     cudaStreamSynchronize(h->stream);
-    DBuf *bufs[] = {&h->m_succ_ptr, &h->m_succ_te, &h->m_edge_d, &h->m_npts, &h->m_ax, &h->m_ay, &h->b_order,
-                    &h->b_x0, &h->b_y0, &h->b_yaw0, &h->b_trim0,
-                    &h->b_refx, &h->b_refy, &h->b_vref, &h->b_slot, &h->b_poly, &h->b_vx, &h->b_vy,
-                    &h->b_plx, &h->b_ply, &h->b_plxy, &h->b_llxy, &h->b_lane, &h->b_lx, &h->b_ly, &h->b_llx, &h->b_lly,
-                    &h->work_counter, &h->b_seed, &h->a_a, &h->a_b, &h->a_cs, &h->a_heap, &h->t_ids, &h->t_n};
-    for (DBuf *b : bufs) b->release();
-    h->d_in_pack.release();
-    h->d_out_pack.release();
-    h->d_deps.release();
-    h->d_done.release();
-    h->j_veh.release();
-    h->j_node.release();
-    h->j_heap.release();
-    h->d_depx.release();
-    h->d_depy.release();
-    h->d_depn.release();
-    h->wc_chunks.release();
-    for (DBuf *b : {&h->r_bptr, &h->r_bx, &h->r_by, &h->r_pptr, &h->r_px, &h->r_py, &h->r_lptr, &h->r_lidx, &h->r_pidx,
-                    &h->q_rptr, &h->q_rx, &h->q_ry, &h->q_x, &h->q_y, &h->q_yaw, &h->q_speed, &h->q_trim, &h->q_sptr, &h->q_sidx,
-                    &h->q_pptr, &h->q_pidx, &h->q_cs, &h->q_cntp, &h->q_cntv, &h->q_slot, &h->q_vbase, &h->q_poly, &h->q_vx, &h->q_vy,
-                    &h->r_loop, &h->r_speed, &h->i_pid, &h->i_x, &h->i_y, &h->i_speed, &h->i_refx, &h->i_refy, &h->i_vref,
-                    &h->i_ridx, &h->i_cur, &h->i_pred, &h->i_pre, &h->i_cnt, &h->i_lptr, &h->i_lx, &h->i_ly})
-        b->release();
-    for (DBuf *b : {&h->cl_valid, &h->cl_trims, &h->cl_traj, &h->cl_npts, &h->cl_sx, &h->cl_sy, &h->cf_slot, &h->cf_still,
-                    &h->cf_npts, &h->cf_x, &h->cf_y, &h->cf_traj, &h->cf_trims})
-        b->release();
-    h->esc.release();
-    h->esc_rows.release();
-    if (h->pin_esc) cudaFreeHost(h->pin_esc);
-
-    if (h->pin_order) cudaFreeHost(h->pin_order);
     for (cudaEvent_t e : h->ev_chunk) cudaEventDestroy(e);
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
     for (cudaStream_t st : h->s_comp)
         if (st) cudaStreamDestroy(st);
     for (cudaStream_t st : {h->s_in, h->s_out})
         if (st) cudaStreamDestroy(st);
-    if (h->pin_deps) cudaFreeHost(h->pin_deps);
-    if (h->pin_in) cudaFreeHost(h->pin_in);
-    if (h->pin_out) cudaFreeHost(h->pin_out);
     if (h->ev_pack) cudaEventDestroy(h->ev_pack);
     for (auto &ev : h->ev)
         if (ev) cudaEventDestroy(ev);
     cudaStreamDestroy(h->stream);
-    delete h;
+    delete h;   // the device and pinned buffers free themselves
     return PDMPC_OK;
 }
 
@@ -386,7 +453,7 @@ int pdmpc_host_free(void *p) {
 
 int pdmpc_set_variant(pdmpc_handle *h, int32_t variant) {
     if (!h) return PDMPC_ERR_BAD_INPUT;
-    if (variant < 0 || variant > 5)
+    if (variant < kShapeAuto || variant > kShapeCtaValid)
         return fail(h, PDMPC_ERR_BAD_INPUT,
                     "variant must be 0 (auto), 1 (one search per warp), 2 / 3 (tiles: 2 / 4 searches per warp), 4 (cta) or 5 (cta, valid-only queue)");
     h->variant_mode = variant;
@@ -606,35 +673,19 @@ static int validate_batch(pdmpc_handle *h, const pdmpc_batch_in *in) {
 
 constexpr size_t kPackLimit = 1u << 20;   // batches whose arrays total at most 1 MiB take the packed path
 
-static int ensure_pinned(pdmpc_handle *h, void **p, size_t *cap, size_t bytes) {
-    if (bytes <= *cap) return PDMPC_OK;
-    if (*p) cudaFreeHost(*p);
-    *p = nullptr;
-    *cap = 0;
-    const size_t want = bytes + bytes / 4 + 4096;
-    if (cudaHostAlloc(p, want, cudaHostAllocDefault) != cudaSuccess) {
-        *p = nullptr;
-        return fail(h, PDMPC_ERR_ALLOC, "pinned staging buffer allocation failed");
-    }
-    *cap = want;
-    return PDMPC_OK;
+static int ensure_pinned(pdmpc_handle *h, PinnedBuf &buf, size_t bytes) {
+    return buf.reserve(bytes) == cudaSuccess ? PDMPC_OK : fail(h, PDMPC_ERR_ALLOC, "pinned staging buffer allocation failed");
 }
 
 // All output arrays live in one device block (d_out_pack) so that a small batch needs a single
 // device->host copy; the order is the one of pdmpc_batch_out, the counters come last.
 static int ensure_outputs(pdmpc_handle *h, int n) {
-    const size_t Hp = (size_t)h->mpa.Hp;
+    const OutFields f = out_fields(h->mpa.Hp);
     const size_t n1 = std::max(n, 1);
-    const size_t sizes[14] = {
-        n1 * sizeof(int), n1, n1 * sizeof(int), n1 * sizeof(int), n1 * sizeof(uint64_t),
-        n1 * (Hp + 1) * sizeof(int), n1 * (Hp + 1) * sizeof(int), n1 * Hp * 3 * sizeof(double),
-        n1 * (Hp + 1) * sizeof(double), n1 * (Hp + 1) * sizeof(double), n1 * Hp * sizeof(int),
-        n1 * Hp * PDMPC_AREA_STRIDE * sizeof(double), n1 * Hp * PDMPC_AREA_STRIDE * sizeof(double),
-        16 * sizeof(unsigned long long)};
     size_t off = 0;
-    for (int i = 0; i < 14; ++i) {
+    for (int i = 0; i <= kNumOut; ++i) {
         h->out_off[i] = off;
-        off = (off + sizes[i] + 15) / 16 * 16;
+        off = (off + (i < kNumOut ? n1 * f.bytes[i] : kCounterBytes) + 15) / 16 * 16;
     }
     h->out_bytes = off;
     CU_TRY(h, h->d_out_pack.reserve(off));
@@ -654,50 +705,85 @@ static int ensure_outputs(pdmpc_handle *h, int n) {
     o.shape_npts = reinterpret_cast<int *>(base + h->out_off[10]);
     o.shape_x = reinterpret_cast<double *>(base + h->out_off[11]);
     o.shape_y = reinterpret_cast<double *>(base + h->out_off[12]);
-    o.counters = reinterpret_cast<unsigned long long *>(base + h->out_off[13]);
+    o.counters = reinterpret_cast<unsigned long long *>(base + h->out_off[kNumOut]);
     return PDMPC_OK;
 }
 
-// The device side of staging: `dptr` = the fifteen batch arrays in device memory (order of pdmpc_stage_batch's `srcs`);
-// polylines of the InterX checker, output block.  Shared by the host-buffer path and pdmpc_plan_timestep_from_states.
-static int stage_finish(pdmpc_handle *h, int n, int checker, double dt, const void *const dptr[15], int np, int nv, int nl) {
-    int rc = PDMPC_OK;
+// The statistics in the counter block of a finished launch.
+static void read_counters(pdmpc_handle *h, const unsigned long long counters[16]) {
+    h->stats.total_pops = (int64_t)counters[0];
+    h->stats.total_nodes = (int64_t)counters[1];
+    h->stats.total_obstacle_cols = (int64_t)counters[2];
+    if (counters[3]) h->stats.handed_over = (int32_t)counters[3];   // shape 5: searches re-run with the exact queue
+    h->stats.escalated = (int32_t)counters[6];
+#ifdef PDMPC_PROFILE
+    {
+#ifdef PDMPC_PROFILE_CHECKER
+        static const char *names[8] = {"c:wait_job", "c:tables+place", "c:interx_obstacles", "c:interx_rest", "c:sincos+publish", "-", "-", "c:other"};
+#else
+        static const char *names[8] = {"setup", "heap_pop", "loads+place", "check", "expand", "heap_push", "wait_children", "loop"};
+        // (CTA kernel master: set-up, pending children, loads + heap pop, flag wait, job hand-over, children, pushes, end)
+#endif
+        double tot = 0;
+        for (int i = 0; i < 8; ++i) tot += (double)counters[8 + i];
+        fprintf(stderr, "[pdmpc profile] cycles per pop:");
+        for (int i = 0; i < 8; ++i)
+            fprintf(stderr, " %s=%.0f", names[i], (double)counters[8 + i] / (double)std::max<unsigned long long>(counters[0], 1));
+        fprintf(stderr, " total=%.0f\n", tot / (double)std::max<unsigned long long>(counters[0], 1));
+        if (counters[5])
+            fprintf(stderr, "[pdmpc profile] checker 0: %.0f cycles per job over %llu jobs\n",
+                    (double)counters[4] / (double)counters[5], counters[5]);
+    }
+#endif
+}
+
+// InterX checker: NaN-separated polylines (vectorize_all_obstacles.m) of the obstacles and lanelet bounds, built on the
+// device.  reserve_polylines sizes them for the staged batch with np polygons, nv vertices and nl lanelet points and
+// names them in it (the SAT checker has none); build_polylines builds those of polygons [p0, p1) and of the lanelet
+// bounds of searches [s0, s1) on stream S.
+static int reserve_polylines(pdmpc_handle *h, int np, int nv, int nl) {
     BatchDev &b = h->batch;
-    b.n = n; b.checker = checker; b.dt = dt;
-    b.x0 = (const double *)dptr[0]; b.y0 = (const double *)dptr[1]; b.yaw0 = (const double *)dptr[2];
-    b.trim0 = (const int *)dptr[3];
-    b.ref_x = (const double *)dptr[4]; b.ref_y = (const double *)dptr[5]; b.v_ref = (const double *)dptr[6];
-    b.slot_ptr = (const int *)dptr[7]; b.poly_ptr = (const int *)dptr[8];
-    b.vert_x = (const double *)dptr[9]; b.vert_y = (const double *)dptr[10];
-    b.lane_ptr = (const int *)dptr[11]; b.lane_x = (const double *)dptr[12]; b.lane_y = (const double *)dptr[13];
-    b.order = n > 1 ? (const int *)dptr[14] : nullptr;
     b.pl_x = b.pl_y = b.ll_x = b.ll_y = nullptr;
     b.pl_xy = b.ll_xy = nullptr;
-    h->stats.kernel_launches = 0;
-    if (checker == PDMPC_CHECKER_INTERX) {
-        // NaN-separated polylines (vectorize_all_obstacles.m) built on the device
-        CU_TRY(h, h->b_plx.reserve(((size_t)nv + np + 1) * sizeof(double)));
-        CU_TRY(h, h->b_ply.reserve(((size_t)nv + np + 1) * sizeof(double)));
-        CU_TRY(h, h->b_llx.reserve(((size_t)nl + 2 * n + 1) * sizeof(double)));
-        CU_TRY(h, h->b_lly.reserve(((size_t)nl + 2 * n + 1) * sizeof(double)));
-        CU_TRY(h, h->b_plxy.reserve(((size_t)nv + np + 1) * sizeof(double2)));
-        CU_TRY(h, h->b_llxy.reserve(((size_t)nl + 2 * n + 1) * sizeof(double2)));
-        if (np) {
-            build_polyline_kernel<<<(np + 127) / 128, 128, 0, h->stream>>>(
-                np, b.poly_ptr, b.vert_x, b.vert_y, h->b_plx.as<double>(), h->b_ply.as<double>(), 0, h->b_plxy.as<double2>());
-            h->stats.kernel_launches++;
-        }
-        if (n) {
-            build_polyline_kernel<<<(2 * n + 127) / 128, 128, 0, h->stream>>>(
-                2 * n, b.lane_ptr, b.lane_x, b.lane_y, h->b_llx.as<double>(), h->b_lly.as<double>(), 0, h->b_llxy.as<double2>());
-            h->stats.kernel_launches++;
-        }
-        CU_TRY(h, cudaGetLastError());
-        b.pl_x = h->b_plx.as<double>(); b.pl_y = h->b_ply.as<double>();
-        b.ll_x = h->b_llx.as<double>(); b.ll_y = h->b_lly.as<double>();
-        b.pl_xy = h->b_plxy.as<double2>(); b.ll_xy = h->b_llxy.as<double2>();
+    if (b.checker != PDMPC_CHECKER_INTERX) return PDMPC_OK;
+    CU_TRY(h, h->b_plx.reserve(((size_t)nv + np + 1) * sizeof(double)));
+    CU_TRY(h, h->b_ply.reserve(((size_t)nv + np + 1) * sizeof(double)));
+    CU_TRY(h, h->b_llx.reserve(((size_t)nl + 2 * b.n + 1) * sizeof(double)));
+    CU_TRY(h, h->b_lly.reserve(((size_t)nl + 2 * b.n + 1) * sizeof(double)));
+    CU_TRY(h, h->b_plxy.reserve(((size_t)nv + np + 1) * sizeof(double2)));
+    CU_TRY(h, h->b_llxy.reserve(((size_t)nl + 2 * b.n + 1) * sizeof(double2)));
+    b.pl_x = h->b_plx.as<double>(); b.pl_y = h->b_ply.as<double>();
+    b.ll_x = h->b_llx.as<double>(); b.ll_y = h->b_lly.as<double>();
+    b.pl_xy = h->b_plxy.as<double2>(); b.ll_xy = h->b_llxy.as<double2>();
+    return PDMPC_OK;
+}
+static void build_polylines(pdmpc_handle *h, int p0, int p1, int s0, int s1, cudaStream_t S) {
+    const BatchDev &b = h->batch;
+    if (p1 > p0) {
+        build_polyline_kernel<<<(p1 - p0 + 127) / 128, 128, 0, S>>>(p1 - p0, b.poly_ptr, b.vert_x, b.vert_y, h->b_plx.as<double>(),
+                                                                  h->b_ply.as<double>(), p0, h->b_plxy.as<double2>());
+        h->stats.kernel_launches++;
     }
-    h->n_polys = np; h->n_verts = nv; h->n_lane = nl;
+    if (s1 > s0) {
+        build_polyline_kernel<<<(2 * (s1 - s0) + 127) / 128, 128, 0, S>>>(2 * (s1 - s0), b.lane_ptr, b.lane_x, b.lane_y,
+                                                                        h->b_llx.as<double>(), h->b_lly.as<double>(), 2 * s0,
+                                                                        h->b_llxy.as<double2>());
+        h->stats.kernel_launches++;
+    }
+}
+
+// The device side of staging: `dptr` = the batch's input arrays in device memory, np / nv / nl = its polygons, vertices
+// and lanelet points; polylines of the InterX checker, output block.  Shared by the host-buffer path and
+// pdmpc_plan_timestep_from_states.
+static int stage_finish(pdmpc_handle *h, int n, int checker, double dt, const void *const dptr[kNumIn], int np, int nv, int nl) {
+    set_batch(h->batch, n, checker, dt, dptr);
+    h->stats.kernel_launches = 0;
+    int rc = reserve_polylines(h, np, nv, nl);
+    if (rc != PDMPC_OK) return rc;
+    if (checker == PDMPC_CHECKER_INTERX) {
+        build_polylines(h, 0, np, 0, n, h->stream);
+        CU_TRY(h, cudaGetLastError());
+    }
     rc = ensure_outputs(h, n);
     if (rc != PDMPC_OK) return rc;
     // (caller-owned source buffers were either copied into the pinned block or their copies
@@ -715,16 +801,13 @@ int pdmpc_stage_batch(pdmpc_handle *h, const pdmpc_batch_in *in) {
     if (rc != PDMPC_OK) return rc;
     CU_TRY(h, cudaSetDevice(h->device));
     const int n = in->n_searches, Hp = h->mpa.Hp;
-    const size_t ns = (size_t)n * (Hp + 1);
-    const int np = n ? in->slot_ptr[ns] : 0;
+    const int np = n ? in->slot_ptr[(size_t)n * (Hp + 1)] : 0;
     const int nv = np ? in->poly_ptr[np] : 0;
     const int nl = n ? in->lane_ptr[2 * n] : 0;
     h->staged = false;
     h->stats.h2d_bytes = 0;
     CU_TRY(h, cudaEventRecord(h->ev[0], h->stream));
     static const int zero1[1] = {0};
-    // work order: searches with the most obstacle polygons first (they are the ones most
-    // likely to run long / exhaust), so the tail of the batch is made of short searches
     std::vector<int> order;
     h->deps_staged = false;
     if (n > 1 && (int)h->topo_order.size() == n) {
@@ -733,33 +816,21 @@ int pdmpc_stage_batch(pdmpc_handle *h, const pdmpc_batch_in *in) {
         order.resize(n);
         for (int i = 0; i < n; ++i) order[i] = i;
     } else if (n > 1) {
-        std::vector<int> key(n);
         order.resize(n);
-        int kmax = 0;
-        for (int i = 0; i < n; ++i) {
-            key[i] = in->slot_ptr[(size_t)(i + 1) * (Hp + 1)] - in->slot_ptr[(size_t)i * (Hp + 1)];
-            kmax = std::max(kmax, key[i]);
-        }
-        std::vector<int> cnt(kmax + 2, 0);
-        for (int i = 0; i < n; ++i) cnt[kmax - key[i] + 1]++;          // counting sort, descending key, stable
-        for (int k = 0; k <= kmax; ++k) cnt[k + 1] += cnt[k];
-        for (int i = 0; i < n; ++i) order[cnt[kmax - key[i]]++] = i;
+        heavy_first_order(in->slot_ptr, Hp, 0, n, order.data());
     }
-    const void *srcs[15] = {in->x0, in->y0, in->yaw0, in->trim0, in->ref_x, in->ref_y, in->v_ref,
-                            n ? in->slot_ptr : zero1, n ? in->poly_ptr : zero1, in->vert_x, in->vert_y,
-                            n ? in->lane_ptr : zero1, in->lane_x, in->lane_y, order.data()};
-    const size_t nbytes[15] = {n * sizeof(double), n * sizeof(double), n * sizeof(double), n * sizeof(int),
-                               (size_t)n * Hp * sizeof(double), (size_t)n * Hp * sizeof(double),
-                               (size_t)n * Hp * sizeof(double), (ns + 1) * sizeof(int), ((size_t)np + 1) * sizeof(int),
-                               (size_t)nv * sizeof(double), (size_t)nv * sizeof(double),
-                               ((size_t)2 * n + 1) * sizeof(int), (size_t)nl * sizeof(double),
-                               (size_t)nl * sizeof(double), order.size() * sizeof(int)};
-    size_t in_off[15], in_total = 0;
-    for (int i = 0; i < 15; ++i) {
+    const void *srcs[kNumIn];
+    in_sources(in, order.data(), srcs);
+    if (n == 0) srcs[kInSlotPtr] = srcs[kInPolyPtr] = srcs[kInLanePtr] = zero1;
+    const InRange all = in_range(Hp, 0, n, 0, np, 0, nv, 0, nl);
+    size_t nbytes[kNumIn], in_off[kNumIn], in_total = 0;
+    for (int i = 0; i < kNumIn; ++i) nbytes[i] = all.hi[i] * kInElem[i];
+    nbytes[kInOrder] = order.size() * sizeof(int);   // a single search has none
+    for (int i = 0; i < kNumIn; ++i) {
         in_off[i] = in_total;
         in_total = (in_total + nbytes[i] + 15) / 16 * 16;
     }
-    const void *dptr[15];
+    const void *dptr[kNumIn];
     if (in_total <= kPackLimit) {
         // one pinned staging block, one host->device copy (a level of a time step is a few KB:
         // fifteen separate pageable copies cost more than the search itself)
@@ -767,11 +838,11 @@ int pdmpc_stage_batch(pdmpc_handle *h, const pdmpc_batch_in *in) {
             CU_TRY(h, cudaEventSynchronize(h->ev_pack));
             h->pack_in_flight = false;
         }
-        int rc2 = ensure_pinned(h, &h->pin_in, &h->pin_in_cap, std::max<size_t>(in_total, 16));
+        int rc2 = ensure_pinned(h, h->pin_in, std::max<size_t>(in_total, 16));
         if (rc2 != PDMPC_OK) return rc2;
         CU_TRY(h, h->d_in_pack.reserve(std::max<size_t>(in_total, 16)));
-        unsigned char *pin = static_cast<unsigned char *>(h->pin_in);
-        for (int i = 0; i < 15; ++i) {
+        unsigned char *pin = h->pin_in.as<unsigned char>();
+        for (int i = 0; i < kNumIn; ++i) {
             if (nbytes[i]) memcpy(pin + in_off[i], srcs[i], nbytes[i]);
             dptr[i] = h->d_in_pack.as<unsigned char>() + in_off[i];
         }
@@ -780,12 +851,10 @@ int pdmpc_stage_batch(pdmpc_handle *h, const pdmpc_batch_in *in) {
         h->pack_in_flight = true;
         h->stats.h2d_bytes += (int64_t)in_total;
     } else {
-        DBuf *bufs[15] = {&h->b_x0, &h->b_y0, &h->b_yaw0, &h->b_trim0, &h->b_refx, &h->b_refy, &h->b_vref, &h->b_slot,
-                          &h->b_poly, &h->b_vx, &h->b_vy, &h->b_lane, &h->b_lx, &h->b_ly, &h->b_order};
-        for (int i = 0; i < 15; ++i) {
-            int rc2 = upload(h, *bufs[i], static_cast<const unsigned char *>(srcs[i]), nbytes[i]);
+        for (int i = 0; i < kNumIn; ++i) {
+            int rc2 = upload(h, h->b_in[i], static_cast<const unsigned char *>(srcs[i]), nbytes[i]);
             if (rc2 != PDMPC_OK) return rc2;
-            dptr[i] = bufs[i]->p;
+            dptr[i] = h->b_in[i].p;
         }
         CU_TRY(h, cudaStreamSynchronize(h->stream));   // `order` goes out of scope; callers may reuse their buffers
     }
@@ -795,10 +864,21 @@ int pdmpc_stage_batch(pdmpc_handle *h, const pdmpc_batch_in *in) {
     return stage_finish(h, n, in->checker, in->dt_seconds, dptr, np, nv, nl);
 }
 
+// Node capacity of one search's arena: pdmpc_set_node_capacity, or the full tree from the worst start trim (at most
+// 2^20 nodes), within what the node ids address.
+static int node_cap(const pdmpc_handle *h) {
+    const int cap = h->user_node_cap ? h->user_node_cap : std::min(h->full_tree_nodes + 8, 1 << 20);
+    return std::max(std::min(cap, kMaxNodeCap - 1), 64);
+}
+
+// The CTA kernels (`deps`: their pdmpc_plan_timestep instances) can run: shared memory granted, and the validity flags
+// of a whole search tree fit in shared memory.
+static bool cta_launchable(const pdmpc_handle *h, bool deps) {
+    return (deps ? h->cta_deps_ok : h->cta_ok) && node_cap(h) <= kCtaFlags;
+}
+
 static int ensure_arena(pdmpc_handle *h, int slots) {
-    int cap = h->user_node_cap ? h->user_node_cap : std::min(h->full_tree_nodes + 8, 1 << 20);
-    cap = std::min(cap, kMaxNodeCap - 1);
-    cap = std::max(cap, 64);
+    const int cap = node_cap(h);
     if (slots <= h->arena_slots && cap == h->arena.cap) return PDMPC_OK;
     slots = std::max(slots, h->arena_slots);
     const size_t tot = (size_t)slots * cap;
@@ -820,41 +900,35 @@ static int ensure_arena(pdmpc_handle *h, int slots) {
 }
 
 // ---- warp-level launch shapes -------------------------------------------------------------------------
-//   1 latency   one search per one-warp CTA (search_kernel): every checker, pop traces, dependencies
-//   2 tiles     two searches per warp  (search_tile_kernel<16>): InterX batches, the throughput shape
-//   3 tiles     four searches per warp (search_tile_kernel<8>)
-// Arena slots (concurrently running searches) and grid of shape `shape` for n searches.
-static int warp_shape_grid(const pdmpc_handle *h, int shape, int n, int *slots) {
-    if (shape == 2 || shape == 3) {
-        const int T = shape == 2 ? 2 : 4;
-        const int grid = std::max(1, std::min((n + T - 1) / T, h->num_sms * h->tile_ctas_per_sm[shape - 2]));
-        *slots = grid * T;
-        return grid;
-    }
-    const int grid = std::max(1, std::min(n, h->num_sms * h->lat_ctas_per_sm));
-    *slots = grid;
+// Grid and arena slots (concurrently running searches, if `slots`) of shape `shape` for n searches.
+static int warp_shape_grid(const pdmpc_handle *h, int shape, int n, int *slots = nullptr) {
+    const bool tiles = shape == kShapeTile2 || shape == kShapeTile4;
+    const int T = shape == kShapeTile2 ? 2 : shape == kShapeTile4 ? 4 : 1;
+    const int per_sm = tiles ? h->tile_ctas_per_sm[shape - kShapeTile2] : h->lat_ctas_per_sm;
+    const int grid = std::max(1, std::min((n + T - 1) / T, h->num_sms * per_sm));
+    if (slots) *slots = grid * T;
     return grid;
 }
 
-// The shape a batch of n searches runs in when the caller asked for `variant` (0 = choose).
+// The shape a batch of n searches runs in when the caller asked for `variant` (kShapeAuto = choose).
 static int resolve_warp_shape(const pdmpc_handle *h, int variant, int n, int checker, bool tracing) {
-    if (tracing) return 1;   // pop traces come from the one-search-per-warp kernel
-    if (variant == 0) {
+    if (tracing) return kShapeLatency;   // pop traces come from the one-search-per-warp kernel
+    if (variant == kShapeAuto) {
         // more searches than the latency shape keeps in flight: share the warps (profiles/r02a_*)
-        variant = n > h->num_sms * h->lat_ctas_per_sm ? 2 : 1;
+        variant = n > h->num_sms * h->lat_ctas_per_sm ? kShapeTile2 : kShapeLatency;
     }
-    if ((variant == 2 || variant == 3) && (checker != PDMPC_CHECKER_INTERX || h->tile_ctas_per_sm[variant - 2] < 1))
-        variant = 1;         // the tile shapes hold the InterX checker only
+    if ((variant == kShapeTile2 || variant == kShapeTile4) &&
+        (checker != PDMPC_CHECKER_INTERX || h->tile_ctas_per_sm[variant - kShapeTile2] < 1))
+        variant = kShapeLatency;         // the tile shapes hold the InterX checker only
     return variant;
 }
 
-// One persistent launch of shape 1..3 over batch `bc` on stream S with arena `ar` (sized by warp_shape_grid).
+// One persistent launch of a warp-level shape over batch `bc` on stream S with arena `ar` (sized by warp_shape_grid).
 static int launch_warp_shape(pdmpc_handle *h, int shape, const BatchDev &bc, const ArenaDev &ar, unsigned *wc,
                              const TraceDev &tr, cudaStream_t S) {
-    int slots = 0;
-    const int grid = warp_shape_grid(h, shape, bc.n, &slots);
-    if (shape == 2) KERNEL_TILE2<<<grid, kWarp, kTile2Smem, S>>>(h->mpa, bc, h->out, ar, wc, tr, h->tile_pts_limit);
-    else if (shape == 3) KERNEL_TILE4<<<grid, kWarp, kTile4Smem, S>>>(h->mpa, bc, h->out, ar, wc, tr, h->tile_pts_limit);
+    const int grid = warp_shape_grid(h, shape, bc.n);
+    if (shape == kShapeTile2) KERNEL_TILE2<<<grid, kWarp, kTile2Smem, S>>>(h->mpa, bc, h->out, ar, wc, tr, h->tile_pts_limit);
+    else if (shape == kShapeTile4) KERNEL_TILE4<<<grid, kWarp, kTile4Smem, S>>>(h->mpa, bc, h->out, ar, wc, tr, h->tile_pts_limit);
     else KERNEL_LAT<<<grid, kWarp, sizeof(WarpSmem), S>>>(h->mpa, bc, h->out, ar, wc, tr);
     if (cudaGetLastError() != cudaSuccess) return fail(h, PDMPC_ERR_CUDA, "search kernel launch failed");
     h->stats.kernel_launches++;
@@ -875,8 +949,7 @@ static int escalation_pops(const pdmpc_handle *h, int n) {
     return n >= 300000 ? 4096 : n >= 120000 ? 3072 : PDMPC_ESCALATE_POPS;
 }
 static bool escalation_on(const pdmpc_handle *h, int shape, int n) {
-    const int cap = h->user_node_cap ? h->user_node_cap : std::min(h->full_tree_nodes + 8, 1 << 20);
-    return (shape == 2 || shape == 3) && escalation_pops(h, n) > 0 && h->cta_ok && cap <= kCtaFlags &&
+    return (shape == kShapeTile2 || shape == kShapeTile4) && escalation_pops(h, n) > 0 && cta_launchable(h, false) &&
            n > h->num_sms && h->batch.checker == PDMPC_CHECKER_INTERX;
 }
 
@@ -921,28 +994,26 @@ static int launch_escalated(pdmpc_handle *h, const ArenaDev &ar, int producers, 
 }
 
 // Launches the search of the staged batch (results are identical for all shapes):
-//   1..3 see above;  4 / 5 one CTA per search (pdmpc_cta.cuh), chosen for at most one search per SM
+//   the warp-level shapes see above;  kShapeCta / kShapeCtaValid are chosen for at most one search per SM
 static int launch_search(pdmpc_handle *h, const TraceDev &tr) {
     const int n = h->batch.n;
     CU_TRY(h, cudaSetDevice(h->device));
-    CU_TRY(h, cudaMemsetAsync(h->out.counters, 0, 16 * sizeof(unsigned long long), h->stream));
+    CU_TRY(h, cudaMemsetAsync(h->out.counters, 0, kCounterBytes, h->stream));
     CU_TRY(h, cudaMemsetAsync(h->work_counter.p, 0, 4 * sizeof(unsigned), h->stream));
     h->stats.handed_over = 0;
     h->stats.escalated = 0;
     h->stats.shape = 0;
     h->batch.hash_valid_only = h->cta_valid_only ? 1 : 0;
     if (n == 0) return PDMPC_OK;
-    int variant = h->variant_mode;
-    if (variant == 0 && n <= h->num_sms && tr.search < 0) variant = 4;   // one computation level of a time step
-    if (variant == 4 || variant == 5) {
-        const int cap = h->user_node_cap ? h->user_node_cap : std::min(h->full_tree_nodes + 8, 1 << 20);
-        if (!h->cta_ok || cap > kCtaFlags || tr.search >= 0) variant = 1;   // validity flags of a whole tree must fit in shared memory
-    }
-    if (variant == 4 && h->cta_valid_only) variant = 5;
-    if (variant < 4) variant = resolve_warp_shape(h, variant, n, h->batch.checker, tr.search >= 0);
+    int shape = h->variant_mode;
+    if (shape == kShapeAuto && n <= h->num_sms && tr.search < 0) shape = kShapeCta;   // one computation level of a time step
+    const bool cta = shape == kShapeCta || shape == kShapeCtaValid;
+    if (cta && (!cta_launchable(h, false) || tr.search >= 0)) shape = kShapeLatency;
+    if (shape == kShapeCta && h->cta_valid_only) shape = kShapeCtaValid;
+    if (shape < kShapeCta) shape = resolve_warp_shape(h, shape, n, h->batch.checker, tr.search >= 0);
     unsigned *wc = h->work_counter.as<unsigned>();
-    h->stats.shape = variant;
-    if (variant == 4 || variant == 5) {
+    h->stats.shape = shape;
+    if (shape == kShapeCta || shape == kShapeCtaValid) {
         // at most one search per SM: one master per CTA, every checker serves it; else several masters per CTA
         const bool single = n <= h->num_sms;
         const int nm = single ? 1 : kCtaMasters;
@@ -952,16 +1023,16 @@ static int launch_search(pdmpc_handle *h, const TraceDev &tr) {
         CU_TRY(h, cudaEventRecord(h->ev[2], h->stream));
         if (single)
             KERNEL_CTA<<<grid, CtaShape<1, kCtaCheckers>::kThreads, sizeof(CtaSmemT), h->stream>>>(
-                h->mpa, h->batch, h->out, h->arena, wc, h->cta_heap_smem, variant == 5 ? 1 : 0, DepsDev{});
+                h->mpa, h->batch, h->out, h->arena, wc, h->cta_heap_smem, shape == kShapeCtaValid ? 1 : 0, DepsDev{});
         else
             KERNEL_CTAM<<<grid, CtaShape<kCtaMasters, kCtaCheckers>::kThreads, sizeof(CtaMSmemT), h->stream>>>(
-                h->mpa, h->batch, h->out, h->arena, wc, h->cta_heap_smem, variant == 5 ? 1 : 0, DepsDev{});
+                h->mpa, h->batch, h->out, h->arena, wc, h->cta_heap_smem, shape == kShapeCtaValid ? 1 : 0, DepsDev{});
         CU_TRY(h, cudaGetLastError());
         h->stats.kernel_launches++;
     } else {
         int slots = 0;
-        warp_shape_grid(h, variant, n, &slots);
-        const bool esc = escalation_on(h, variant, n) && tr.search < 0;
+        warp_shape_grid(h, shape, n, &slots);
+        const bool esc = escalation_on(h, shape, n) && tr.search < 0;
         int rc = ensure_arena(h, esc ? slots + h->num_sms * kCtaMasters : slots);
         if (rc != PDMPC_OK) return rc;
         BatchDev bt = h->batch;
@@ -970,14 +1041,10 @@ static int launch_search(pdmpc_handle *h, const TraceDev &tr) {
             if (rc != PDMPC_OK) return rc;
         }
         CU_TRY(h, cudaEventRecord(h->ev[2], h->stream));
-        rc = launch_warp_shape(h, variant, bt, h->arena, wc, tr, h->stream);
+        rc = launch_warp_shape(h, shape, bt, h->arena, wc, tr, h->stream);
         if (rc != PDMPC_OK) return rc;
-        if (esc) {
-            ArenaDev ae = h->arena;   // its own slots behind the tile kernel's
-            const size_t off = (size_t)slots * (size_t)h->arena.cap;
-            ae.a += off; ae.b += off; ae.cs += off; ae.heap += off;
-            int dummy = 0;
-            rc = launch_escalated(h, ae, warp_shape_grid(h, variant, n, &dummy), h->stream);
+        if (esc) {   // its own slots behind the tile kernel's
+            rc = launch_escalated(h, arena_from(h->arena, slots), warp_shape_grid(h, shape, n), h->stream);
             if (rc != PDMPC_OK) return rc;
         }
     }
@@ -1011,73 +1078,44 @@ int pdmpc_fetch_staged(pdmpc_handle *h, pdmpc_batch_out *out) {
     if (!h->staged) return fail(h, PDMPC_ERR_BAD_INPUT, "fetch: no staged batch");
     if (!out || !out->status) return fail(h, PDMPC_ERR_BAD_INPUT, "fetch: out/status is NULL");
     CU_TRY(h, cudaSetDevice(h->device));
-    const size_t n = (size_t)h->batch.n, Hp = (size_t)h->mpa.Hp;
+    const size_t n = (size_t)h->batch.n;
+    const OutFields f = out_fields(h->mpa.Hp, out);
     h->stats.d2h_bytes = 0;
     unsigned long long counters[16] = {0};
-    void *dsts[13] = {out->status, out->is_exhausted, out->n_expanded, out->n_pops, out->pop_hash, out->trims,
-                      out->tree_path, out->y_predicted, out->g_path, out->h_path, out->shape_npts, out->shape_x,
-                      out->shape_y};
-    const size_t bytes[13] = {n * sizeof(int), n, n * sizeof(int), n * sizeof(int), n * sizeof(uint64_t),
-                              n * (Hp + 1) * sizeof(int), n * (Hp + 1) * sizeof(int), n * Hp * 3 * sizeof(double),
-                              n * (Hp + 1) * sizeof(double), n * (Hp + 1) * sizeof(double), n * Hp * sizeof(int),
-                              n * Hp * PDMPC_AREA_STRIDE * sizeof(double), n * Hp * PDMPC_AREA_STRIDE * sizeof(double)};
     const unsigned char *dbase = h->d_out_pack.as<unsigned char>();
     CU_TRY(h, cudaEventRecord(h->ev[4], h->stream));
     if (h->out_bytes <= kPackLimit) {
         // one copy of the whole output block into pinned memory, then scatter on the host
-        int rc = ensure_pinned(h, &h->pin_out, &h->pin_out_cap, h->out_bytes);
+        int rc = ensure_pinned(h, h->pin_out, h->out_bytes);
         if (rc != PDMPC_OK) return rc;
-        CU_TRY(h, cudaMemcpyAsync(h->pin_out, dbase, h->out_bytes, cudaMemcpyDeviceToHost, h->stream));
+        CU_TRY(h, cudaMemcpyAsync(h->pin_out.p, dbase, h->out_bytes, cudaMemcpyDeviceToHost, h->stream));
         CU_TRY(h, cudaEventRecord(h->ev[5], h->stream));
         CU_TRY(h, cudaStreamSynchronize(h->stream));
-        const unsigned char *src = static_cast<const unsigned char *>(h->pin_out);
-        for (int i = 0; i < 13; ++i)
-            if (dsts[i] && bytes[i]) memcpy(dsts[i], src + h->out_off[i], bytes[i]);
-        memcpy(counters, src + h->out_off[13], sizeof(counters));
+        const unsigned char *src = h->pin_out.as<const unsigned char>();
+        for (int i = 0; i < kNumOut; ++i)
+            if (f.dst[i] && n) memcpy(f.dst[i], src + h->out_off[i], n * f.bytes[i]);
+        memcpy(counters, src + h->out_off[kNumOut], sizeof(counters));
         h->stats.d2h_bytes = (int64_t)h->out_bytes;
     } else {
-        for (int i = 0; i < 13; ++i)
-            if (dsts[i] && bytes[i]) {
-                CU_TRY(h, cudaMemcpyAsync(dsts[i], dbase + h->out_off[i], bytes[i], cudaMemcpyDeviceToHost, h->stream));
-                h->stats.d2h_bytes += (int64_t)bytes[i];
+        for (int i = 0; i < kNumOut; ++i)
+            if (f.dst[i] && n) {
+                CU_TRY(h, cudaMemcpyAsync(f.dst[i], dbase + h->out_off[i], n * f.bytes[i], cudaMemcpyDeviceToHost, h->stream));
+                h->stats.d2h_bytes += (int64_t)(n * f.bytes[i]);
             }
-        CU_TRY(h, cudaMemcpyAsync(counters, dbase + h->out_off[13], sizeof(counters), cudaMemcpyDeviceToHost, h->stream));
+        CU_TRY(h, cudaMemcpyAsync(counters, dbase + h->out_off[kNumOut], sizeof(counters), cudaMemcpyDeviceToHost, h->stream));
         CU_TRY(h, cudaEventRecord(h->ev[5], h->stream));
         CU_TRY(h, cudaStreamSynchronize(h->stream));
     }
     h->timing_pending_d2h = true;
-    h->stats.total_pops = (int64_t)counters[0];
-    h->stats.total_nodes = (int64_t)counters[1];
-    h->stats.total_obstacle_cols = (int64_t)counters[2];
-    if (counters[3]) h->stats.handed_over = (int32_t)counters[3];   // shape 5: searches re-run with the exact queue
-    h->stats.escalated = (int32_t)counters[6];
-#ifdef PDMPC_PROFILE
-    {
-#ifdef PDMPC_PROFILE_CHECKER
-        static const char *names[8] = {"c:wait_job", "c:tables+place", "c:interx_obstacles", "c:interx_rest", "c:sincos+publish", "-", "-", "c:other"};
-#else
-        static const char *names[8] = {"setup", "heap_pop", "loads+place", "check", "expand", "heap_push", "wait_children", "loop"};
-        // (CTA kernel master: set-up, pending children, loads + heap pop, flag wait, job hand-over, children, pushes, end)
-#endif
-        double tot = 0;
-        for (int i = 0; i < 8; ++i) tot += (double)counters[8 + i];
-        fprintf(stderr, "[pdmpc profile] cycles per pop:");
-        for (int i = 0; i < 8; ++i)
-            fprintf(stderr, " %s=%.0f", names[i], (double)counters[8 + i] / (double)std::max<unsigned long long>(counters[0], 1));
-        fprintf(stderr, " total=%.0f\n", tot / (double)std::max<unsigned long long>(counters[0], 1));
-        if (counters[5])
-            fprintf(stderr, "[pdmpc profile] checker 0: %.0f cycles per job over %llu jobs\n",
-                    (double)counters[4] / (double)counters[5], counters[5]);
-    }
-#endif
+    read_counters(h, counters);
     return PDMPC_OK;
 }
 
 // Output rows of the escalated searches, packed (pipeline: their slices went to the host before the CTA
 // kernels wrote them).  One warp per item; row = the 13 output fields of one search, each padded to 8 bytes.
 struct PackDesc {
-    const unsigned char *src[13];
-    int bytes[13], off[13];
+    const unsigned char *src[kNumOut];
+    int bytes[kNumOut], off[kNumOut];
     int row_bytes;
 };
 __global__ void pack_rows_kernel(PackDesc d, const unsigned *count, const int *list, unsigned char *rows) {
@@ -1086,7 +1124,7 @@ __global__ void pack_rows_kernel(PackDesc d, const unsigned *count, const int *l
     for (unsigned j = blockIdx.x * (blockDim.x / 32) + threadIdx.x / 32; j < n; j += gridDim.x * (blockDim.x / 32)) {
         const size_t si = (size_t)list[j];
         unsigned char *row = rows + (size_t)j * d.row_bytes;
-        for (int f = 0; f < 13; ++f) {
+        for (int f = 0; f < kNumOut; ++f) {
             if (!d.src[f]) continue;
             const unsigned char *s = d.src[f] + si * (size_t)d.bytes[f];
             for (int q = lane; q < d.bytes[f]; q += 32) row[d.off[f] + q] = s[q];
@@ -1168,10 +1206,9 @@ static int plan_batch_pipelined(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc
     if (!out || !out->status) return fail(h, PDMPC_ERR_BAD_INPUT, "fetch: out/status is NULL");
     CU_TRY(h, cudaSetDevice(h->device));
     const int n = in->n_searches, Hp = h->mpa.Hp;
-    const std::vector<int> bnd = pipeline_bounds(n, C_req);
+    const std::vector<int> bnd = pipeline_bounds(n, C_req);   // chunk c covers the searches [bnd[c], bnd[c + 1])
     const int C = (int)bnd.size() - 1;
-    const size_t ns = (size_t)n * (Hp + 1);
-    const int np = in->slot_ptr[ns];
+    const int np = in->slot_ptr[(size_t)n * (Hp + 1)];
     if (np < 0 || (np > 0 && (!in->vert_x || !in->vert_y)))
         return fail(h, PDMPC_ERR_BAD_INPUT, "plan: malformed obstacle CSR");
     const int nv = np ? in->poly_ptr[np] : 0, nl = in->lane_ptr[2 * n];
@@ -1191,69 +1228,38 @@ static int plan_batch_pipelined(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc
         h->ev_chunk.push_back(e);
     }
     // ---- device arrays for the whole batch ----------------------------------------------------
-    struct Arr { DBuf *buf; const void *src; size_t elem; };
-    Arr arr[15] = {{&h->b_x0, in->x0, 8}, {&h->b_y0, in->y0, 8}, {&h->b_yaw0, in->yaw0, 8}, {&h->b_trim0, in->trim0, 4},
-                   {&h->b_refx, in->ref_x, 8}, {&h->b_refy, in->ref_y, 8}, {&h->b_vref, in->v_ref, 8},
-                   {&h->b_slot, in->slot_ptr, 4}, {&h->b_poly, in->poly_ptr, 4}, {&h->b_vx, in->vert_x, 8},
-                   {&h->b_vy, in->vert_y, 8}, {&h->b_lane, in->lane_ptr, 4}, {&h->b_lx, in->lane_x, 8},
-                   {&h->b_ly, in->lane_y, 8}, {&h->b_order, nullptr, 4}};
-    const size_t total[15] = {(size_t)n, (size_t)n, (size_t)n, (size_t)n, (size_t)n * Hp, (size_t)n * Hp, (size_t)n * Hp,
-                              ns + 1, (size_t)np + 1, (size_t)nv, (size_t)nv, (size_t)2 * n + 1, (size_t)nl, (size_t)nl,
-                              (size_t)n};
-    for (int i = 0; i < 15; ++i) CU_TRY(h, arr[i].buf->reserve(std::max<size_t>(total[i], 1) * arr[i].elem));
-    if (interx) {
-        CU_TRY(h, h->b_plx.reserve(((size_t)nv + np + 1) * sizeof(double)));
-        CU_TRY(h, h->b_ply.reserve(((size_t)nv + np + 1) * sizeof(double)));
-        CU_TRY(h, h->b_llx.reserve(((size_t)nl + 2 * n + 1) * sizeof(double)));
-        CU_TRY(h, h->b_lly.reserve(((size_t)nl + 2 * n + 1) * sizeof(double)));
-        CU_TRY(h, h->b_plxy.reserve(((size_t)nv + np + 1) * sizeof(double2)));
-        CU_TRY(h, h->b_llxy.reserve(((size_t)nl + 2 * n + 1) * sizeof(double2)));
+    const InRange all = in_range(Hp, 0, n, 0, np, 0, nv, 0, nl);
+    const void *dptr[kNumIn];
+    for (int i = 0; i < kNumIn; ++i) {
+        CU_TRY(h, h->b_in[i].reserve(std::max<size_t>(all.hi[i], 1) * kInElem[i]));
+        dptr[i] = h->b_in[i].p;
     }
+    BatchDev &b = h->batch;
+    set_batch(b, n, in->checker, in->dt_seconds, dptr);
+    rc = reserve_polylines(h, np, nv, nl);
+    if (rc != PDMPC_OK) return rc;
     rc = ensure_outputs(h, n);
     if (rc != PDMPC_OK) return rc;
-    rc = ensure_pinned(h, &h->pin_order, &h->pin_order_cap, (size_t)n * sizeof(int));
+    rc = ensure_pinned(h, h->pin_order, (size_t)n * sizeof(int));
     if (rc != PDMPC_OK) return rc;
     CU_TRY(h, h->wc_chunks.reserve(kPipelineMaxChunks * sizeof(unsigned)));
     // one-warp CTAs leave an SM one by one as their searches end, so the next chunk's CTAs move in early
     constexpr int kLanes = 8;   // most concurrent chunk kernels (streams, arenas)
-    auto bound = [&](int c) -> int { return bnd[c]; };   // chunk c covers the searches [bound(c), bound(c + 1))
     int per_chunk = 1;
-    for (int c = 0; c < C; ++c) per_chunk = std::max(per_chunk, bound(c + 1) - bound(c));
+    for (int c = 0; c < C; ++c) per_chunk = std::max(per_chunk, bnd[c + 1] - bnd[c]);
     const int shape = resolve_warp_shape(h, h->variant_mode, per_chunk, in->checker, false);
     int slots = 0;
     warp_shape_grid(h, shape, per_chunk, &slots);
     int lanes = std::min(C, kLanes);
     {   // node arenas of all lanes within 32 GiB
-        const int cap = std::max(64, std::min(h->user_node_cap ? h->user_node_cap : std::min(h->full_tree_nodes + 8, 1 << 20),
-                                              kMaxNodeCap - 1));
-        const double per_lane = (double)slots * cap * (sizeof(NodeA) + sizeof(NodeB) + sizeof(NodeCS) + sizeof(HEnt));
+        const double per_lane = (double)slots * node_cap(h) * (sizeof(NodeA) + sizeof(NodeB) + sizeof(NodeCS) + sizeof(HEnt));
         lanes = std::max(2, std::min(lanes, (int)(32.0 * 1024 * 1024 * 1024 / per_lane)));
     }
-    h->batch.checker = in->checker;
     const bool esc = escalation_on(h, shape, n);
     rc = ensure_arena(h, esc ? lanes * slots + h->num_sms * kCtaMasters : lanes * slots);
     if (rc != PDMPC_OK) return rc;
-    ArenaDev ar[kLanes];
     cudaStream_t comp[kLanes] = {h->stream, h->s_comp[0], h->s_comp[1], h->s_comp[2],
                                  h->s_comp[3], h->s_comp[4], h->s_comp[5], h->s_comp[6]};
-    for (int i = 0; i < lanes; ++i) {
-        const size_t off = (size_t)i * (size_t)slots * (size_t)h->arena.cap;
-        ar[i] = h->arena;
-        ar[i].a += off; ar[i].b += off; ar[i].cs += off; ar[i].heap += off;
-    }
-    BatchDev &b = h->batch;
-    b.n = n; b.checker = in->checker; b.dt = in->dt_seconds;
-    b.x0 = h->b_x0.as<double>(); b.y0 = h->b_y0.as<double>(); b.yaw0 = h->b_yaw0.as<double>();
-    b.trim0 = h->b_trim0.as<int>();
-    b.ref_x = h->b_refx.as<double>(); b.ref_y = h->b_refy.as<double>(); b.v_ref = h->b_vref.as<double>();
-    b.slot_ptr = h->b_slot.as<int>(); b.poly_ptr = h->b_poly.as<int>();
-    b.vert_x = h->b_vx.as<double>(); b.vert_y = h->b_vy.as<double>();
-    b.lane_ptr = h->b_lane.as<int>(); b.lane_x = h->b_lx.as<double>(); b.lane_y = h->b_ly.as<double>();
-    b.order = h->b_order.as<int>();
-    b.pl_x = interx ? h->b_plx.as<double>() : nullptr; b.pl_y = interx ? h->b_ply.as<double>() : nullptr;
-    b.ll_x = interx ? h->b_llx.as<double>() : nullptr; b.ll_y = interx ? h->b_lly.as<double>() : nullptr;
-    b.pl_xy = interx ? h->b_plxy.as<double2>() : nullptr; b.ll_xy = interx ? h->b_llxy.as<double2>() : nullptr;
-    h->n_polys = np; h->n_verts = nv; h->n_lane = nl;
     h->stats.h2d_bytes = 0;
     h->stats.d2h_bytes = 0;
     h->stats.kernel_launches = 0;
@@ -1264,13 +1270,13 @@ static int plan_batch_pipelined(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc
     b.pop_limit = 0; b.esc_list = nullptr; b.esc_count = nullptr; b.esc_done = nullptr; b.esc_producers = 0;
     BatchDev bproto = b;     // what the chunk kernels see: + the escalation list
 
-    CU_TRY(h, cudaMemsetAsync(h->out.counters, 0, 16 * sizeof(unsigned long long), h->stream));
+    CU_TRY(h, cudaMemsetAsync(h->out.counters, 0, kCounterBytes, h->stream));
     CU_TRY(h, cudaMemsetAsync(h->wc_chunks.p, 0, kPipelineMaxChunks * sizeof(unsigned), h->stream));
     CU_TRY(h, cudaMemsetAsync(h->work_counter.p, 0, 4 * sizeof(unsigned), h->stream));
     if (esc) {
         rc = escalation_prepare(h, n, &bproto, h->stream);
         if (rc != PDMPC_OK) return rc;
-        rc = ensure_pinned(h, &h->pin_esc, &h->pin_esc_cap, 4096);
+        rc = ensure_pinned(h, h->pin_esc, 4096);
         if (rc != PDMPC_OK) return rc;
     }
     CU_TRY(h, cudaEventRecord(h->ev_fork, h->stream));
@@ -1280,17 +1286,11 @@ static int plan_batch_pipelined(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc
     CU_TRY(h, cudaEventRecord(h->ev[2], h->stream));
     bool d2h_started = false;
     int esc_producers = 0;   // tile CTAs launched: the escalation kernel ends when all of them have
-    int *pin_order = static_cast<int *>(h->pin_order);
+    int *pin_order = h->pin_order.as<int>();
+    const void *srcs[kNumIn];
+    in_sources(in, pin_order, srcs);
+    const OutFields f = out_fields(Hp, out);
     const TraceDev tr{-1, nullptr, 0, nullptr};
-    void *dsts[13] = {out->status, out->is_exhausted, out->n_expanded, out->n_pops, out->pop_hash, out->trims,
-                      out->tree_path, out->y_predicted, out->g_path, out->h_path, out->shape_npts, out->shape_x,
-                      out->shape_y};
-    const size_t per_search[13] = {sizeof(int), 1, sizeof(int), sizeof(int), sizeof(uint64_t),
-                                   ((size_t)Hp + 1) * sizeof(int), ((size_t)Hp + 1) * sizeof(int),
-                                   (size_t)Hp * 3 * sizeof(double), ((size_t)Hp + 1) * sizeof(double),
-                                   ((size_t)Hp + 1) * sizeof(double), (size_t)Hp * sizeof(int),
-                                   (size_t)Hp * PDMPC_AREA_STRIDE * sizeof(double),
-                                   (size_t)Hp * PDMPC_AREA_STRIDE * sizeof(double)};
     const unsigned char *dbase = h->d_out_pack.as<unsigned char>();
     auto bail = [&](int code) {
         pipeline_sync_all(h);
@@ -1300,41 +1300,22 @@ static int plan_batch_pipelined(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc
     h->chunk_host_ms.assign(C, 0.0);
     h->chunks_last = C;
     for (int c = 0; c < C; ++c) {
-        const int s0 = bound(c), s1 = bound(c + 1);
+        const int s0 = bnd[c], s1 = bnd[c + 1];
         if (s1 == s0) continue;
         const int p0 = in->slot_ptr[(size_t)s0 * (Hp + 1)], p1 = in->slot_ptr[(size_t)s1 * (Hp + 1)];
         const int v0 = in->poly_ptr[p0], v1 = in->poly_ptr[p1];
         const int l0 = in->lane_ptr[2 * s0], l1 = in->lane_ptr[2 * s1];
         if (p0 < 0 || p1 > np || p1 < p0 || v0 < 0 || v1 > nv || v1 < v0 || l0 < 0 || l1 > nl || l1 < l0)   // the arrays were sized from the totals
             return bail(fail(h, PDMPC_ERR_BAD_INPUT, "plan: CSR offsets exceed their totals"));
-        {   // work order inside the chunk: most obstacle polygons first (counting sort, stable)
-            int kmax = 0, kmin = 0;
-            for (int i = s0; i < s1; ++i) {
-                const int d = in->slot_ptr[(size_t)(i + 1) * (Hp + 1)] - in->slot_ptr[(size_t)i * (Hp + 1)];
-                kmax = std::max(kmax, d);
-                kmin = std::min(kmin, d);
-            }
-            if (kmin < 0) return bail(fail(h, PDMPC_ERR_BAD_INPUT, "plan: slot_ptr not monotone"));   // (validated in full below)
-            std::vector<int> cnt(kmax + 2, 0);
-            for (int i = s0; i < s1; ++i)
-                cnt[kmax - (in->slot_ptr[(size_t)(i + 1) * (Hp + 1)] - in->slot_ptr[(size_t)i * (Hp + 1)]) + 1]++;
-            for (int k = 0; k <= kmax; ++k) cnt[k + 1] += cnt[k];
-            for (int i = s0; i < s1; ++i)
-                pin_order[s0 + cnt[kmax - (in->slot_ptr[(size_t)(i + 1) * (Hp + 1)] - in->slot_ptr[(size_t)i * (Hp + 1)])]++] = i;
-        }
-        // slices [lo, hi) of every input array that belong to this chunk (offset arrays: one more entry)
-        const size_t lo[15] = {(size_t)s0, (size_t)s0, (size_t)s0, (size_t)s0, (size_t)s0 * Hp, (size_t)s0 * Hp, (size_t)s0 * Hp,
-                               (size_t)s0 * (Hp + 1), (size_t)p0, (size_t)v0, (size_t)v0, (size_t)2 * s0, (size_t)l0, (size_t)l0,
-                               (size_t)s0};
-        const size_t hi[15] = {(size_t)s1, (size_t)s1, (size_t)s1, (size_t)s1, (size_t)s1 * Hp, (size_t)s1 * Hp, (size_t)s1 * Hp,
-                               (size_t)s1 * (Hp + 1) + 1, (size_t)p1 + 1, (size_t)v1, (size_t)v1, (size_t)2 * s1 + 1, (size_t)l1,
-                               (size_t)l1, (size_t)s1};
-        for (int i = 0; i < 15; ++i) {
-            if (hi[i] <= lo[i]) continue;
-            const unsigned char *src = static_cast<const unsigned char *>(i == 14 ? (const void *)pin_order : arr[i].src);
-            const size_t bytes = (hi[i] - lo[i]) * arr[i].elem;
-            if (cudaMemcpyAsync(arr[i].buf->as<unsigned char>() + lo[i] * arr[i].elem, src + lo[i] * arr[i].elem, bytes,
-                                cudaMemcpyHostToDevice, h->s_in) != cudaSuccess)
+        if (!heavy_first_order(in->slot_ptr, Hp, s0, s1, pin_order + s0))
+            return bail(fail(h, PDMPC_ERR_BAD_INPUT, "plan: slot_ptr not monotone"));   // (validated in full below)
+        const InRange r = in_range(Hp, s0, s1, p0, p1, v0, v1, l0, l1);
+        for (int i = 0; i < kNumIn; ++i) {
+            if (r.hi[i] <= r.lo[i]) continue;
+            const size_t e = kInElem[i], bytes = (r.hi[i] - r.lo[i]) * e;
+            if (cudaMemcpyAsync(h->b_in[i].as<unsigned char>() + r.lo[i] * e,
+                                static_cast<const unsigned char *>(srcs[i]) + r.lo[i] * e, bytes, cudaMemcpyHostToDevice,
+                                h->s_in) != cudaSuccess)
                 return bail(fail(h, PDMPC_ERR_CUDA, std::string("pipeline H2D: ") + cudaGetErrorString(cudaGetLastError())));
             h->stats.h2d_bytes += (int64_t)bytes;
         }
@@ -1346,28 +1327,14 @@ static int plan_batch_pipelined(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc
         cudaStream_t S = comp[c % lanes];
         if (cudaEventRecord(ev_in, h->s_in) != cudaSuccess || cudaStreamWaitEvent(S, ev_in, 0) != cudaSuccess)
             return bail(fail(h, PDMPC_ERR_CUDA, "pipeline: event"));
-        if (interx) {
-            if (p1 > p0) {
-                build_polyline_kernel<<<(p1 - p0 + 127) / 128, 128, 0, S>>>(p1 - p0, b.poly_ptr, b.vert_x, b.vert_y,
-                                                                          h->b_plx.as<double>(), h->b_ply.as<double>(), p0,
-                                                                          h->b_plxy.as<double2>());
-                h->stats.kernel_launches++;
-            }
-            build_polyline_kernel<<<(2 * (s1 - s0) + 127) / 128, 128, 0, S>>>(2 * (s1 - s0), b.lane_ptr, b.lane_x, b.lane_y,
-                                                                          h->b_llx.as<double>(), h->b_lly.as<double>(), 2 * s0,
-                                                                          h->b_llxy.as<double2>());
-            h->stats.kernel_launches++;
-        }
+        if (interx) build_polylines(h, p0, p1, s0, s1, S);
         BatchDev bc = bproto;
         bc.n = s1 - s0;
-        bc.order = h->b_order.as<int>() + s0;
+        bc.order = b.order + s0;
         unsigned *wc = h->wc_chunks.as<unsigned>() + c;
-        if (launch_warp_shape(h, shape, bc, ar[c % lanes], wc, tr, S) != PDMPC_OK)
+        if (launch_warp_shape(h, shape, bc, arena_from(h->arena, (size_t)(c % lanes) * slots), wc, tr, S) != PDMPC_OK)
             return bail(PDMPC_ERR_CUDA);
-        {
-            int dummy = 0;
-            esc_producers += warp_shape_grid(h, shape, bc.n, &dummy);
-        }
+        esc_producers += warp_shape_grid(h, shape, bc.n);
         if (cudaGetLastError() != cudaSuccess || cudaEventRecord(ev_done, S) != cudaSuccess ||
             cudaStreamWaitEvent(h->s_out, ev_done, 0) != cudaSuccess)
             return bail(fail(h, PDMPC_ERR_CUDA, "pipeline: search kernel launch failed"));
@@ -1376,25 +1343,22 @@ static int plan_batch_pipelined(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc
             cudaEventRecord(h->ev[4], h->s_out);
             d2h_started = true;
         }
-        for (int i = 0; i < 13; ++i) {
-            if (!dsts[i]) continue;
-            const size_t o0 = (size_t)s0 * per_search[i], bytes = (size_t)(s1 - s0) * per_search[i];
-            if (cudaMemcpyAsync(static_cast<unsigned char *>(dsts[i]) + o0, dbase + h->out_off[i] + o0, bytes,
+        for (int i = 0; i < kNumOut; ++i) {
+            if (!f.dst[i]) continue;
+            const size_t o0 = (size_t)s0 * f.bytes[i], bytes = (size_t)(s1 - s0) * f.bytes[i];
+            if (cudaMemcpyAsync(static_cast<unsigned char *>(f.dst[i]) + o0, dbase + h->out_off[i] + o0, bytes,
                                 cudaMemcpyDeviceToHost, h->s_out) != cudaSuccess)
                 return bail(fail(h, PDMPC_ERR_CUDA, "pipeline D2H failed"));
             h->stats.d2h_bytes += (int64_t)bytes;
         }
     }
     for (int c = 0; c < C; ++c)   // every chunk joins the handle's stream
-        if (c % lanes != 0 && bound(c + 1) > bound(c))
+        if (c % lanes != 0 && bnd[c + 1] > bnd[c])
             CU_TRY(h, cudaStreamWaitEvent(h->stream, h->ev_chunk[2 * c + 1], 0));
     if (esc) {   // the searches the chunk kernels give up: CTA shape, all chunks' leftovers in one launch
-        ArenaDev ae = h->arena;
-        const size_t off = (size_t)lanes * (size_t)slots * (size_t)h->arena.cap;
-        ae.a += off; ae.b += off; ae.cs += off; ae.heap += off;
-        rc = launch_escalated(h, ae, esc_producers, h->stream);
+        rc = launch_escalated(h, arena_from(h->arena, (size_t)lanes * slots), esc_producers, h->stream);
         if (rc != PDMPC_OK) return bail(rc);
-        CU_TRY(h, cudaMemcpyAsync(h->pin_esc, h->esc.p, 4 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+        CU_TRY(h, cudaMemcpyAsync(h->pin_esc.p, h->esc.p, 4 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     }
     CU_TRY(h, cudaEventRecord(h->ev[1], h->s_in));
     CU_TRY(h, cudaEventRecord(h->ev[3], h->stream));
@@ -1403,48 +1367,44 @@ static int plan_batch_pipelined(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc
         CU_TRY(h, cudaStreamWaitEvent(h->s_out, h->ev_fork, 0));
     }
     unsigned long long counters[16] = {0};
-    CU_TRY(h, cudaMemcpyAsync(counters, dbase + h->out_off[13], sizeof(counters), cudaMemcpyDeviceToHost, h->s_out));
+    CU_TRY(h, cudaMemcpyAsync(counters, dbase + h->out_off[kNumOut], sizeof(counters), cudaMemcpyDeviceToHost, h->s_out));
     CU_TRY(h, cudaEventRecord(h->ev[5], h->s_out));
     rc = pipeline_sync_all(h);
     if (rc != PDMPC_OK) return rc;
-    if (esc && *static_cast<const unsigned *>(h->pin_esc) > 0) {
+    if (esc && *h->pin_esc.as<const unsigned>() > 0) {
         // their output rows: packed on the device, one copy, scattered into the caller's arrays
-        const unsigned cnt = *static_cast<const unsigned *>(h->pin_esc);
+        const unsigned cnt = *h->pin_esc.as<const unsigned>();
         PackDesc pd;
         int off = 0;
-        for (int i = 0; i < 13; ++i) {
-            pd.src[i] = dsts[i] ? dbase + h->out_off[i] : nullptr;
-            pd.bytes[i] = (int)per_search[i];
+        for (int i = 0; i < kNumOut; ++i) {
+            pd.src[i] = f.dst[i] ? dbase + h->out_off[i] : nullptr;
+            pd.bytes[i] = (int)f.bytes[i];
             pd.off[i] = off;
-            off += ((int)per_search[i] + 7) / 8 * 8;
+            off += ((int)f.bytes[i] + 7) / 8 * 8;
         }
         pd.row_bytes = off;
         const size_t list_bytes = ((size_t)cnt * sizeof(int) + 15) / 16 * 16;
         CU_TRY(h, h->esc_rows.reserve((size_t)cnt * off));
-        rc = ensure_pinned(h, &h->pin_esc, &h->pin_esc_cap, list_bytes + (size_t)cnt * off);
+        rc = ensure_pinned(h, h->pin_esc, list_bytes + (size_t)cnt * off);
         if (rc != PDMPC_OK) return rc;
         pack_rows_kernel<<<std::min<unsigned>((cnt + 3) / 4, 256u), 128, 0, h->stream>>>(
             pd, h->esc.as<unsigned>(), h->esc.as<int>() + 4, h->esc_rows.as<unsigned char>());
         CU_TRY(h, cudaGetLastError());
         h->stats.kernel_launches++;
-        unsigned char *pin = static_cast<unsigned char *>(h->pin_esc);
+        unsigned char *pin = h->pin_esc.as<unsigned char>();
         CU_TRY(h, cudaMemcpyAsync(pin, h->esc.as<int>() + 4, (size_t)cnt * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
         CU_TRY(h, cudaMemcpyAsync(pin + list_bytes, h->esc_rows.p, (size_t)cnt * off, cudaMemcpyDeviceToHost, h->stream));
         CU_TRY(h, cudaStreamSynchronize(h->stream));
         const int *list = reinterpret_cast<const int *>(pin);
         for (unsigned j = 0; j < cnt; ++j) {
             const unsigned char *row = pin + list_bytes + (size_t)j * off;
-            for (int i = 0; i < 13; ++i)
-                if (dsts[i]) memcpy(static_cast<unsigned char *>(dsts[i]) + (size_t)list[j] * per_search[i], row + pd.off[i], per_search[i]);
+            for (int i = 0; i < kNumOut; ++i)
+                if (f.dst[i]) memcpy(static_cast<unsigned char *>(f.dst[i]) + (size_t)list[j] * f.bytes[i], row + pd.off[i], f.bytes[i]);
         }
         h->stats.d2h_bytes += (int64_t)(list_bytes + (size_t)cnt * off);
     }
     h->timing_pending_h2d = h->timing_pending_kernel = h->timing_pending_d2h = true;
-    h->stats.total_pops = (int64_t)counters[0];
-    h->stats.total_nodes = (int64_t)counters[1];
-    h->stats.total_obstacle_cols = (int64_t)counters[2];
-    if (counters[3]) h->stats.handed_over = (int32_t)counters[3];
-    h->stats.escalated = (int32_t)counters[6];
+    read_counters(h, counters);
     h->staged = true;   // the device holds the whole batch: pdmpc_run_staged / pdmpc_fetch_staged work on it
     return PDMPC_OK;
 }
@@ -1486,7 +1446,7 @@ int pdmpc_set_pipeline_chunks(pdmpc_handle *h, int32_t chunks) {
 }
 
 int pdmpc_plan_batch(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc_batch_out *out) {
-    if (h && in && h->has_mpa && h->pipeline_chunks != 1 && h->variant_mode <= 3 &&
+    if (h && in && h->has_mpa && h->pipeline_chunks != 1 && h->variant_mode < kShapeCta &&
         (h->pipeline_chunks > 1 ? in->n_searches >= 2 * h->pipeline_chunks : in->n_searches >= kPipelineMinSearches)) {
         return plan_batch_pipelined(h, in, out, h->pipeline_chunks > 1 ? h->pipeline_chunks : 0);
     }
@@ -1500,16 +1460,11 @@ int pdmpc_plan_batch(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc_batch_out 
 // One whole time step (or many) as ONE dependency-ordered launch: see include/pdmpc_b200.h.
 // slot / standstill != NULL: the closed-loop variant — fallback plans come from (and final plans go to) the state on
 // the device (pdmpc_fallback.cuh); deps->fb_* are then ignored.
-// `dev` != NULL: the batch is in device memory already (pdmpc_plan_timestep_from_states: dev->dptr = its fourteen arrays
-// in the order of pdmpc_stage_batch, totals = polygons, vertices, lanelet points); `in` then only carries n_searches,
-// checker and dt_seconds.
-struct DeviceBatch {
-    const void *dptr[14];
-    int np, nv, nl;
-};
+// `dev` != NULL: the batch is in device memory already (pdmpc_plan_timestep_from_states: its input arrays but the work
+// order, dev_totals = polygons, vertices, lanelet points); `in` then only carries n_searches, checker and dt_seconds.
 static int plan_timestep_impl(pdmpc_handle *h, const pdmpc_batch_in *in, const pdmpc_timestep_deps *deps,
                               pdmpc_batch_out *out, const int32_t *slot, const uint8_t *standstill,
-                              const DeviceBatch *dev = nullptr) {
+                              const void **dev = nullptr, const int *dev_totals = nullptr) {
     if (!h) return PDMPC_ERR_BAD_INPUT;
     if (!h->has_mpa) return fail(h, PDMPC_ERR_NO_MPA, "plan_timestep: call pdmpc_upload_mpa first");
     if (!in || !deps || !deps->pred_ptr) return fail(h, PDMPC_ERR_BAD_INPUT, "plan_timestep: NULL argument");
@@ -1519,10 +1474,9 @@ static int plan_timestep_impl(pdmpc_handle *h, const pdmpc_batch_in *in, const p
     // trees beyond what that kernel holds — one warp per search; pdmpc_set_variant 1..3 / 4..5 force either
     bool use_cta;
     {
-        const int cap = h->user_node_cap ? h->user_node_cap : std::min(h->full_tree_nodes + 8, 1 << 20);
-        const bool cta_possible = h->cta_deps_ok && cap <= kCtaFlags;
-        if (h->variant_mode >= 4) use_cta = cta_possible;
-        else if (h->variant_mode >= 1) use_cta = false;
+        const bool cta_possible = cta_launchable(h, true);
+        if (h->variant_mode >= kShapeCta) use_cta = cta_possible;
+        else if (h->variant_mode >= kShapeLatency) use_cta = false;
         // measured (profiles/r01h_closed_loop_sweep.txt): a time step is bound by its chains of dependent
         // searches, so the 2.5x lower per-pop latency of the CTA shape beats the 12x higher concurrency of the
         // warp shape up to several thousand searches per call
@@ -1581,14 +1535,12 @@ static int plan_timestep_impl(pdmpc_handle *h, const pdmpc_batch_in *in, const p
         h->staged = false;
         h->deps_staged = false;
         CU_TRY(h, cudaEventRecord(h->ev[0], h->stream));
-        UP(h, h->b_order, order.data(), n);      // the only array that still comes from the host
+        UP(h, h->b_in[kInOrder], order.data(), n);      // the only array that still comes from the host
         CU_TRY(h, cudaStreamSynchronize(h->stream));   // `order` is pageable
         CU_TRY(h, cudaEventRecord(h->ev[1], h->stream));
         h->timing_pending_h2d = true;
-        const void *dptr[15];
-        for (int i = 0; i < 14; ++i) dptr[i] = dev->dptr[i];
-        dptr[14] = h->b_order.p;
-        rc = stage_finish(h, n, in->checker, in->dt_seconds, dptr, dev->np, dev->nv, dev->nl);
+        dev[kInOrder] = h->b_in[kInOrder].p;
+        rc = stage_finish(h, n, in->checker, in->dt_seconds, dev, dev_totals[0], dev_totals[1], dev_totals[2]);
     } else {
         h->topo_order.swap(order);
         rc = pdmpc_stage_batch(h, in);
@@ -1612,11 +1564,11 @@ static int plan_timestep_impl(pdmpc_handle *h, const pdmpc_batch_in *in, const p
         off[i] = tot;
         tot = (tot + sz[i] + 15) / 16 * 16;
     }
-    rc = ensure_pinned(h, &h->pin_deps, &h->pin_deps_cap, tot);
+    rc = ensure_pinned(h, h->pin_deps, tot);
     if (rc != PDMPC_OK) return rc;
     CU_TRY(h, h->d_deps.reserve(tot));
     CU_TRY(h, h->d_done.reserve((size_t)n * sizeof(int)));
-    unsigned char *pin = static_cast<unsigned char *>(h->pin_deps);
+    unsigned char *pin = h->pin_deps.as<unsigned char>();
     for (int i = 0; i < 5; ++i)
         if (sz[i] && src[i]) memcpy(pin + off[i], src[i], i == 1 ? (size_t)total * sizeof(int) : sz[i]);
     CU_TRY(h, cudaMemcpyAsync(h->d_deps.p, pin, tot, cudaMemcpyHostToDevice, h->stream));
@@ -1651,7 +1603,7 @@ static int plan_timestep_impl(pdmpc_handle *h, const pdmpc_batch_in *in, const p
         dp.fb_npts = fbd.fb_npts; dp.fb_x = fbd.fb_x; dp.fb_y = fbd.fb_y;
     }
     // ---- one persistent launch: CTAs / warps take the searches in topological order ----------------
-    CU_TRY(h, cudaMemsetAsync(h->out.counters, 0, 16 * sizeof(unsigned long long), h->stream));
+    CU_TRY(h, cudaMemsetAsync(h->out.counters, 0, kCounterBytes, h->stream));
     CU_TRY(h, cudaMemsetAsync(h->work_counter.p, 0, sizeof(unsigned), h->stream));
     const bool cta_single = n <= h->num_sms;
     const int cta_nm = cta_single ? 1 : kCtaMastersDeps;
@@ -1664,9 +1616,9 @@ static int plan_timestep_impl(pdmpc_handle *h, const pdmpc_batch_in *in, const p
         CU_TRY(h, h->d_depn.reserve((size_t)grid * (kDepCols / kAreaStride) * sizeof(int)));
         dp.dep_x = h->d_depx.as<double>(); dp.dep_y = h->d_depy.as<double>(); dp.dep_n = h->d_depn.as<int>();
     }
-    const bool cta_fast = h->variant_mode == 5 || h->cta_valid_only;
+    const bool cta_fast = h->variant_mode == kShapeCtaValid || h->cta_valid_only;
     h->batch.hash_valid_only = h->cta_valid_only ? 1 : 0;   // one kind of pop_hash whatever shape runs
-    h->stats.shape = use_cta ? (cta_fast ? 5 : 4) : 1;
+    h->stats.shape = use_cta ? (cta_fast ? kShapeCtaValid : kShapeCta) : kShapeLatency;
     CU_TRY(h, cudaEventRecord(h->ev[2], h->stream));
     if (use_cta && cta_single)
         KERNEL_CTA_DEPS<<<grid, CtaShape<1, kCtaCheckers>::kThreads, sizeof(CtaDepsSmemT), h->stream>>>(
@@ -1785,25 +1737,22 @@ int pdmpc_plan_timestep_from_states(pdmpc_handle *h, const pdmpc_timestep_states
     const long long poly_cap = (long long)st->succ_ptr[n] + (long long)Hp * st->par_ptr[n];
     const long long vert_cap = 5LL * st->succ_ptr[n] + (long long)Hp * st->par_ptr[n] * std::max(h->reach_max_pts, 1);
     if (poly_cap > 0x3fffffff || vert_cap > 0x3fffffff) return fail(h, PDMPC_ERR_CAPACITY, "plan_timestep_from_states: too many obstacles");
-    int totals[2] = {0, 0}, nl = 0;
+    int totals[3] = {0, 0, 0};   // polygons, vertices, lanelet points
     rc = run_assemble_obstacles(h, &ci, (int)poly_cap, (int)vert_cap, totals);
     if (rc != PDMPC_OK) return rc;
-    CU_TRY(h, cudaMemcpyAsync(&nl, h->i_lptr.as<int>() + 2 * n, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CU_TRY(h, cudaMemcpyAsync(&totals[2], h->i_lptr.as<int>() + 2 * n, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CU_TRY(h, cudaStreamSynchronize(h->stream));
-    if (nl > lane_cap) return fail(h, PDMPC_ERR_CAPACITY, "plan_timestep_from_states: the lanelet bounds need more than 512 points per vehicle");
+    if (totals[2] > lane_cap) return fail(h, PDMPC_ERR_CAPACITY, "plan_timestep_from_states: the lanelet bounds need more than 512 points per vehicle");
     if (totals[0] > poly_cap || totals[1] > vert_cap) return fail(h, PDMPC_ERR_CAPACITY, "plan_timestep_from_states: obstacle capacity");
-    DeviceBatch dev;
-    const void *d[14] = {h->q_x.p, h->q_y.p, h->q_yaw.p, h->q_trim.p, h->i_refx.p, h->i_refy.p, h->i_vref.p,
-                         h->q_slot.p, h->q_poly.p, h->q_vx.p, h->q_vy.p, h->i_lptr.p, h->i_lx.p, h->i_ly.p};
-    for (int i = 0; i < 14; ++i) dev.dptr[i] = d[i];
-    dev.np = totals[0]; dev.nv = totals[1]; dev.nl = nl;
+    const void *dev[kNumIn] = {h->q_x.p,    h->q_y.p,  h->q_yaw.p, h->q_trim.p, h->i_refx.p, h->i_refy.p, h->i_vref.p, h->q_slot.p,
+                               h->q_poly.p, h->q_vx.p, h->q_vy.p,  h->i_lptr.p, h->i_lx.p,   h->i_ly.p,   nullptr};   // + the work order
     pdmpc_batch_in stub;
     memset(&stub, 0, sizeof(stub));
     stub.n_searches = n; stub.checker = st->checker; stub.dt_seconds = st->dt_seconds;
     pdmpc_timestep_deps deps;
     memset(&deps, 0, sizeof(deps));
     deps.pred_ptr = st->pred_ptr; deps.pred_idx = st->pred_idx;
-    return plan_timestep_impl(h, &stub, &deps, out, st->slot, still.data(), &dev);
+    return plan_timestep_impl(h, &stub, &deps, out, st->slot, still.data(), dev, totals);
 }
 
 // Centralized (joint) search: rows = searches x n_vehicles (pdmpc_joint.cuh).
@@ -1825,7 +1774,7 @@ int pdmpc_joint_plan_batch(pdmpc_handle *h, const pdmpc_batch_in *in, int32_t n_
             h->staged = false;
             return fail(h, PDMPC_ERR_BAD_INPUT, "joint: obstacle slots of rows other than a search's first row must be empty");
         }
-    CU_TRY(h, cudaMemsetAsync(h->out.counters, 0, 16 * sizeof(unsigned long long), h->stream));
+    CU_TRY(h, cudaMemsetAsync(h->out.counters, 0, kCounterBytes, h->stream));
     CU_TRY(h, cudaMemsetAsync(h->work_counter.p, 0, sizeof(unsigned), h->stream));
     h->stats.kernel_launches = 0;
     h->batch.hash_valid_only = h->cta_valid_only ? 1 : 0;
@@ -1853,7 +1802,7 @@ int pdmpc_joint_plan_batch(pdmpc_handle *h, const pdmpc_batch_in *in, int32_t n_
         CU_TRY(h, cudaEventRecord(h->ev[3], h->stream));
         h->timing_pending_kernel = true;
         h->stats.kernel_launches = 1;
-        h->stats.shape = 1;
+        h->stats.shape = kShapeLatency;
     }
     return pdmpc_fetch_staged(h, out);
 }
@@ -1869,7 +1818,7 @@ int pdmpc_mcts_run_staged(pdmpc_handle *h, const pdmpc_mcts_params *prm) {
     if (h->max_branch > PDMPC_MCTS_MAX_BRANCH)
         return fail(h, PDMPC_ERR_BAD_INPUT, "mcts: branching factor of the MPA exceeds PDMPC_MCTS_MAX_BRANCH");
     CU_TRY(h, cudaSetDevice(h->device));
-    CU_TRY(h, cudaMemsetAsync(h->out.counters, 0, 16 * sizeof(unsigned long long), h->stream));
+    CU_TRY(h, cudaMemsetAsync(h->out.counters, 0, kCounterBytes, h->stream));
     CU_TRY(h, cudaMemsetAsync(h->work_counter.p, 0, sizeof(unsigned), h->stream));
     h->stats.kernel_launches = 0;
     if (n == 0) return PDMPC_OK;

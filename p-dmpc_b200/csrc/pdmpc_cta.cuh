@@ -145,12 +145,11 @@ search_cta_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_co
     constexpr int kBarThreads = Shape::kBarThreads;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     CtaSmem<HS, SP, NC, NM, DEPS> &sm = *reinterpret_cast<CtaSmem<HS, SP, NC, NM, DEPS> *>(smem_raw);
-    Tables tb;
-    tb.succ_ptr = m.succ_ptr; tb.succ_te = m.succ_te; tb.edge_d = m.edge_d;
-    tb.area_npts = m.area_npts; tb.area_x = m.area_x; tb.area_y = m.area_y;
 
     const int warp_id = threadIdx.x / kWarp;
     const int lane = threadIdx.x % kWarp;
+    Tile<kWarp> t;
+    t.shift = 0; t.lane = lane; t.mask = FULL;
     const int Hp = m.Hp, nT = m.nT;
     volatile unsigned *vdone = sm.done;
     // work items: the batch — or, with b.esc_producers > 0, the escalation list of the tile kernel(s) (BatchDev;
@@ -197,17 +196,17 @@ search_cta_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_co
                 // consecutive expansions start at different checkers: with 3-4 children per expansion a fixed
                 // child -> checker map would serialise every job on checkers 0..3
                 for (int ci = (w - jb.rot + NC) % NC; ci < nchild; ci += NC) {
-                    const int te = tb.succ_te[sbase + ci];
+                    const int te = m.succ_te[sbase + ci];
                     const int edge = te >> 8;
                     const unsigned nid = nid0 + (unsigned)ci;
                     const int bkind = (cK == Hp) ? PDMPC_AREA_LARGE_OFFSET : PDMPC_AREA_WITHOUT_OFFSET;  // GraphSearch.m:166-174
-                    const int ns = tb.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
-                    const int nbs = tb.area_npts[edge * 3 + bkind];
+                    const int ns = m.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
+                    const int nbs = m.area_npts[edge * 3 + bkind];
                     // place both areas by the PARENT pose (GraphSearch.m:155-160); the tail repeats the last vertex
                     if (lane < 16) {
                         const int sel = lane >> 3, i = lane & 7;
                         const int ab = (edge * 3 + (sel ? bkind : PDMPC_AREA_NORMAL)) * kAreaStride + i;   // (padded by the last point)
-                        const double ax = tb.area_x[ab], ay = tb.area_y[ab];
+                        const double ax = m.area_x[ab], ay = m.area_y[ab];
                         sts_f64x2(sshp + 16u * (unsigned)lane, pc * ax - ps * ay + ppx, ps * ax + pc * ay + ppy);
                     }
                     __syncwarp();
@@ -291,8 +290,6 @@ search_cta_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_co
                             (lane < 8 ? sy : by)[lane & 7] = v.y;
                         }
                         __syncwarp();
-                        Tile<kWarp> t;
-                        t.shift = 0; t.lane = lane; t.mask = FULL;
                         const int *slot = S.slot;
                         const int dp0 = __ldg(slot + cK), dp1 = __ldg(slot + cK + 1);
                         for (int pass = 0; pass < 2 && valid; ++pass) {
@@ -328,7 +325,7 @@ search_cta_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_co
                             // cos/sin of the child's yaw for ITS expansion (expand_node.m:50-51);
                             // yaw' = yaw + dyaw exactly as the master computes it (:55)
                             NodeCS ecs;
-                            sincos_ref(pyaw + tb.edge_d[edge * 4 + 2], ecs.s, ecs.c);
+                            sincos_ref(pyaw + m.edge_d[edge * 4 + 2], ecs.s, ecs.c);
                             ncs[nid] = ecs;
                         }
                         fence_cta();
@@ -433,10 +430,7 @@ search_cta_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_co
             si = b.order ? __ldg(b.order + si_u) : (int)si_u;
         }
         for (int i = lane; i <= clear_upto / 16; i += kWarp) S.flag2[i] = 0u;
-        for (int k = lane; k < Hp; k += kWarp) {
-            S.refx[k] = __ldg(b.ref_x + (size_t)si * Hp + k);
-            S.refy[k] = __ldg(b.ref_y + (size_t)si * Hp + k);
-        }
+        stage_reference(b, si, Hp, S.refx, S.refy, nullptr, t);
         if (lane >= 1 && lane < Hp) {   // d_traveled_max of expand_node.m:68 for children of step k'
             double d = 0.0;
             for (int it = 1; it <= Hp - lane; ++it) {
@@ -460,15 +454,9 @@ search_cta_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_co
         if (b.checker == PDMPC_CHECKER_INTERX) {
             // polyline layout (vectorize_all_obstacles.m:27-63) as if everything were staged: lanelets
             // [left, NaN, right, NaN] at [0, nl), obstacle slot s at nl + rng[s]
-            const int sp0 = __ldg(slot + 0), spE = __ldg(slot + Hp + 1);
-            const int lp0 = __ldg(b.lane_ptr + 2 * si), lp2 = __ldg(b.lane_ptr + 2 * si + 2);
-            const int ob_lo = __ldg(b.poly_ptr + sp0) + sp0, ob_hi = __ldg(b.poly_ptr + spE) + spE;
-            const int ll_lo = lp0 + 2 * si, ll_hi = lp2 + 2 * si + 2;
-            const int nl = ll_hi - ll_lo, no = ob_hi - ob_lo;
-            for (int k = lane; k <= Hp + 1; k += kWarp) {
-                const int q = __ldg(slot + k);
-                S.rng[k] = __ldg(b.poly_ptr + q) + q - ob_lo;
-            }
+            const SearchPolylines pl = search_polylines(b, si, Hp, S.rng, t);
+            const int ll_lo = pl.ll_lo, ob_lo = pl.ob_lo;
+            const int nl = pl.ll_hi - ll_lo, no = pl.ob_hi - ob_lo;
             const bool lst = nl <= SP, ost = (lst ? nl : 0) + no <= SP;
             if (lst)
                 for (int j = lane; j < nl; j += kWarp)
@@ -485,40 +473,16 @@ search_cta_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_co
         }
         // (everything above is independent of the predecessors: it overlaps their searches)
         if (DEPS) {
-            // ---- consider_predecessors (PrioritizedController.m:449-506) on the device ------------
             // Work items are handed out in a topological order of the DAG (the host sorts them), so every
             // predecessor's ticket is below this one's: it is finished or running on another master, never
             // waiting behind this one.
-            const int q0 = __ldg(dp.pred_ptr + si), q1 = __ldg(dp.pred_ptr + si + 1);
-            const int npred = q1 - q0;
-            for (int r = lane; r < npred; r += kWarp) {
-                const int *flag = dp.done + __ldg(dp.pred_idx + q0 + r);
-                while (ld_acquire_gpu(flag) == 0) __nanosleep(100);
-            }
-            __syncwarp();
-            if (lane == 0) S.n_pred = npred;
-            const double qn = nan("");
-            for (int idx = lane; idx < npred * Hp * kAreaStride; idx += kWarp) {
-                const int v = idx % kAreaStride, pk = idx / kAreaStride;   // pk = (k - 1) * npred + r
-                const int r = pk % npred, k0 = pk / npred;
-                const int j = __ldg(dp.pred_idx + q0 + r);
-                const bool planned = ld_acquire_gpu(dp.done + j) == 1;
-                const size_t os = (size_t)j * Hp + k0;
-                int np = 0;
-                double vx = qn, vy = qn;
-                if (planned) {   // what j has just written: read from L2, never through the read-only path
-                    np = __ldcg(o.shape_npts + os);
-                    if (v < np) { vx = __ldcg(o.shape_x + os * kAreaStride + v); vy = __ldcg(o.shape_y + os * kAreaStride + v); }
-                } else if (dp.fb_npts) {
-                    np = __ldg(dp.fb_npts + os);
-                    if (v < np) { vx = __ldg(dp.fb_x + os * kAreaStride + v); vy = __ldg(dp.fb_y + os * kAreaStride + v); }
-                }
-                S.dep[idx] = make_double2(vx, vy);
-                if (v == 0) {
+            const int npred = gather_predecessor_areas(
+                dp, o, si, Hp, 100, t, [&](int idx, double x, double y) { S.dep[idx] = make_double2(x, y); },
+                [&](int pk, int k0, int np) {
                     S.dep_n[pk] = np;
                     if (np) atomicAdd(&S.dep_cols[k0 + 1], np + 1);
-                }
-            }
+                });
+            if (lane == 0) S.n_pred = npred;
         }
 
         HeapSplit heap;
@@ -527,7 +491,7 @@ search_cta_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_co
         heap.hs = min(heap_smem, HS);   // smaller values only exercise the arena overflow (tests)
         heap.len = 1;
         int n_nodes = 1, n_pops = 0, status = PDMPC_OK;
-        unsigned long long hash = 0xcbf29ce484222325ULL;
+        unsigned long long hash = kHashSeed;
         bool exhausted = false, tie = false;
         unsigned goal = 0, last_ticket = 0;
         bool any_job = false;
@@ -565,18 +529,7 @@ search_cta_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_co
                 __nanosleep(20);
             }
         };
-        if (lane == 0) {   // root: GraphSearch.m:34-46
-            NodeA ra;
-            ra.x = __ldg(b.x0 + si); ra.y = __ldg(b.y0 + si); ra.yaw = __ldg(b.yaw0 + si); ra.g = 0.0;
-            NodeCS rcs;
-            sincos_ref(ra.yaw, rcs.s, rcs.c);
-            NodeB rb;
-            rb.h = 0.0; rb.parent = 0; rb.edge = 0xffff; rb.trim = (unsigned char)trim0; rb.k = 0;
-            na[1] = ra; nb[1] = rb; ncs[1] = rcs;
-            HEnt re;
-            re.f = 0.0; re.w = HEnt::pack(1u, 0u, 0u, 0u, (unsigned)trim0);
-            heap.st(0, re);
-        }
+        if (lane == 0) heap.st(0, init_root(b, si, trim0, na, nb, ncs));
         __threadfence_block();
         __syncwarp();
 
@@ -598,8 +551,8 @@ search_cta_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_co
             double2 cs0 = __ldcg(reinterpret_cast<const double2 *>(ncs + id0));
             int sbase = 0, nchild = 0;
             if (k0 < Hp) {
-                sbase = tb.succ_ptr[k0 * nT + (tr0 - 1)];
-                nchild = tb.succ_ptr[k0 * nT + (tr0 - 1) + 1] - sbase;
+                sbase = m.succ_ptr[k0 * nT + (tr0 - 1)];
+                nchild = m.succ_ptr[k0 * nT + (tr0 - 1) + 1] - sbase;
             }
             const HEnt top = heap.pop<true>(lane);
             PROF_MARK(2);   // early loads + heap pop
@@ -637,10 +590,10 @@ search_cta_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_co
                 he.f = 0.0; he.w = 0;
                 const unsigned nid = (unsigned)(n_nodes + 1 + ci);
                 if (ci < nchild) {
-                    const int te = tb.succ_te[sbase + ci];
+                    const int te = m.succ_te[sbase + ci];
                     const int cedge = te >> 8, t2 = (te & 0xff) + 1;
-                    const double mdx = tb.edge_d[cedge * 4 + 0], mdy = tb.edge_d[cedge * 4 + 1],
-                                 mdyaw = tb.edge_d[cedge * 4 + 2];
+                    const double mdx = m.edge_d[cedge * 4 + 0], mdy = m.edge_d[cedge * 4 + 1],
+                                 mdyaw = m.edge_d[cedge * 4 + 2];
                     NodeA ea;
                     ea.x = c * mdx - s * mdy + ca.x;          // :53
                     ea.y = s * mdx + c * mdy + ca.y;          // :54
@@ -734,69 +687,9 @@ search_cta_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_co
             redo_exact = true;
             continue;
         }
-        if (lane == 0) {
-            unsigned cur = goal;
-            for (int d = Hp; d >= 0; --d) {           // Tree.m:44-52 path_to_root, flipped
-                S.path[d] = exhausted ? 0u : cur;
-                if (!exhausted && d > 0) cur = nb[cur].parent;
-            }
-            o.status[si] = status;
-            if (o.is_exhausted) o.is_exhausted[si] = exhausted ? 1 : 0;
-            if (o.n_expanded) o.n_expanded[si] = n_nodes;
-            if (o.n_pops) o.n_pops[si] = n_pops;
-            if (o.pop_hash) o.pop_hash[si] = hash;
-            atomicAdd(o.counters + 0, (unsigned long long)n_pops);
-            atomicAdd(o.counters + 1, (unsigned long long)n_nodes);
-        }
-        __syncwarp();
-        const double qnan = nan("");
-        for (int d = lane; d <= Hp; d += kWarp) {
-            const unsigned pid = S.path[d];
-            NodeA pa = {qnan, qnan, qnan, qnan};
-            NodeB pb;
-            pb.h = qnan; pb.parent = 0; pb.edge = 0; pb.trim = 0; pb.k = 0;
-            if (!exhausted) { pa = na[pid]; pb = nb[pid]; }
-            const size_t oo = (size_t)si * (Hp + 1) + d;
-            if (o.trims) o.trims[oo] = exhausted ? (d == 0 ? trim0 : 0) : (int)pb.trim;
-            if (o.tree_path) o.tree_path[oo] = (int)pid;
-            if (o.g_path) o.g_path[oo] = pa.g;
-            if (o.h_path) o.h_path[oo] = pb.h;
-            if (d >= 1) {
-                const size_t os = (size_t)si * Hp + (d - 1);
-                if (o.y_predicted) {                   // return_path_to.m:11-25
-                    o.y_predicted[os * 3 + 0] = pa.x;
-                    o.y_predicted[os * 3 + 1] = pa.y;
-                    o.y_predicted[os * 3 + 2] = pa.yaw;
-                }
-                if (o.shape_npts) {                    // return_path_area.m:5-7
-                    int edge = 0, ns = 0;
-                    NodeA qa = {0.0, 0.0, 0.0, 0.0};
-                    double2 qcs = make_double2(0.0, 0.0);
-                    if (!exhausted) {
-                        const unsigned qid = S.path[d - 1];   // parent on the path (valid, depth < Hp)
-                        qa = na[qid];
-                        qcs = __ldcg(reinterpret_cast<const double2 *>(ncs + qid));
-                        edge = pb.edge;
-                        ns = tb.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
-                    }
-                    o.shape_npts[os] = ns;
-                    if (o.shape_x && o.shape_y) {
-                        for (int i = 0; i < kAreaStride; ++i) {
-                            double ox = 0.0, oy = 0.0;
-                            if (i < ns) place_point(tb, edge, PDMPC_AREA_NORMAL, i, qcs.x, qcs.y, qa.x, qa.y, ox, oy);
-                            o.shape_x[os * kAreaStride + i] = ox;
-                            o.shape_y[os * kAreaStride + i] = oy;
-                        }
-                    }
-                }
-            }
-        }
-        if (DEPS) {   // publish_predictions (PrioritizedController.m:355-364): the areas above are final
-            __threadfence();
-            __syncwarp();
-            if (lane == 0) st_release_gpu(dp.done + si, exhausted ? 2 : 1);
-        }
-        __syncwarp();
+        // (the checkers count the obstacle columns)
+        write_search_result(m, o, na, nb, ncs, S.path, si, trim0, goal, status, exhausted, n_nodes, n_pops, hash, 0ull,
+                            true, DEPS ? dp.done : nullptr, t);
     }
     // ---- the last master to run out of work releases the checkers -----------------------------------------
     unsigned fin = 0;

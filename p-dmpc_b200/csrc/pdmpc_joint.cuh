@@ -63,9 +63,6 @@ __global__ void __launch_bounds__(kWarp) joint_search_kernel(MpaDev m, BatchDev 
     constexpr int TILE = kWarp;
     extern __shared__ __align__(16) unsigned char joint_smem_raw[];
     JointSmem &sm = *reinterpret_cast<JointSmem *>(joint_smem_raw);
-    Tables tb;
-    tb.succ_ptr = m.succ_ptr; tb.succ_te = m.succ_te; tb.edge_d = m.edge_d;
-    tb.area_npts = m.area_npts; tb.area_x = m.area_x; tb.area_y = m.area_y;
     Tile<TILE> t;
     t.shift = 0; t.lane = threadIdx.x; t.mask = 0xffffffffu;
     const int Hp = m.Hp, nT = m.nT, nV = ar.nV;
@@ -109,7 +106,7 @@ __global__ void __launch_bounds__(kWarp) joint_search_kernel(MpaDev m, BatchDev 
         heap.len = 1;
         const int *slot = b.slot_ptr + (size_t)r0 * (Hp + 1);
         int n_nodes = 1, n_pops = 0, status = PDMPC_OK;
-        unsigned long long hash = 0xcbf29ce484222325ULL, cols = 0;
+        unsigned long long hash = kHashSeed, cols = 0;
         bool exhausted = false;
         unsigned goal = 0;
         __threadfence_block();
@@ -134,16 +131,16 @@ __global__ void __launch_bounds__(kWarp) joint_search_kernel(MpaDev m, BatchDev 
                     if (pv_i < nV) {
                         const JVeh pv = nv[(size_t)par * nV + pv_i];
                         const int edge = (int)nv[(size_t)id * nV + pv_i].edge;
-                        place_point(tb, edge, PDMPC_AREA_NORMAL, pt_i, pv.c, pv.s, pv.x, pv.y, sm.shx[pv_i][pt_i], sm.shy[pv_i][pt_i]);
-                        place_point(tb, edge, bkind, pt_i, pv.c, pv.s, pv.x, pv.y, sm.bhx[pv_i][pt_i], sm.bhy[pv_i][pt_i]);
+                        place_point(m, edge, PDMPC_AREA_NORMAL, pt_i, pv.c, pv.s, pv.x, pv.y, sm.shx[pv_i][pt_i], sm.shy[pv_i][pt_i]);
+                        place_point(m, edge, bkind, pt_i, pv.c, pv.s, pv.x, pv.y, sm.bhx[pv_i][pt_i], sm.bhy[pv_i][pt_i]);
                         if (pt_i == 0) sm.edge_of[pv_i] = edge;
                     }
                     t.sync();
                 }
                 for (int v = 0; v < nV && valid; ++v) {
                     const int edge = sm.edge_of[v];
-                    const int ns = tb.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
-                    const int nbs = tb.area_npts[edge * 3 + bkind];
+                    const int ns = m.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
+                    const int nbs = m.area_npts[edge * 3 + bkind];
                     // are_constraints_satisfied_sat.m:15-35: static obstacles, dynamic obstacles of this step
                     for (int pass = 0; pass < 2 && valid; ++pass) {
                         const int q0 = pass == 0 ? sp0 : dp0, q1 = pass == 0 ? sp1 : dp1;
@@ -156,7 +153,7 @@ __global__ void __launch_bounds__(kWarp) joint_search_kernel(MpaDev m, BatchDev 
                     // :37-44 vehicles of the same node with a lower index
                     for (int u = v - 1; u >= 0 && valid; --u) {
                         const int eu = sm.edge_of[u];
-                        const int nsu = tb.area_npts[eu * 3 + PDMPC_AREA_NORMAL];
+                        const int nsu = m.area_npts[eu * 3 + PDMPC_AREA_NORMAL];
                         cols += (unsigned long long)nsu;
                         if (sat_collide<TILE, false>(sm.shx[u], sm.shy[u], nsu, sm.shx[v], sm.shy[v], ns, t)) valid = false;
                     }
@@ -182,8 +179,8 @@ __global__ void __launch_bounds__(kWarp) joint_search_kernel(MpaDev m, BatchDev 
             for (int v = 0; v < kMaxJoint; ++v) {
                 if (v < nV) {
                     cv[v] = nv[(size_t)id * nV + v];
-                    sbase[v] = tb.succ_ptr[(k_exp - 1) * nT + ((int)cv[v].trim - 1)];
-                    nsucc[v] = tb.succ_ptr[(k_exp - 1) * nT + ((int)cv[v].trim - 1) + 1] - sbase[v];
+                    sbase[v] = m.succ_ptr[(k_exp - 1) * nT + ((int)cv[v].trim - 1)];
+                    nsucc[v] = m.succ_ptr[(k_exp - 1) * nT + ((int)cv[v].trim - 1) + 1] - sbase[v];
                     total *= nsucc[v];
                 }
             }
@@ -203,9 +200,9 @@ __global__ void __launch_bounds__(kWarp) joint_search_kernel(MpaDev m, BatchDev 
                         if (v < nV) {
                             const int iv = (int)(rem % nsucc[v]);   // cartprod: first vehicle fastest
                             rem /= nsucc[v];
-                            const int te = tb.succ_te[sbase[v] + iv];
+                            const int te = m.succ_te[sbase[v] + iv];
                             const int cedge = te >> 8, t2 = (te & 0xff) + 1;
-                            const double mdx = tb.edge_d[cedge * 4 + 0], mdy = tb.edge_d[cedge * 4 + 1], mdyaw = tb.edge_d[cedge * 4 + 2];
+                            const double mdx = m.edge_d[cedge * 4 + 0], mdy = m.edge_d[cedge * 4 + 1], mdyaw = m.edge_d[cedge * 4 + 2];
                             JVeh ev;
                             ev.x = cv[v].c * mdx - cv[v].s * mdy + cv[v].x;      // :53
                             ev.y = cv[v].s * mdx + cv[v].c * mdy + cv[v].y;      // :54
@@ -284,12 +281,12 @@ __global__ void __launch_bounds__(kWarp) joint_search_kernel(MpaDev m, BatchDev 
                     if (!exhausted) {
                         qv = nv[(size_t)sm.path[d - 1] * nV + v];
                         edge = (int)pv.edge;
-                        ns = tb.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
+                        ns = m.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
                     }
                     o.shape_npts[os] = ns;
                     for (int i = 0; i < kAreaStride; ++i) {
                         double ox = 0.0, oy = 0.0;
-                        if (i < ns) place_point(tb, edge, PDMPC_AREA_NORMAL, i, qv.c, qv.s, qv.x, qv.y, ox, oy);
+                        if (i < ns) place_point(m, edge, PDMPC_AREA_NORMAL, i, qv.c, qv.s, qv.x, qv.y, ox, oy);
                         o.shape_x[os * kAreaStride + i] = ox;
                         o.shape_y[os * kAreaStride + i] = oy;
                     }

@@ -34,6 +34,9 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <cstddef>
+#include <type_traits>
+
 #include "../../include/pdmpc_b200.h"
 
 // Optional per-phase cycle accounting (build with -DPDMPC_PROFILE; profiling builds only)
@@ -419,23 +422,194 @@ __device__ __forceinline__ bool lanelet_side_sat(const double *sx, const double 
 }
 
 // FNV-1a over the popped ids taken as 32-bit words (parity trace of the pop order)
+constexpr unsigned long long kHashSeed = 0xcbf29ce484222325ULL;
 __device__ __forceinline__ unsigned long long hash_step(unsigned long long h, unsigned v) {
     return (h ^ (unsigned long long)v) * 0x100000001b3ULL;
 }
 
-// Table pointers as seen by the kernel body (shared-memory copies or the global arrays).
-struct Tables {
-    const int *succ_ptr, *succ_te, *area_npts;
-    const double *edge_d, *area_x, *area_y;
-};
-
 // Rotate/translate one maneuver area point: GraphSearch.m:158-159.
-__device__ __forceinline__ void place_point(const Tables &tb, int edge, int kind, int i, double c, double s,
+__device__ __forceinline__ void place_point(const MpaDev &m, int edge, int kind, int i, double c, double s,
                                             double px, double py, double &ox, double &oy) {
     const int base = (edge * 3 + kind) * kAreaStride + i;
-    const double ax = tb.area_x[base], ay = tb.area_y[base];
+    const double ax = m.area_x[base], ay = m.area_y[base];
     ox = c * ax - s * ay + px;
     oy = s * ax + c * ay + py;
+}
+
+// ---- per-search pieces every launch shape shares ------------------------------------------------------------
+// Each is called by the TILE lanes that own the search, outside the pop loop.
+
+// Root of search si (GraphSearch.m:34-46): writes node 1 and returns the first heap entry for the caller to store.
+__device__ __forceinline__ HEnt init_root(const BatchDev &b, int si, int trim0, NodeA *na, NodeB *nb, NodeCS *ncs) {
+    NodeA ra;
+    ra.x = __ldg(b.x0 + si); ra.y = __ldg(b.y0 + si); ra.yaw = __ldg(b.yaw0 + si); ra.g = 0.0;
+    NodeCS rcs;
+    sincos_ref(ra.yaw, rcs.s, rcs.c);
+    NodeB rb;
+    rb.h = 0.0; rb.parent = 0; rb.edge = 0xffff; rb.trim = (unsigned char)trim0; rb.k = 0;
+    na[1] = ra; nb[1] = rb; ncs[1] = rcs;
+    HEnt re;
+    re.f = 0.0; re.w = HEnt::pack(1u, 0u, 0u, 0u, (unsigned)trim0);
+    return re;
+}
+
+// Reference trajectory of search si into shared memory, and its speeds unless vref is nullptr (a shape that
+// keeps running sums of them instead).
+template <int TILE, class VRef>
+__device__ __forceinline__ void stage_reference(const BatchDev &b, int si, int Hp, double *refx, double *refy,
+                                                VRef vref, const Tile<TILE> &t) {
+    for (int k = t.lane; k < Hp; k += TILE) {
+        refx[k] = __ldg(b.ref_x + (size_t)si * Hp + k);
+        refy[k] = __ldg(b.ref_y + (size_t)si * Hp + k);
+        if constexpr (!std::is_same<VRef, std::nullptr_t>::value) vref[k] = __ldg(b.v_ref + (size_t)si * Hp + k);
+    }
+}
+
+// Polyline layout of search si (vectorize_all_obstacles.m:27-63): obstacle slot s covers
+// [ob_lo + rng[s], ob_lo + rng[s+1]), the lanelet bounds [left, NaN, right, NaN] cover [ll_lo, ll_hi).
+// Fills rng[0..Hp+1]; staging the points is the caller's (each shape has its own layout).
+struct SearchPolylines {
+    int ob_lo, ob_hi, ll_lo, ll_hi;
+};
+template <int TILE>
+__device__ __forceinline__ SearchPolylines search_polylines(const BatchDev &b, int si, int Hp, int *rng,
+                                                            const Tile<TILE> &t) {
+    const int *slot = b.slot_ptr + (size_t)si * (Hp + 1);
+    const int sp0 = __ldg(slot + 0), spE = __ldg(slot + Hp + 1);
+    const int lp0 = __ldg(b.lane_ptr + 2 * si), lp2 = __ldg(b.lane_ptr + 2 * si + 2);
+    SearchPolylines p;
+    p.ob_lo = __ldg(b.poly_ptr + sp0) + sp0; p.ob_hi = __ldg(b.poly_ptr + spE) + spE;
+    p.ll_lo = lp0 + 2 * si; p.ll_hi = lp2 + 2 * si + 2;
+    for (int k = t.lane; k <= Hp + 1; k += TILE) {
+        const int q = __ldg(slot + k);
+        rng[k] = __ldg(b.poly_ptr + q) + q - p.ob_lo;
+    }
+    return p;
+}
+
+// consider_predecessors (PrioritizedController.m:449-506) on the device.  Waits until every predecessor of search
+// si is done, then hands each column of their areas to put_pt(idx, x, y) and each area's point count to
+// put_n(pk, k0, np): predecessor r at step k0 + 1 is area pk = k0 * n_pred + r, its columns are
+// [pk * kAreaStride, (pk + 1) * kAreaStride), points first, then NaN.  A planned predecessor's areas were written
+// during this launch and are read through L2; an exhausted one's are its fallback areas.  Returns n_pred.
+template <int TILE, class PutPt, class PutN>
+__device__ __forceinline__ int gather_predecessor_areas(const DepsDev &dp, const OutDev &o, int si, int Hp,
+                                                        unsigned nap_ns, const Tile<TILE> &t, PutPt put_pt,
+                                                        PutN put_n) {
+    const int q0 = __ldg(dp.pred_ptr + si);
+    const int n_pred = __ldg(dp.pred_ptr + si + 1) - q0;
+    for (int r = t.lane; r < n_pred; r += TILE) {
+        const int *flag = dp.done + __ldg(dp.pred_idx + q0 + r);
+        while (ld_acquire_gpu(flag) == 0) __nanosleep(nap_ns);
+    }
+    t.sync();
+    const double qn = nan("");
+    for (int idx = t.lane; idx < n_pred * Hp * kAreaStride; idx += TILE) {
+        const int v = idx % kAreaStride, pk = idx / kAreaStride;
+        const int r = pk % n_pred, k0 = pk / n_pred;
+        const int j = __ldg(dp.pred_idx + q0 + r);
+        const bool planned = ld_acquire_gpu(dp.done + j) == 1;
+        const size_t os = (size_t)j * Hp + k0;
+        int np = 0;
+        double vx = qn, vy = qn;
+        if (planned) {
+            np = __ldcg(o.shape_npts + os);
+            if (v < np) { vx = __ldcg(o.shape_x + os * kAreaStride + v); vy = __ldcg(o.shape_y + os * kAreaStride + v); }
+        } else if (dp.fb_npts) {
+            np = __ldg(dp.fb_npts + os);
+            if (v < np) { vx = __ldg(dp.fb_x + os * kAreaStride + v); vy = __ldg(dp.fb_y + os * kAreaStride + v); }
+        }
+        put_pt(idx, vx, vy);
+        if (v == 0) put_n(pk, k0, np);
+    }
+    return n_pred;
+}
+
+// Results of one search: GraphSearch.m:58-60 / :82-89.  A search that failed takes the "no plan" defaults of an
+// exhausted one.  path is the caller's shared scratch of Hp + 1 ids.  cols is added to the obstacle-column
+// counter when non-zero (a shape whose checkers count them passes 0).  cs_l2 reads the nodes' cos/sin through L2:
+// the CTA shape needs it (its checker warps write them).  A warp that wrote them itself may use either; the choice
+// is the one that keeps its pop loop as compiled before (with an L2 read in the one-search-per-warp kernel ptxas can
+// no longer prove the warp converged at the pop loop's collectives, and its DEPS instance needs the L2 read to stay
+// at 166 registers).  With `done` set (time-step dependencies), done[si] is released once the areas are written:
+// publish_predictions, PrioritizedController.m:355-364.
+template <int TILE>
+__device__ __forceinline__ void write_search_result(const MpaDev &m, const OutDev &o, const NodeA *na, const NodeB *nb,
+                                                    const NodeCS *ncs, unsigned *path, int si, int trim0,
+                                                    unsigned goal, int status, bool exhausted, int n_nodes,
+                                                    int n_pops, unsigned long long hash, unsigned long long cols,
+                                                    bool cs_l2, int *done, const Tile<TILE> &t) {
+    const int Hp = m.Hp;
+    if (status != PDMPC_OK) exhausted = true;
+    t.sync();
+    if (t.lane == 0) {
+        unsigned cur = goal;
+        for (int d = Hp; d >= 0; --d) {           // Tree.m:44-52 path_to_root, flipped
+            path[d] = exhausted ? 0u : cur;
+            if (!exhausted && d > 0) cur = nb[cur].parent;
+        }
+        o.status[si] = status;
+        if (o.is_exhausted) o.is_exhausted[si] = exhausted ? 1 : 0;
+        if (o.n_expanded) o.n_expanded[si] = n_nodes;
+        if (o.n_pops) o.n_pops[si] = n_pops;
+        if (o.pop_hash) o.pop_hash[si] = hash;
+        atomicAdd(o.counters + 0, (unsigned long long)n_pops);
+        atomicAdd(o.counters + 1, (unsigned long long)n_nodes);
+        if (cols) atomicAdd(o.counters + 2, cols);
+    }
+    t.sync();
+    const double qnan = nan("");
+    for (int d = t.lane; d <= Hp; d += TILE) {
+        const unsigned pid = path[d];
+        NodeA pa = {qnan, qnan, qnan, qnan};
+        NodeB pb;
+        pb.h = qnan; pb.parent = 0; pb.edge = 0; pb.trim = 0; pb.k = 0;
+        if (!exhausted) { pa = na[pid]; pb = nb[pid]; }
+        const size_t oo = (size_t)si * (Hp + 1) + d;
+        if (o.trims) o.trims[oo] = exhausted ? (d == 0 ? trim0 : 0) : (int)pb.trim;
+        if (o.tree_path) o.tree_path[oo] = (int)pid;
+        if (o.g_path) o.g_path[oo] = pa.g;
+        if (o.h_path) o.h_path[oo] = pb.h;
+        if (d >= 1) {
+            const size_t os = (size_t)si * Hp + (d - 1);
+            if (o.y_predicted) {                   // return_path_to.m:11-25
+                o.y_predicted[os * 3 + 0] = pa.x;
+                o.y_predicted[os * 3 + 1] = pa.y;
+                o.y_predicted[os * 3 + 2] = pa.yaw;
+            }
+            if (o.shape_npts) {                    // return_path_area.m:5-7
+                int edge = 0, ns = 0;
+                NodeA qa = {0.0, 0.0, 0.0, 0.0};
+                NodeCS qcs = {0.0, 0.0};
+                if (!exhausted) {
+                    const unsigned qid = path[d - 1];   // parent on the path (was expanded)
+                    qa = na[qid];
+                    if (cs_l2) {
+                        const double2 v = __ldcg(reinterpret_cast<const double2 *>(ncs + qid));
+                        qcs.c = v.x; qcs.s = v.y;
+                    } else {
+                        qcs = ncs[qid];
+                    }
+                    edge = pb.edge;
+                    ns = m.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
+                }
+                o.shape_npts[os] = ns;
+                if (o.shape_x && o.shape_y) {
+                    for (int i = 0; i < kAreaStride; ++i) {
+                        double ox = 0.0, oy = 0.0;
+                        if (i < ns) place_point(m, edge, PDMPC_AREA_NORMAL, i, qcs.c, qcs.s, qa.x, qa.y, ox, oy);
+                        o.shape_x[os * kAreaStride + i] = ox;
+                        o.shape_y[os * kAreaStride + i] = oy;
+                    }
+                }
+            }
+        }
+    }
+    if (done) {   // the areas above are final
+        __threadfence();
+        t.sync();
+        if (t.lane == 0) st_release_gpu(done + si, exhausted ? 2 : 1);
+    }
 }
 
 template <int HS, int SP>
@@ -472,12 +646,8 @@ __global__ void __launch_bounds__(kWarp, PDMPC_MIN_CTAS_LAT) search_kernel(MpaDe
     constexpr int WARPS = 1;
     const unsigned n_work = (unsigned)b.n;
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    Tables tb;
-    unsigned char *warp_base = smem_raw;
-    tb.succ_ptr = m.succ_ptr; tb.succ_te = m.succ_te; tb.edge_d = m.edge_d;
-    tb.area_npts = m.area_npts; tb.area_x = m.area_x; tb.area_y = m.area_y;
     const int warp_id = threadIdx.x / kWarp;
-    TileSmem<HS, SP> &sm = reinterpret_cast<TileSmem<HS, SP> *>(warp_base)[warp_id];
+    TileSmem<HS, SP> &sm = reinterpret_cast<TileSmem<HS, SP> *>(smem_raw)[warp_id];
 
     Tile<TILE> t;
     t.shift = 0;
@@ -525,72 +695,8 @@ __global__ void __launch_bounds__(kWarp, PDMPC_MIN_CTAS_LAT) search_kernel(MpaDe
         PROF_MARK(7);
         if (phase == DONE) {
             PROF_FLUSH(o, t.lane == 0);
-            // ---- results: GraphSearch.m:58-60 / :82-89 --------------------------
-            t.sync();
-            if (status != PDMPC_OK) exhausted = true;   // outputs take the "no plan" defaults
-            if (t.lane == 0) {
-                unsigned cur = goal;
-                for (int d = Hp; d >= 0; --d) {           // Tree.m:44-52 path_to_root, flipped
-                    sm.path[d] = exhausted ? 0u : cur;
-                    if (!exhausted && d > 0) cur = nb[cur].parent;
-                }
-                o.status[si] = status;
-                if (o.is_exhausted) o.is_exhausted[si] = exhausted ? 1 : 0;
-                if (o.n_expanded) o.n_expanded[si] = n_nodes;
-                if (o.n_pops) o.n_pops[si] = n_pops;
-                if (o.pop_hash) o.pop_hash[si] = hash;
-                atomicAdd(o.counters + 0, (unsigned long long)n_pops);
-                atomicAdd(o.counters + 1, (unsigned long long)n_nodes);
-                atomicAdd(o.counters + 2, cols);
-            }
-            t.sync();
-            const double qnan = nan("");
-            for (int d = t.lane; d <= Hp; d += TILE) {
-                const unsigned pid = sm.path[d];
-                NodeA pa = {qnan, qnan, qnan, qnan};
-                NodeB pb;
-                pb.h = qnan; pb.parent = 0; pb.edge = 0; pb.trim = 0; pb.k = 0;
-                if (!exhausted) { pa = na[pid]; pb = nb[pid]; }
-                const size_t oo = (size_t)si * (Hp + 1) + d;
-                if (o.trims) o.trims[oo] = exhausted ? (d == 0 ? trim0 : 0) : (int)pb.trim;
-                if (o.tree_path) o.tree_path[oo] = (int)pid;
-                if (o.g_path) o.g_path[oo] = pa.g;
-                if (o.h_path) o.h_path[oo] = pb.h;
-                if (d >= 1) {
-                    const size_t os = (size_t)si * Hp + (d - 1);
-                    if (o.y_predicted) {                   // return_path_to.m:11-25
-                        o.y_predicted[os * 3 + 0] = pa.x;
-                        o.y_predicted[os * 3 + 1] = pa.y;
-                        o.y_predicted[os * 3 + 2] = pa.yaw;
-                    }
-                    if (o.shape_npts) {                    // return_path_area.m:5-7
-                        int edge = 0, ns = 0;
-                        NodeA qa = {0.0, 0.0, 0.0, 0.0};
-                        NodeCS qcs = {0.0, 0.0};
-                        if (!exhausted) {
-                            const unsigned qid = sm.path[d - 1];   // parent on the path (was expanded)
-                            qa = na[qid];
-                            qcs = ncs[qid];
-                            edge = pb.edge;
-                            ns = tb.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
-                        }
-                        o.shape_npts[os] = ns;
-                        if (o.shape_x && o.shape_y) {
-                            for (int i = 0; i < kAreaStride; ++i) {
-                                double ox = 0.0, oy = 0.0;
-                                if (i < ns) place_point(tb, edge, PDMPC_AREA_NORMAL, i, qcs.c, qcs.s, qa.x, qa.y, ox, oy);
-                                o.shape_x[os * kAreaStride + i] = ox;
-                                o.shape_y[os * kAreaStride + i] = oy;
-                            }
-                        }
-                    }
-                }
-            }
-            if (DEPS) {   // publish_predictions (PrioritizedController.m:355-364): the areas above are final
-                __threadfence();
-                t.sync();
-                if (t.lane == 0) st_release_gpu(dp.done + si, exhausted ? 2 : 1);
-            }
+            write_search_result(m, o, na, nb, ncs, sm.path, si, trim0, goal, status, exhausted, n_nodes, n_pops, hash,
+                                cols, DEPS, DEPS ? dp.done : nullptr, t);
             phase = IDLE;
         }
         if (phase == IDLE) {
@@ -601,33 +707,10 @@ __global__ void __launch_bounds__(kWarp, PDMPC_MIN_CTAS_LAT) search_kernel(MpaDe
             si = b.order ? __ldg(b.order + si_u) : (int)si_u;
             // ---- per-search set-up ------------------------------------------------
             t.sync();
-            if (DEPS) {   // consider_predecessors (PrioritizedController.m:449-506) on the device
-                const int q0 = __ldg(dp.pred_ptr + si);
-                n_pred = __ldg(dp.pred_ptr + si + 1) - q0;
-                for (int r = t.lane; r < n_pred; r += TILE) {
-                    const int *flag = dp.done + __ldg(dp.pred_idx + q0 + r);
-                    while (ld_acquire_gpu(flag) == 0) __nanosleep(200);
-                }
-                t.sync();
-                const double qn = nan("");
-                for (int idx = t.lane; idx < n_pred * Hp * kAreaStride; idx += TILE) {
-                    const int v = idx % kAreaStride, pk = idx / kAreaStride;   // pk = (k - 1) * n_pred + r
-                    const int r = pk % n_pred, k0 = pk / n_pred;
-                    const int j = __ldg(dp.pred_idx + q0 + r);
-                    const bool planned = ld_acquire_gpu(dp.done + j) == 1;
-                    const size_t os = (size_t)j * Hp + k0;
-                    int np = 0;
-                    double vx = qn, vy = qn;
-                    if (planned) {   // written during this launch: L2, never the read-only path
-                        np = __ldcg(o.shape_npts + os);
-                        if (v < np) { vx = __ldcg(o.shape_x + os * kAreaStride + v); vy = __ldcg(o.shape_y + os * kAreaStride + v); }
-                    } else if (dp.fb_npts) {
-                        np = __ldg(dp.fb_npts + os);
-                        if (v < np) { vx = __ldg(dp.fb_x + os * kAreaStride + v); vy = __ldg(dp.fb_y + os * kAreaStride + v); }
-                    }
-                    dpx[idx] = vx; dpy[idx] = vy;
-                    if (v == 0) dpn[pk] = np;
-                }
+            if (DEPS) {
+                n_pred = gather_predecessor_areas(
+                    dp, o, si, Hp, 200, t, [=](int idx, double x, double y) { dpx[idx] = x; dpy[idx] = y; },
+                    [=](int pk, int, int np) { dpn[pk] = np; });
                 __threadfence_block();
                 t.sync();
                 my_dep_cols = 0;
@@ -637,66 +720,41 @@ __global__ void __launch_bounds__(kWarp, PDMPC_MIN_CTAS_LAT) search_kernel(MpaDe
                         if (np) my_dep_cols += np + 1;
                     }
             }
-            for (int k = t.lane; k < Hp; k += TILE) {
-                sm.refx[k] = __ldg(b.ref_x + (size_t)si * Hp + k);
-                sm.refy[k] = __ldg(b.ref_y + (size_t)si * Hp + k);
-                sm.vref[k] = __ldg(b.v_ref + (size_t)si * Hp + k);
-            }
+            stage_reference(b, si, Hp, sm.refx, sm.refy, sm.vref, t);
             slot = b.slot_ptr + (size_t)si * (Hp + 1);
             trim0 = __ldg(b.trim0 + si);
             for (int k = t.lane; k < kParentCache; k += TILE) sm.pc_id[k] = 0u;
-            if (t.lane == 0) {   // root: GraphSearch.m:34-46
-                NodeA ra;
-                ra.x = __ldg(b.x0 + si); ra.y = __ldg(b.y0 + si); ra.yaw = __ldg(b.yaw0 + si); ra.g = 0.0;
-                NodeCS rcs;
-                sincos_ref(ra.yaw, rcs.s, rcs.c);
-                ncs[1] = rcs;
-                NodeB rb;
-                rb.h = 0.0; rb.parent = 0; rb.edge = 0xffff; rb.trim = (unsigned char)trim0; rb.k = 0;
-                na[1] = ra;
-                nb[1] = rb;
-                HEnt re;
-                re.f = 0.0; re.w = HEnt::pack(1u, 0u, 0u, 0u, (unsigned)trim0);
-                heap.st(0, re);
-            }
+            if (t.lane == 0) heap.st(0, init_root(b, si, trim0, na, nb, ncs));
             heap.len = 1;
             sp0 = __ldg(slot + 0); sp1 = __ldg(slot + 1);
             lp0 = __ldg(b.lane_ptr + 2 * si); lp1 = __ldg(b.lane_ptr + 2 * si + 1);
             lp2 = __ldg(b.lane_ptr + 2 * si + 2);
             if (b.checker == PDMPC_CHECKER_INTERX) {
-                // polyline layout (vectorize_all_obstacles.m): obstacle slot s of this search
-                // covers [ob_lo + rng[s], ob_lo + rng[s+1]); lanelets [ll_lo, ll_hi)
-                const int spE = __ldg(slot + Hp + 1);
-                const int ob_lo = __ldg(b.poly_ptr + sp0) + sp0, ob_hi = __ldg(b.poly_ptr + spE) + spE;
-                const int ll_lo = lp0 + 2 * si, ll_hi = lp2 + 2 * si + 2;
-                for (int k = t.lane; k <= Hp + 1; k += TILE) {
-                    const int q = __ldg(slot + k);
-                    sm.rng[k] = __ldg(b.poly_ptr + q) + q - ob_lo;
-                }
-                const int nl = ll_hi - ll_lo, no = ob_hi - ob_lo;
+                const SearchPolylines pl = search_polylines(b, si, Hp, sm.rng, t);
+                const int nl = pl.ll_hi - pl.ll_lo, no = pl.ob_hi - pl.ob_lo;
                 int used = 0;
                 if (nl <= SP) {      // stage the lanelet polyline
                     for (int j = t.lane; j < nl; j += TILE) {
-                        sm.pts_x[j] = __ldg(b.ll_x + ll_lo + j);
-                        sm.pts_y[j] = __ldg(b.ll_y + ll_lo + j);
+                        sm.pts_x[j] = __ldg(b.ll_x + pl.ll_lo + j);
+                        sm.pts_y[j] = __ldg(b.ll_y + pl.ll_lo + j);
                     }
                     lpx = sm.pts_x; lpy = sm.pts_y; llo = 0; lhi = nl;
                     used = nl;
                 } else {
-                    lpx = b.ll_x; lpy = b.ll_y; llo = ll_lo; lhi = ll_hi;
+                    lpx = b.ll_x; lpy = b.ll_y; llo = pl.ll_lo; lhi = pl.ll_hi;
                 }
                 if (used + no <= SP) {   // stage the obstacle polylines of all steps
                     for (int j = t.lane; j < no; j += TILE) {
-                        sm.pts_x[used + j] = __ldg(b.pl_x + ob_lo + j);
-                        sm.pts_y[used + j] = __ldg(b.pl_y + ob_lo + j);
+                        sm.pts_x[used + j] = __ldg(b.pl_x + pl.ob_lo + j);
+                        sm.pts_y[used + j] = __ldg(b.pl_y + pl.ob_lo + j);
                     }
                     opx = sm.pts_x; opy = sm.pts_y; obase = used;
                 } else {
-                    opx = b.pl_x; opy = b.pl_y; obase = ob_lo;
+                    opx = b.pl_x; opy = b.pl_y; obase = pl.ob_lo;
                 }
             }
             n_nodes = 1; n_pops = 0;
-            hash = 0xcbf29ce484222325ULL; cols = 0;
+            hash = kHashSeed; cols = 0;
             status = PDMPC_OK;
             exhausted = false;
             goal = 0;
@@ -728,8 +786,8 @@ __global__ void __launch_bounds__(kWarp, PDMPC_MIN_CTAS_LAT) search_kernel(MpaDe
         const int k_exp = cK + 1;
         int sbase = 0, nchild = 0;
         if (cK < Hp) {
-            sbase = tb.succ_ptr[(k_exp - 1) * nT + (ctrim - 1)];
-            nchild = tb.succ_ptr[(k_exp - 1) * nT + (ctrim - 1) + 1] - sbase;
+            sbase = m.succ_ptr[(k_exp - 1) * nT + (ctrim - 1)];
+            nchild = m.succ_ptr[(k_exp - 1) * nT + (ctrim - 1) + 1] - sbase;
         }
         bool valid = true;
         if (par != 0) {   // eval_edge_exact :137-192 (root is valid unchecked)
@@ -746,15 +804,15 @@ __global__ void __launch_bounds__(kWarp, PDMPC_MIN_CTAS_LAT) search_kernel(MpaDe
             }
             const int edge = (int)top.edge();
             const int bkind = (cK == Hp) ? PDMPC_AREA_LARGE_OFFSET : PDMPC_AREA_WITHOUT_OFFSET;  // :166-174
-            const int ns = tb.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
-            const int nbs = tb.area_npts[edge * 3 + bkind];
+            const int ns = m.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
+            const int nbs = m.area_npts[edge * 3 + bkind];
             // (no barrier needed before the writes: the vote that ended the previous edge check
             // ordered all lanes' reads of the shape arrays)
             // all 8 (zero padded) points of both areas are placed; only the first ns / nbs are used
             if (t.lane < 8)
-                place_point(tb, edge, PDMPC_AREA_NORMAL, t.lane, pc, ps, ppx, ppy, sm.shx[t.lane], sm.shy[t.lane]);
+                place_point(m, edge, PDMPC_AREA_NORMAL, t.lane, pc, ps, ppx, ppy, sm.shx[t.lane], sm.shy[t.lane]);
             else if (t.lane < 16)
-                place_point(tb, edge, bkind, t.lane - 8, pc, ps, ppx, ppy, sm.bhx[t.lane - 8], sm.bhy[t.lane - 8]);
+                place_point(m, edge, bkind, t.lane - 8, pc, ps, ppx, ppy, sm.bhx[t.lane - 8], sm.bhy[t.lane - 8]);
             t.sync();
             PROF_MARK(2);   // record loads + shape placement
 
@@ -824,10 +882,10 @@ __global__ void __launch_bounds__(kWarp, PDMPC_MIN_CTAS_LAT) search_kernel(MpaDe
             he.f = 0.0; he.w = 0;
             const unsigned nid = (unsigned)(n_nodes + 1 + ci);
             if (ci < nchild) {
-                const int te = tb.succ_te[sbase + ci];
+                const int te = m.succ_te[sbase + ci];
                 const int cedge = te >> 8, t2 = (te & 0xff) + 1;
-                const double mdx = tb.edge_d[cedge * 4 + 0], mdy = tb.edge_d[cedge * 4 + 1],
-                             mdyaw = tb.edge_d[cedge * 4 + 2];
+                const double mdx = m.edge_d[cedge * 4 + 0], mdy = m.edge_d[cedge * 4 + 1],
+                             mdyaw = m.edge_d[cedge * 4 + 2];
                 NodeA ea;
                 ea.x = c * mdx - s * mdy + ca.x;          // :53
                 ea.y = s * mdx + c * mdy + ca.y;          // :54

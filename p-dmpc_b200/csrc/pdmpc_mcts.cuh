@@ -115,9 +115,6 @@ __global__ void __launch_bounds__(kWarp) mcts_kernel(MpaDev m, BatchDev b, OutDe
 
     Tile<kWarp> t;
     t.shift = 0; t.lane = lane; t.mask = 0xffffffffu;
-    Tables tb;
-    tb.succ_ptr = m.succ_ptr; tb.succ_te = m.succ_te; tb.edge_d = m.edge_d;
-    tb.area_npts = m.area_npts; tb.area_x = m.area_x; tb.area_y = m.area_y;
     const int Hp = m.Hp, nT = m.nT;
     const int n_rand = Hp * mc.n_max;
 
@@ -192,14 +189,14 @@ __global__ void __launch_bounds__(kWarp) mcts_kernel(MpaDev m, BatchDev b, OutDe
             npar[1] = 0; nedge[1] = 0xffff; ntrim[1] = (unsigned char)trim0;
         }
         if (lane < kMctsBranch) {
-            const int nroot = tb.succ_ptr[(trim0 - 1) + 1] - tb.succ_ptr[trim0 - 1];   // successor_trims{trim, 1}
+            const int nroot = m.succ_ptr[(trim0 - 1) + 1] - m.succ_ptr[trim0 - 1];   // successor_trims{trim, 1}
             children[1 * kMctsBranch + lane] = lane < nroot ? 1 : 0;
         }
         __syncwarp();
 
         int n_nodes = 1, n_exp = 0, n_trav = 0, status = PDMPC_OK;
         bool finished = false;
-        unsigned long long hash = 0xcbf29ce484222325ULL, cols = 0;
+        unsigned long long hash = kHashSeed, cols = 0;
         double best_f = 0.0;
         int best_id = 0;
 
@@ -248,17 +245,17 @@ __global__ void __launch_bounds__(kWarp) mcts_kernel(MpaDev m, BatchDev b, OutDe
                 ++n_exp;                                                // :146
                 node_parent = node;
                 const int ptrim = ntrim[node];
-                const int sbase = tb.succ_ptr[(step - 1) * nT + (ptrim - 1)];
-                const int te = tb.succ_te[sbase + pos];
+                const int sbase = m.succ_ptr[(step - 1) * nT + (ptrim - 1)];
+                const int te = m.succ_te[sbase + pos];
                 const int edge = te >> 8, gtrim = (te & 0xff) + 1;
                 const double px = nx[node], py = ny[node], pyaw = nyaw[node], c = ncos[node], s = nsin[node];
                 const int bkind = (step == Hp) ? PDMPC_AREA_LARGE_OFFSET : PDMPC_AREA_WITHOUT_OFFSET;   // :153-159
-                const int ns = tb.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
-                const int nbs = tb.area_npts[edge * 3 + bkind];
+                const int ns = m.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
+                const int nbs = m.area_npts[edge * 3 + bkind];
                 if (lane < 8)
-                    place_point(tb, edge, PDMPC_AREA_NORMAL, lane, c, s, px, py, shx[lane], shy[lane]);
+                    place_point(m, edge, PDMPC_AREA_NORMAL, lane, c, s, px, py, shx[lane], shy[lane]);
                 else if (lane < 16)
-                    place_point(tb, edge, bkind, lane - 8, c, s, px, py, bhx[lane - 8], bhy[lane - 8]);
+                    place_point(m, edge, bkind, lane - 8, c, s, px, py, bhx[lane - 8], bhy[lane - 8]);
                 __syncwarp();
                 valid = true;
                 if (b.checker == PDMPC_CHECKER_INTERX) {
@@ -299,13 +296,13 @@ __global__ void __launch_bounds__(kWarp) mcts_kernel(MpaDev m, BatchDev b, OutDe
                 const int id = n_nodes;
                 int nsucc = 0;
                 if (step < Hp) {
-                    const int sb2 = tb.succ_ptr[step * nT + (gtrim - 1)];
-                    nsucc = tb.succ_ptr[step * nT + (gtrim - 1) + 1] - sb2;
+                    const int sb2 = m.succ_ptr[step * nT + (gtrim - 1)];
+                    nsucc = m.succ_ptr[step * nT + (gtrim - 1) + 1] - sb2;
                 }
                 if (lane < kMctsBranch) children[id * kMctsBranch + lane] = lane < nsucc ? 1 : 0;
                 if (lane == 0) {
-                    const double mdx = tb.edge_d[edge * 4 + 0], mdy = tb.edge_d[edge * 4 + 1],
-                                 mdyaw = tb.edge_d[edge * 4 + 2];
+                    const double mdx = m.edge_d[edge * 4 + 0], mdy = m.edge_d[edge * 4 + 1],
+                                 mdyaw = m.edge_d[edge * 4 + 2];
                     const double ex = px + (c * mdx - s * mdy);         // :127-132
                     const double ey = py + (s * mdx + c * mdy);
                     const double eyaw = pyaw + mdyaw;
@@ -370,14 +367,14 @@ __global__ void __launch_bounds__(kWarp) mcts_kernel(MpaDev m, BatchDev b, OutDe
                     if (!exhausted) {
                         qid = path[d - 1];
                         edge = nedge[pid];
-                        ns = tb.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
+                        ns = m.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
                     }
                     o.shape_npts[os] = ns;
                     if (o.shape_x && o.shape_y) {
                         for (int i = 0; i < kAreaStride; ++i) {
                             double ox = 0.0, oy = 0.0;
                             if (i < ns)
-                                place_point(tb, edge, PDMPC_AREA_NORMAL, i, ncos[qid], nsin[qid], nx[qid], ny[qid], ox, oy);
+                                place_point(m, edge, PDMPC_AREA_NORMAL, i, ncos[qid], nsin[qid], nx[qid], ny[qid], ox, oy);
                             o.shape_x[os * kAreaStride + i] = ox;
                             o.shape_y[os * kAreaStride + i] = oy;
                         }

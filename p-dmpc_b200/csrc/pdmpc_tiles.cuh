@@ -116,6 +116,8 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
     // read once: nvcc otherwise re-derives them from SR_TID.X (a slow special-register read) all over the pop loop
     const int tl = (int)keep_u32((unsigned)(lane % TILE)), shift = (int)keep_u32((unsigned)(tile * TILE));
     const unsigned tmask = TB << shift;
+    Tile<TILE> t;
+    t.mask = tmask; t.shift = shift; t.lane = tl;
     TileSm<HS, SP> &sm = reinterpret_cast<TileSm<HS, SP> *>(smem_raw)[tile];
     const unsigned sf = shared_base_once(sm.hf), sw = shared_base_once(sm.hw);
     const unsigned spts = shared_base_once(sm.pts), sshp = shared_base_once(sm.shp), sec = shared_base_once(sm.ec);
@@ -187,73 +189,9 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
             phase = IDLE;
         }
         if (phase == DONE) {
-            // ---- results: GraphSearch.m:58-60 / :82-89 (tile-masked: other tiles wait) ----------
-            __syncwarp(tmask);
-            if (status != PDMPC_OK) exhausted = true;   // outputs take the "no plan" defaults
-            if (tl == 0) {
-                unsigned cur = goal;
-                for (int d = Hp; d >= 0; --d) {           // Tree.m:44-52 path_to_root, flipped
-                    sm.path[d] = exhausted ? 0u : cur;
-                    if (!exhausted && d > 0) cur = nb[cur].parent;
-                }
-                o.status[si] = status;
-                if (o.is_exhausted) o.is_exhausted[si] = exhausted ? 1 : 0;
-                if (o.n_expanded) o.n_expanded[si] = n_nodes;
-                if (o.n_pops) o.n_pops[si] = n_pops;
-                if (o.pop_hash) o.pop_hash[si] = hash;
-                atomicAdd(o.counters + 0, (unsigned long long)n_pops);
-                atomicAdd(o.counters + 1, (unsigned long long)n_nodes);
-                atomicAdd(o.counters + 2, cols);
-            }
-            __syncwarp(tmask);
-            const double qnan = nan("");
-            for (int d = tl; d <= Hp; d += TILE) {
-                const unsigned pid = sm.path[d];
-                NodeA pa = {qnan, qnan, qnan, qnan};
-                NodeB pb;
-                pb.h = qnan; pb.parent = 0; pb.edge = 0; pb.trim = 0; pb.k = 0;
-                if (!exhausted) { pa = na[pid]; pb = nb[pid]; }
-                const size_t oo = (size_t)si * (Hp + 1) + d;
-                if (o.trims) o.trims[oo] = exhausted ? (d == 0 ? trim0 : 0) : (int)pb.trim;
-                if (o.tree_path) o.tree_path[oo] = (int)pid;
-                if (o.g_path) o.g_path[oo] = pa.g;
-                if (o.h_path) o.h_path[oo] = pb.h;
-                if (d >= 1) {
-                    const size_t os = (size_t)si * Hp + (d - 1);
-                    if (o.y_predicted) {                   // return_path_to.m:11-25
-                        o.y_predicted[os * 3 + 0] = pa.x;
-                        o.y_predicted[os * 3 + 1] = pa.y;
-                        o.y_predicted[os * 3 + 2] = pa.yaw;
-                    }
-                    if (o.shape_npts) {                    // return_path_area.m:5-7
-                        int edge = 0, ns = 0;
-                        NodeA qa = {0.0, 0.0, 0.0, 0.0};
-                        NodeCS qcs = {0.0, 0.0};
-                        if (!exhausted) {
-                            const unsigned qid = sm.path[d - 1];   // parent on the path (was expanded)
-                            qa = na[qid];
-                            qcs = ncs[qid];
-                            edge = pb.edge;
-                            ns = m.area_npts[edge * 3 + PDMPC_AREA_NORMAL];
-                        }
-                        o.shape_npts[os] = ns;
-                        if (o.shape_x && o.shape_y) {
-                            for (int i = 0; i < kAreaStride; ++i) {
-                                double ox = 0.0, oy = 0.0;
-                                if (i < ns) {
-                                    const int ab = (edge * 3 + PDMPC_AREA_NORMAL) * kAreaStride + i;
-                                    const double ax = m.area_x[ab], ay = m.area_y[ab];
-                                    ox = qcs.c * ax - qcs.s * ay + qa.x;   // GraphSearch.m:158-159
-                                    oy = qcs.s * ax + qcs.c * ay + qa.y;
-                                }
-                                o.shape_x[os * kAreaStride + i] = ox;
-                                o.shape_y[os * kAreaStride + i] = oy;
-                            }
-                        }
-                    }
-                }
-            }
-            __syncwarp(tmask);
+            // ---- results (tile-masked: other tiles wait) ----------------------------------------------
+            write_search_result(m, o, na, nb, ncs, sm.path, si, trim0, goal, status, exhausted, n_nodes, n_pops, hash,
+                                cols, false, nullptr, t);
             phase = IDLE;
         }
         while (phase == IDLE) {
@@ -263,50 +201,25 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
             si_u = __shfl_sync(tmask, si_u, shift);
             if (si_u >= (unsigned)b.n) { phase = EXIT; break; }
             si = b.order ? __ldg(b.order + si_u) : (int)si_u;
-            const int *slot = b.slot_ptr + (size_t)si * (Hp + 1);
-            const int sp0 = __ldg(slot + 0), spE = __ldg(slot + Hp + 1);
-            const int lp0 = __ldg(b.lane_ptr + 2 * si), lp2 = __ldg(b.lane_ptr + 2 * si + 2);
-            // polyline layout (vectorize_all_obstacles.m:27-63): obstacle slot s of this search covers
-            // [ob_lo + rng[s], ob_lo + rng[s+1]); lanelets [ll_lo, ll_hi) = [left, NaN, right, NaN]
-            const int ob_lo = __ldg(b.poly_ptr + sp0) + sp0, ob_hi = __ldg(b.poly_ptr + spE) + spE;
-            const int ll_lo = lp0 + 2 * si, ll_hi = lp2 + 2 * si + 2;
-            const int nl = ll_hi - ll_lo, no = ob_hi - ob_lo;
+            __syncwarp(tmask);
+            stage_reference(b, si, Hp, sm.refx, sm.refy, sm.vref, t);
+            const SearchPolylines pl = search_polylines(b, si, Hp, sm.rng, t);
+            const int nl = pl.ll_hi - pl.ll_lo, no = pl.ob_hi - pl.ob_lo;
             const int sp_lim = pts_limit > 0 ? min(pts_limit, SP) : SP;
             const bool lst = nl <= sp_lim, ost = (lst ? nl : 0) + no <= sp_lim;
-            __syncwarp(tmask);
-            for (int k = tl; k < Hp; k += TILE) {
-                sm.refx[k] = __ldg(b.ref_x + (size_t)si * Hp + k);
-                sm.refy[k] = __ldg(b.ref_y + (size_t)si * Hp + k);
-                sm.vref[k] = __ldg(b.v_ref + (size_t)si * Hp + k);
-            }
-            for (int k = tl; k <= Hp + 1; k += TILE) {
-                const int q = __ldg(slot + k);
-                sm.rng[k] = __ldg(b.poly_ptr + q) + q - ob_lo;
-            }
             // lanelet bounds first (they are tested at every pop), then the obstacle slots
             if (lst)
-                for (int j = tl; j < nl; j += TILE) sm.pts[j] = __ldg(b.ll_xy + ll_lo + j);
+                for (int j = tl; j < nl; j += TILE) sm.pts[j] = __ldg(b.ll_xy + pl.ll_lo + j);
             if (ost)
-                for (int j = tl; j < no; j += TILE) sm.pts[(lst ? nl : 0) + j] = __ldg(b.pl_xy + ob_lo + j);
-            Lp = lst ? sm.pts : b.ll_xy + ll_lo;
-            Op = ost ? sm.pts + (lst ? nl : 0) : b.pl_xy + ob_lo;
+                for (int j = tl; j < no; j += TILE) sm.pts[(lst ? nl : 0) + j] = __ldg(b.pl_xy + pl.ob_lo + j);
+            Lp = lst ? sm.pts : b.ll_xy + pl.ll_lo;
+            Op = ost ? sm.pts + (lst ? nl : 0) : b.pl_xy + pl.ob_lo;
             nlan = nl;
             trim0 = __ldg(b.trim0 + si);
-            if (tl == 0) {   // root: GraphSearch.m:34-46
-                NodeA ra;
-                ra.x = __ldg(b.x0 + si); ra.y = __ldg(b.y0 + si); ra.yaw = __ldg(b.yaw0 + si); ra.g = 0.0;
-                NodeCS rcs;
-                sincos_ref(ra.yaw, rcs.s, rcs.c);
-                NodeB rb;
-                rb.h = 0.0; rb.parent = 0; rb.edge = 0xffff; rb.trim = (unsigned char)trim0; rb.k = 0;
-                na[1] = ra; nb[1] = rb; ncs[1] = rcs;
-                HEnt re;
-                re.f = 0.0; re.w = HEnt::pack(1u, 0u, 0u, 0u, (unsigned)trim0);
-                h_st(0, re);
-            }
+            if (tl == 0) h_st(0, init_root(b, si, trim0, na, nb, ncs));
             len = 1;
             n_nodes = 1; n_pops = 0;
-            hash = 0xcbf29ce484222325ULL; cols = 0;
+            hash = kHashSeed; cols = 0;
             status = PDMPC_OK;
             exhausted = false;
             goal = 0;

@@ -46,7 +46,7 @@ constexpr size_t kSmemLimit = 227 * 1024;
 // tiles: TILE lanes per search; heap entries / staged polyline points per search in shared memory;
 // one-warp CTAs per SM the shape is compiled for (register cap) — sized so that the CTAs fill 228 KB
 #ifndef PDMPC_TILE2_CTAS
-#define PDMPC_TILE2_CTAS 20
+#define PDMPC_TILE2_CTAS 24
 #endif
 #ifndef PDMPC_TILE4_CTAS
 #define PDMPC_TILE4_CTAS 8
@@ -68,6 +68,8 @@ constexpr int kTile4Heap = PDMPC_TILE4_HEAP, kTile4Pts = PDMPC_TILE4_PTS, kTile4
 #define KERNEL_TILE2 search_tile_kernel<16, kTile2Heap, kTile2Pts, kTile2Ctas>
 #define KERNEL_TILE4 search_tile_kernel<8, kTile4Heap, kTile4Pts, kTile4Ctas>
 constexpr size_t kTile2Smem = 2 * sizeof(TileSm<kTile2Heap, kTile2Pts>);
+// the CTAs the register cap is compiled for must also fit the SM's 228 KB of shared memory (1 KB reserved per CTA)
+static_assert(kTile2Ctas * (kTile2Smem + 1024) <= 233472, "tile<16> CTAs per SM exceed the shared memory");
 constexpr size_t kTile4Smem = 4 * sizeof(TileSm<kTile4Heap, kTile4Pts>);
 // "cta" = masters + shared checker warps, one CTA per SM (pdmpc_cta.cuh).  Two configurations:
 //   1 master, 12 checkers (+ 3 parked warps): a batch of at most one search per SM — lowest latency
@@ -1251,9 +1253,10 @@ static int plan_batch_pipelined(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc
     int slots = 0;
     warp_shape_grid(h, shape, per_chunk, &slots);
     int lanes = std::min(C, kLanes);
-    {   // node arenas of all lanes within 32 GiB
+    {   // node arenas of all lanes within 40 GiB: three lanes of the tile<16> shape at 24 CTAs per SM (12.5 GB each for
+        // triple_speed) — with two, a chunk kernel's tail no longer overlaps the next chunks' searches
         const double per_lane = (double)slots * node_cap(h) * (sizeof(NodeA) + sizeof(NodeB) + sizeof(NodeCS) + sizeof(HEnt));
-        lanes = std::max(2, std::min(lanes, (int)(32.0 * 1024 * 1024 * 1024 / per_lane)));
+        lanes = std::max(2, std::min(lanes, (int)(40.0 * 1024 * 1024 * 1024 / per_lane)));
     }
     const bool esc = escalation_on(h, shape, n);
     rc = ensure_arena(h, esc ? lanes * slots + h->num_sms * kCtaMasters : lanes * slots);

@@ -94,10 +94,17 @@ struct __align__(16) TileSm {
     unsigned long long hw[HS];              // heap payloads
     double2 pts[SP];                        // staged polylines (x, y): [lanelet bounds][obstacle slots 0..Hp]
     double2 shp[2][kAreaStride];            // placed areas: [0] normal offset, [1] boundary check; tail = last vertex
-    double ec[2][kAreaStride][4];           // per shape edge: dx1, dy1, S1, -
+    double2 ed[2][kAreaStride];             // per shape edge: dx1, dy1
+    double es[2][kAreaStride];              // per shape edge: S1
     double refx[kMaxHp], refy[kMaxHp], vref[kMaxHp];
     int rng[kMaxHp + 2];                    // polyline offset of obstacle slot s
     unsigned path[kMaxHp + 1];
+    // the current search's state that the pop loop reads at most once per pop: kept here rather than in
+    // registers of each of the tile's lanes (the pop loop's register peak caps the warps per SM)
+    const double2 *op, *lp;                 // obstacle slot s at op + rng[s]; lanelet bounds [lp, lp + nlan)
+    int si, trim0, nlan, status;
+    unsigned goal;
+    int exhausted;
 };
 
 
@@ -118,28 +125,31 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
     const unsigned tmask = TB << shift;
     Tile<TILE> t;
     t.mask = tmask; t.shift = shift; t.lane = tl;
-    TileSm<HS, SP> &sm = reinterpret_cast<TileSm<HS, SP> *>(smem_raw)[tile];
-    const unsigned sf = shared_base_once(sm.hf), sw = shared_base_once(sm.hw);
-    const unsigned spts = shared_base_once(sm.pts), sshp = shared_base_once(sm.shp), sec = shared_base_once(sm.ec);
+    using Sm = TileSm<HS, SP>;
+    Sm &sm = reinterpret_cast<Sm *>(smem_raw)[tile];
+    // every shared address of the pop loop is this one base plus a compile-time offset
+    const unsigned smb = shared_base_once(&sm);
+    constexpr unsigned oHf = offsetof(Sm, hf), oHw = offsetof(Sm, hw), oShp = offsetof(Sm, shp);
+    constexpr unsigned oEd = offsetof(Sm, ed), oEs = offsetof(Sm, es);
 
     const int Hp = m.Hp, nT = m.nT;
-    const size_t slot_base = ((size_t)blockIdx.x * T + tile) * (size_t)ar.cap;
-    NodeA *__restrict__ na = ar.a + slot_base;
-    NodeB *__restrict__ nb = ar.b + slot_base;
-    NodeCS *__restrict__ ncs = ar.cs + slot_base;
-    HEnt *__restrict__ hgl = ar.heap + slot_base;
+    // the tile's arena slot; node and heap addresses are formed from it where they are used
+    const unsigned slot = blockIdx.x * T + tile;
+    auto node = [&](auto *base, unsigned i) { return base + ((size_t)slot * (unsigned)ar.cap + i); };
 
     // ---- heap access: entries [0, HS) in shared memory, the rest in the slot's arena ----------------
-    auto h_f = [&](int i) -> double { return i < HS ? lds_f64(sf + 8u * (unsigned)(i + 1)) : hgl[i].f; };
+    auto h_f = [&](int i) -> double {
+        return i < HS ? lds_f64(smb + oHf + 8u * (unsigned)(i + 1)) : node(ar.heap, (unsigned)i)->f;
+    };
     auto h_ld = [&](int i) -> HEnt {
         HEnt e;
-        if (i < HS) { e.f = lds_f64(sf + 8u * (unsigned)(i + 1)); e.w = lds_u64(sw + 8u * (unsigned)i); }
-        else e = hgl[i];
+        if (i < HS) { e.f = lds_f64(smb + oHf + 8u * (unsigned)(i + 1)); e.w = lds_u64(smb + oHw + 8u * (unsigned)i); }
+        else e = *node(ar.heap, (unsigned)i);
         return e;
     };
     auto h_st = [&](int i, const HEnt &e) {
-        if (i < HS) { sts_f64(sf + 8u * (unsigned)(i + 1), e.f); sts_u64(sw + 8u * (unsigned)i, e.w); }
-        else hgl[i] = e;
+        if (i < HS) { sts_f64(smb + oHf + 8u * (unsigned)(i + 1), e.f); sts_u64(smb + oHw + 8u * (unsigned)i, e.w); }
+        else *node(ar.heap, (unsigned)i) = e;
     };
     // __push_heap(first, p, 0, v) for the tiles with `su` (stl_heap.h:135-147): lanes <-> ancestors of p
     auto sift_up_at = [&](bool su, int p, const HEnt &v) {
@@ -168,15 +178,9 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
 
     enum { IDLE = 0, RUN = 1, DONE = 2, EXIT = 3 };
     int phase = IDLE;
-    int si = 0, trim0 = 0, len = 0;
-    // polylines of the current search as (x, y) pairs, read through GENERIC pointers: the staged copy in shared
-    // memory or, when a polyline does not fit, the batch's interleaved arrays (L1 / L2) — one code path for both
-    const double2 *Op = nullptr, *Lp = nullptr;   // obstacle slot s at Op + rng[s]; lanelet bounds [Lp, Lp + nlan)
-    int nlan = 0;
-    int n_nodes = 0, n_pops = 0, status = PDMPC_OK;
+    int len = 0;
+    int n_nodes = 0, n_pops = 0;
     unsigned long long hash = 0, cols = 0;
-    bool exhausted = false;
-    unsigned goal = 0;
 
     for (;;) {
         if (phase == RUN && b.pop_limit > 0 && n_pops >= b.pop_limit) {
@@ -184,14 +188,15 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
             //      runs it from scratch at a fraction of the per-pop latency.  Nothing of it is written here.
             if (tl == 0) {
                 const unsigned q = atomicAdd(b.esc_count, 1u);
-                st_release_gpu(b.esc_list + q, si);
+                st_release_gpu(b.esc_list + q, sm.si);
             }
             phase = IDLE;
         }
         if (phase == DONE) {
             // ---- results (tile-masked: other tiles wait) ----------------------------------------------
-            write_search_result(m, o, na, nb, ncs, sm.path, si, trim0, goal, status, exhausted, n_nodes, n_pops, hash,
-                                cols, false, nullptr, t);
+            __syncwarp(tmask);   // goal / status / exhausted were stored by the tile's lane 0
+            write_search_result(m, o, node(ar.a, 0), node(ar.b, 0), node(ar.cs, 0), sm.path, sm.si, sm.trim0, sm.goal,
+                                sm.status, sm.exhausted != 0, n_nodes, n_pops, hash, cols, false, nullptr, t);
             phase = IDLE;
         }
         while (phase == IDLE) {
@@ -200,7 +205,7 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
             if (tl == 0) si_u = atomicAdd(work_counter, 1u);
             si_u = __shfl_sync(tmask, si_u, shift);
             if (si_u >= (unsigned)b.n) { phase = EXIT; break; }
-            si = b.order ? __ldg(b.order + si_u) : (int)si_u;
+            const int si = b.order ? __ldg(b.order + si_u) : (int)si_u;
             __syncwarp(tmask);
             stage_reference(b, si, Hp, sm.refx, sm.refy, sm.vref, t);
             const SearchPolylines pl = search_polylines(b, si, Hp, sm.rng, t);
@@ -212,17 +217,20 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
                 for (int j = tl; j < nl; j += TILE) sm.pts[j] = __ldg(b.ll_xy + pl.ll_lo + j);
             if (ost)
                 for (int j = tl; j < no; j += TILE) sm.pts[(lst ? nl : 0) + j] = __ldg(b.pl_xy + pl.ob_lo + j);
-            Lp = lst ? sm.pts : b.ll_xy + pl.ll_lo;
-            Op = ost ? sm.pts + (lst ? nl : 0) : b.pl_xy + pl.ob_lo;
-            nlan = nl;
-            trim0 = __ldg(b.trim0 + si);
-            if (tl == 0) h_st(0, init_root(b, si, trim0, na, nb, ncs));
+            const int trim0 = __ldg(b.trim0 + si);
+            if (tl == 0) {
+                // polylines of the search as (x, y) pairs, read through GENERIC pointers: the staged copy in shared
+                // memory or, when a polyline does not fit, the batch's interleaved arrays (L1 / L2) — one code
+                // path for both
+                sm.lp = lst ? sm.pts : b.ll_xy + pl.ll_lo;
+                sm.op = ost ? sm.pts + (lst ? nl : 0) : b.pl_xy + pl.ob_lo;
+                sm.si = si; sm.trim0 = trim0; sm.nlan = nl;
+                sm.status = PDMPC_OK; sm.goal = 0; sm.exhausted = 0;
+                h_st(0, init_root(b, si, trim0, node(ar.a, 0), node(ar.b, 0), node(ar.cs, 0)));
+            }
             len = 1;
             n_nodes = 1; n_pops = 0;
             hash = kHashSeed; cols = 0;
-            status = PDMPC_OK;
-            exhausted = false;
-            goal = 0;
             phase = RUN;
             __threadfence_block();
             __syncwarp(tmask);
@@ -233,17 +241,19 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
         // =========== one pop for every running tile: GraphSearch.m:53-107 ==========================
         const bool run = phase == RUN;
         const bool has = run && len > 0;
-        if (run && !has) { exhausted = true; phase = DONE; }                // :57-61
+        if (run && !has) {                                                  // :57-61
+            if (tl == 0) sm.exhausted = 1;
+            phase = DONE;
+        }
         HEnt top;
         top.f = 0.0; top.w = 0;
-        if (has) { top.f = lds_f64(sf + 8u); top.w = lds_u64(sw); }
+        if (has) { top.f = lds_f64(smb + oHf + 8u); top.w = lds_u64(smb + oHw); }
         const unsigned id = top.id(), par = top.pid();
         const int cK = (int)top.k(), ctrim = (int)top.trim(), edge = (int)top.edge();
         const bool chk = has && par != 0;       // eval_edge_exact :137-139: the root is valid unchecked
-        // ---- early loads (their latency hides behind the heap walk): own record, parent pose,
-        //      successor list, point counts of the maneuver's areas
-        NodeA ca = {0.0, 0.0, 0.0, 0.0};
-        NodeCS ccs = {0.0, 0.0}, pcs = {0.0, 0.0};
+        // ---- early loads (their latency hides behind the heap walk): parent pose, successor list, point counts
+        //      of the maneuver's areas.  The own record is loaded after the edge check, by the tiles that expand.
+        NodeCS pcs = {0.0, 0.0};
         double2 pxy = make_double2(0.0, 0.0);
         int sbase = 0, send = 0, ns = 0, nbs = 0;   // consumed after the heap walk (their loads overlap it)
         const int bkind = (cK == Hp) ? PDMPC_AREA_LARGE_OFFSET : PDMPC_AREA_WITHOUT_OFFSET;   // :166-174
@@ -262,22 +272,20 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
             }
         }
         if (has) {
-            if (cK < Hp) {                                // own record and successor list: only an expansion reads them
-                ca = na[id];
-                ccs = ncs[id];
+            if (cK < Hp) {                                // successor list: only an expansion reads it
                 const int q = cK * nT + (ctrim - 1);      // step k_exp = cK + 1
                 sbase = __ldg(m.succ_ptr + q);
                 send = __ldg(m.succ_ptr + q + 1);
             }
             if (par != 0) {
-                pxy = *reinterpret_cast<const double2 *>(na + par);
-                pcs = ncs[par];                            // cos/sin(parent yaw), :155-156
+                pxy = *reinterpret_cast<const double2 *>(node(ar.a, par));
+                pcs = *node(ar.cs, par);                   // cos/sin(parent yaw), :155-156
                 ns = __ldg(m.area_npts + edge * 3 + PDMPC_AREA_NORMAL);
                 nbs = __ldg(m.area_npts + edge * 3 + bkind);
             }
             ++n_pops;
             if (!b.hash_valid_only) hash = hash_step(hash, id);
-            if (tr.search == si && tl == 0) {
+            if (tr.search >= 0 && tl == 0 && tr.search == sm.si) {
                 if (n_pops <= tr.cap) tr.ids[n_pops - 1] = (long long)id;
                 *tr.n = n_pops;
             }
@@ -294,14 +302,14 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
                 const int lim = (n - 1) >> 1;       // hole < lim: both children exist
                 if (n <= HS) {
                     while (hole < lim) {            // the hole follows the smaller child (right unless right.f > left.f)
-                        const double2 p = lds_f64x2(sf + 16u * (unsigned)hole + 16u);
+                        const double2 p = lds_f64x2(smb + oHf + 16u * (unsigned)hole + 16u);
                         hole = 2 * hole + 2 - (p.y > p.x ? 1 : 0);
                         ++D;
                     }
                 } else {
                     while (hole < lim) {
                         if (2 * hole + 2 < HS) {
-                            const double2 p = lds_f64x2(sf + 16u * (unsigned)hole + 16u);
+                            const double2 p = lds_f64x2(smb + oHf + 16u * (unsigned)hole + 16u);
                             hole = 2 * hole + 2 - (p.y > p.x ? 1 : 0);
                             ++D;
                             continue;
@@ -347,31 +355,31 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
         bool valid = has;
         if (TILE >= 16) {
             if (chk && tl < 16)
-                sts_f64x2(sshp + 16u * (unsigned)tl, pcs.c * ax0 - pcs.s * ay0 + pxy.x, pcs.s * ax0 + pcs.c * ay0 + pxy.y);
+                sts_f64x2(smb + oShp + 16u * (unsigned)tl, pcs.c * ax0 - pcs.s * ay0 + pxy.x, pcs.s * ax0 + pcs.c * ay0 + pxy.y);
         } else if (chk) {
-            sts_f64x2(sshp + 16u * (unsigned)tl, pcs.c * ax0 - pcs.s * ay0 + pxy.x, pcs.s * ax0 + pcs.c * ay0 + pxy.y);
-            sts_f64x2(sshp + 16u * (unsigned)(8 + tl), pcs.c * ax1 - pcs.s * ay1 + pxy.x, pcs.s * ax1 + pcs.c * ay1 + pxy.y);
+            sts_f64x2(smb + oShp + 16u * (unsigned)tl, pcs.c * ax0 - pcs.s * ay0 + pxy.x, pcs.s * ax0 + pcs.c * ay0 + pxy.y);
+            sts_f64x2(smb + oShp + 16u * (unsigned)(8 + tl), pcs.c * ax1 - pcs.s * ay1 + pxy.x, pcs.s * ax1 + pcs.c * ay1 + pxy.y);
         }
         __syncwarp();
         // edge constants of InterX.m:63,67 — dx1, dy1, S1 = dx1*y1 - dy1*x1 — one edge per lane
         if (TILE >= 16) {
             if (chk && tl < 16) {
                 const int i = tl & 7;
-                const double2 v0 = lds_f64x2(sshp + 16u * (unsigned)tl);
-                const double2 v1 = lds_f64x2(sshp + 16u * (unsigned)((tl & 8) + min(i + 1, 7)));
+                const double2 v0 = lds_f64x2(smb + oShp + 16u * (unsigned)tl);
+                const double2 v1 = lds_f64x2(smb + oShp + 16u * (unsigned)((tl & 8) + min(i + 1, 7)));
                 const double dx1 = v1.x - v0.x, dy1 = v1.y - v0.y;
-                sts_f64x2(sec + 32u * (unsigned)tl, dx1, dy1);
-                sts_f64(sec + 32u * (unsigned)tl + 16u, dx1 * v0.y - dy1 * v0.x);
+                sts_f64x2(smb + oEd + 16u * (unsigned)tl, dx1, dy1);
+                sts_f64(smb + oEs + 8u * (unsigned)tl, dx1 * v0.y - dy1 * v0.x);
             }
         } else {
 #pragma unroll
             for (int sel = 0; sel < 2; ++sel) {
                 if (chk) {
-                    const double2 v0 = lds_f64x2(sshp + 16u * (unsigned)(sel * 8 + tl));
-                    const double2 v1 = lds_f64x2(sshp + 16u * (unsigned)(sel * 8 + min(tl + 1, 7)));
+                    const double2 v0 = lds_f64x2(smb + oShp + 16u * (unsigned)(sel * 8 + tl));
+                    const double2 v1 = lds_f64x2(smb + oShp + 16u * (unsigned)(sel * 8 + min(tl + 1, 7)));
                     const double dx1 = v1.x - v0.x, dy1 = v1.y - v0.y;
-                    sts_f64x2(sec + 32u * (unsigned)(sel * 8 + tl), dx1, dy1);
-                    sts_f64(sec + 32u * (unsigned)(sel * 8 + tl) + 16u, dx1 * v0.y - dy1 * v0.x);
+                    sts_f64x2(smb + oEd + 16u * (unsigned)(sel * 8 + tl), dx1, dy1);
+                    sts_f64(smb + oEs + 8u * (unsigned)(sel * 8 + tl), dx1 * v0.y - dy1 * v0.x);
                 }
             }
         }
@@ -382,11 +390,13 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
         if (chk) {
             const int st_lo = sm.rng[0], st_hi = sm.rng[1];
             const int dy_lo = sm.rng[cK], dy_hi = sm.rng[cK + 1];
+            const int nlan = sm.nlan;
             cols += (unsigned long long)((st_hi - st_lo) + (dy_hi - dy_lo) + nlan);
             n0 = max(st_hi - st_lo - 1, 0);                       // InterX.m:48-52 and single-column inputs
             n01 = n0 + max(dy_hi - dy_lo - 1, 0);
             ntot = n01 + max(nlan - 1, 0);
-            P0 = Op + st_lo; P1 = Op + (dy_lo - n0); P2 = Lp - n01;
+            const double2 *Op = sm.op;
+            P0 = Op + st_lo; P1 = Op + (dy_lo - n0); P2 = sm.lp - n01;
         }
         // widest shape of the warp: edges evaluated per item (others see their padded last vertex)
         const int ne_max = __reduce_max_sync(FULL, chk ? max(ns, nbs) - 1 : 0);
@@ -405,13 +415,13 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
                     const double2 p0 = pp[0], p1 = pp[1];
                     const double dx2 = p1.x - p0.x, dy2 = p1.y - p0.y;          // InterX.m:64
                     const double S2 = dx2 * p0.y - dy2 * p0.x;                  // :68
-                    unsigned c2 = interx_c2_row<NE, CLOSED>(lb ? sshp + 128u : sshp, dx2, dy2, S2);   // :71
+                    unsigned c2 = interx_c2_row<NE, CLOSED>(smb + oShp + (lb ? 128u : 0u), dx2, dy2, S2);   // :71
                     if (NE == 4) c2 &= (1u << ne_max) - 1u;                     // ne_max < 4: the instance is wider
-                    const unsigned ebase = lb ? sec + 256u : sec;
+                    const unsigned edb = smb + oEd + (lb ? 128u : 0u), esb = smb + oEs + (lb ? 64u : 0u);
                     for (unsigned cc = c2; cc; cc &= cc - 1u) {                 // C1 of the edges with C2, :70
-                        const unsigned eb = ebase + 32u * (unsigned)(__ffs(cc) - 1);
-                        const double2 d1 = lds_f64x2(eb);
-                        const double S1 = lds_f64(eb + 16u);
+                        const unsigned i = (unsigned)(__ffs(cc) - 1);
+                        const double2 d1 = lds_f64x2(edb + 16u * i);
+                        const double S1 = lds_f64(esb + 8u * i);
                         const double a0 = (d1.x * p0.y - d1.y * p0.x) - S1;
                         const double a1 = (d1.x * p1.y - d1.y * p1.x) - S1;
                         if (a0 * a1 < 0) hit = true;
@@ -441,12 +451,27 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
 
         // ---- :75-90 ------------------------------------------------------------------------------
         if (has && valid && b.hash_valid_only) hash = hash_step(hash, id);
-        if (has && valid && cK == Hp) { goal = id; phase = DONE; }
+        if (has && valid && cK == Hp) {
+            if (tl == 0) sm.goal = id;
+            phase = DONE;
+        }
         bool doexp = has && valid && cK < Hp;
-        if (doexp && n_nodes + nchild >= ar.cap) { status = PDMPC_ERR_CAPACITY; phase = DONE; doexp = false; }
+        if (doexp && n_nodes + nchild >= ar.cap) {
+            if (tl == 0) sm.status = PDMPC_ERR_CAPACITY;
+            phase = DONE;
+            doexp = false;
+        }
         if (!__any_sync(FULL, doexp)) continue;
 
         // ---- expand_node.m:1-91 (nV == 1): lane q creates child q ---------------------------------
+        // the own record is loaded here rather than with the early loads: held through the heap walk and the
+        // InterX loop, it set the kernel's register peak
+        NodeA ca = {0.0, 0.0, 0.0, 0.0};
+        NodeCS ccs = {0.0, 0.0};
+        if (doexp) {
+            ca = *node(ar.a, id);
+            ccs = *node(ar.cs, id);
+        }
         const int k_exp = cK + 1;
         const int to_go = Hp - k_exp;               // :37
         const double s = ccs.s, c = ccs.c;          // :50-51, computed when the node was created
@@ -490,12 +515,12 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
                 NodeB eb;
                 eb.h = eh; eb.parent = id; eb.edge = (unsigned short)cedge;
                 eb.trim = (unsigned char)t2; eb.k = (unsigned char)k_exp;
-                na[nid] = ea;                               // Tree.m:54-70 add_nodes
-                nb[nid] = eb;
+                *node(ar.a, nid) = ea;                      // Tree.m:54-70 add_nodes
+                *node(ar.b, nid) = eb;
                 if (k_exp < Hp) {                           // cos/sin of the child's yaw: for ITS expansion and for placing
                     NodeCS ecs;                             // its children's areas — a node of depth Hp has neither
                     sincos_ref(ea.yaw, ecs.s, ecs.c);
-                    ncs[nid] = ecs;
+                    *node(ar.cs, nid) = ecs;
                 }
                 he.f = ea.g + eh;                           // GraphSearch.m:102 (weights 1)
                 he.w = HEnt::pack(nid, id, (unsigned)cedge, (unsigned)k_exp, (unsigned)t2);

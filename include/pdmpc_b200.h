@@ -487,6 +487,48 @@ typedef struct pdmpc_timestep_states {
 } pdmpc_timestep_states;
 int pdmpc_plan_timestep_from_states(pdmpc_handle *h, const pdmpc_timestep_states *states, pdmpc_batch_out *out);
 
+/* ---- Coupling, priorities and computation levels of a time step on the device: what the host decides before
+ *      pdmpc_plan_timestep_from_states, for every scenario of the time step in one call (DESIGN.md §4.12).
+ *        - coupling (ReachableSetCoupler.m:5-54): rows i, j of one scenario are coupled iff the step-Hp reachable sets of
+ *          their current trims (reachable_sets{i, end}, pdmpc_upload_reachable_sets) placed at their poses overlap by more
+ *          than 1e-3 (:39-42).  [dev] the overlap is the Sutherland-Hodgman clipping of DESIGN.md §4.12 in FP64 (the
+ *          sets are convex), not polyshape intersect; the lanelet clipping of HighLevelController.m:241-246 is not done;
+ *        - priorities: PDMPC_PRIORITY_CONSTANT (ConstantPrioritizer.m:6-18, the lower row first) or
+ *          PDMPC_PRIORITY_COLORING (ColoringPrioritizer.m:11-153); directed coupling D(i, j) = coupled and prio(i) < prio(j);
+ *        - sequential relation seq: the predecessors of row j that stay sequential so that no row sits deeper than
+ *          max_num_CLs computation levels (equal to D when max_num_CLs >= the depth); level = kahn(seq), 1-based;
+ *        - the three relations of pdmpc_timestep_states: successors = D(i, :), parallel = D(:, i) & ~seq(:, i),
+ *          predecessors = seq(:, i); global 0-based rows, ascending within each list. ---- */
+#define PDMPC_PRIORITY_CONSTANT 0      /* ConstantPrioritizer.m:6-18 */
+#define PDMPC_PRIORITY_COLORING 1      /* ColoringPrioritizer.m:11-153 */
+#define PDMPC_COUPLE_MAX_VEHICLES 64   /* rows per scenario */
+typedef struct pdmpc_couple_params {
+    int32_t n_scenarios;
+    const int32_t *scenario_ptr;   /* [n_scenarios+1]: rows of scenario s are [ptr[s], ptr[s+1]), ptr[0] == 0, ptr[n_scenarios] == n */
+    int32_t prioritizer;           /* PDMPC_PRIORITY_* */
+    int32_t max_num_CLs;           /* >= 1 */
+} pdmpc_couple_params;
+typedef struct pdmpc_couple_out {  /* caller-owned host buffers; NULL fields are not copied back */
+    int32_t *succ_ptr, *succ_idx;  /* [n+1], [idx_capacity]: as pdmpc_timestep_states */
+    int32_t *par_ptr, *par_idx;
+    int32_t *pred_ptr, *pred_idx;
+    int32_t idx_capacity;          /* entries of each *_idx array; PDMPC_ERR_CAPACITY if a relation has more */
+    int32_t *level;                /* [n] 1-based computation level */
+    double *overlap_area;          /* [sum of n_s^2] per scenario an n_s x n_s row-major matrix; 0.0 on the diagonal */
+} pdmpc_couple_out;
+/* Needs pdmpc_upload_mpa and pdmpc_upload_reachable_sets (of that automaton; at most 129 points per set).  x, y, yaw,
+ * trim: [n] measured pose and current trim (1-based) of every row.  Errors: PDMPC_ERR_BAD_INPUT for a missing or foreign
+ * reachable-set table, a trim out of range, a malformed scenario_ptr, a scenario of more than PDMPC_COUPLE_MAX_VEHICLES
+ * rows, an unknown prioritizer or max_num_CLs < 1; PDMPC_ERR_CAPACITY when idx_capacity is too small. */
+int pdmpc_couple(pdmpc_handle *h, int32_t n, const double *x, const double *y, const double *yaw, const int32_t *trim,
+                 const pdmpc_couple_params *prm, pdmpc_couple_out *out);
+/* pdmpc_plan_timestep_from_states with the three relations decided by pdmpc_couple first (same call, one small
+ * device->host copy of the relations in between): st's succ / par / pred pointers must be NULL (PDMPC_ERR_BAD_INPUT
+ * otherwise).  The relations used are returned in `rel` (may be NULL); PDMPC_ERR_CAPACITY, before anything is planned,
+ * when they do not fit rel->idx_capacity. */
+int pdmpc_plan_timestep_from_states_coupled(pdmpc_handle *h, const pdmpc_timestep_states *st, const pdmpc_couple_params *prm,
+                                            pdmpc_couple_out *rel, pdmpc_batch_out *out);
+
 /* Pinned host buffers for callers that want full-rate host<->device copies. */
 int pdmpc_host_alloc(void **p, size_t bytes);
 int pdmpc_host_free(void *p);

@@ -35,6 +35,7 @@ EXPORTED_SYMBOLS = (
     "pdmpc_run_staged", "pdmpc_sync", "pdmpc_fetch_staged", "pdmpc_get_stats", "pdmpc_stream",
     "pdmpc_mcts_plan_batch", "pdmpc_mcts_run_staged", "pdmpc_set_cta_heap_smem", "pdmpc_plan_timestep",
     "pdmpc_set_pipeline_chunks", "pdmpc_measure_fp64_peak", "pdmpc_joint_plan_batch",
+    "pdmpc_couple", "pdmpc_plan_timestep_from_states_coupled",
 )
 
 _p_u8 = C.POINTER(C.c_uint8)
@@ -114,7 +115,19 @@ class TimestepStatesC(C.Structure):
                 ("half_length", C.c_double), ("half_width", C.c_double), ("dt_seconds", C.c_double), ("checker", C.c_int32)]
 
 
+class CoupleParamsC(C.Structure):
+    _fields_ = [("n_scenarios", C.c_int32), ("scenario_ptr", _p_i32), ("prioritizer", C.c_int32), ("max_num_CLs", C.c_int32)]
+
+
+class CoupleOutC(C.Structure):
+    _fields_ = [("succ_ptr", _p_i32), ("succ_idx", _p_i32), ("par_ptr", _p_i32), ("par_idx", _p_i32),
+                ("pred_ptr", _p_i32), ("pred_idx", _p_i32), ("idx_capacity", C.c_int32), ("level", _p_i32),
+                ("overlap_area", _p_f64)]
+
+
 MAX_PRED_LANELETS = 8
+PRIORITY_CONSTANT, PRIORITY_COLORING = 0, 1
+COUPLE_MAX_VEHICLES = 64
 
 
 class Stats(C.Structure):
@@ -235,6 +248,11 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
     lib.pdmpc_pipeline_bounds.restype = C.c_int
     lib.pdmpc_plan_timestep_from_states.argtypes = [H, C.POINTER(TimestepStatesC), C.POINTER(BatchOut)]
     lib.pdmpc_plan_timestep_from_states.restype = C.c_int
+    lib.pdmpc_couple.argtypes = [H, C.c_int32, _p_f64, _p_f64, _p_f64, _p_i32, C.POINTER(CoupleParamsC), C.POINTER(CoupleOutC)]
+    lib.pdmpc_couple.restype = C.c_int
+    lib.pdmpc_plan_timestep_from_states_coupled.argtypes = [H, C.POINTER(TimestepStatesC), C.POINTER(CoupleParamsC),
+                                                            C.POINTER(CoupleOutC), C.POINTER(BatchOut)]
+    lib.pdmpc_plan_timestep_from_states_coupled.restype = C.c_int
     lib.pdmpc_closed_loop_reset.argtypes = [H, C.c_int32, C.c_double, C.c_double]
     lib.pdmpc_closed_loop_reset.restype = C.c_int
     lib.pdmpc_plan_timestep_closed_loop.argtypes = [H, C.POINTER(BatchIn), C.POINTER(TimestepDepsC), _p_i32,
@@ -555,6 +573,68 @@ class Planner:
             bad = int(np.flatnonzero(r.status != PDMPC_OK)[0])
             raise PdmpcError(int(r.status[bad]), f"search {bad} failed")
         return r
+
+    def _couple_args(self, n: int, priority, max_num_CLs: int, scenario_ptr, idx_capacity: int):
+        """(params, out struct, relations dict, keepalive) of pdmpc_couple / pdmpc_plan_timestep_from_states_coupled."""
+        sp = np.ascontiguousarray([0, n] if scenario_ptr is None else scenario_ptr, dtype=np.int32)
+        if isinstance(priority, str):
+            priority = {"constant": PRIORITY_CONSTANT, "coloring": PRIORITY_COLORING}[priority]
+        sizes = np.diff(sp).astype(np.int64)
+        cap = int(idx_capacity) or max(1, int((sizes * (sizes - 1) // 2).sum()))
+        rel = {k: np.zeros(n + 1, dtype=np.int32) for k in ("succ_ptr", "par_ptr", "pred_ptr")}
+        rel.update({k: np.zeros(cap, dtype=np.int32) for k in ("succ_idx", "par_idx", "pred_idx")})
+        rel["level"] = np.zeros(max(n, 1), dtype=np.int32)
+        area = np.zeros(max(1, int((sizes * sizes).sum())))
+        prm = CoupleParamsC(n_scenarios=int(sp.size - 1), scenario_ptr=_ptr(sp, _p_i32), prioritizer=int(priority),
+                            max_num_CLs=int(max_num_CLs))
+        oc = CoupleOutC(idx_capacity=cap, overlap_area=_ptr(area, _p_f64), **{k: _ptr(v, _p_i32) for k, v in rel.items()})
+        return prm, oc, rel, (sp, sizes, area)
+
+    @staticmethod
+    def _relations(n: int, rel: dict, keep) -> dict:
+        _sp, sizes, area = keep
+        for k in ("succ", "par", "pred"):
+            rel[f"{k}_idx"] = rel[f"{k}_idx"][: int(rel[f"{k}_ptr"][-1])]
+        rel["level"] = rel["level"][:n]
+        ends = np.cumsum(sizes * sizes)
+        rel["overlap_area"] = [area[e - s * s:e].reshape(s, s) for s, e in zip(sizes, ends)]
+        return rel
+
+    def couple(self, x, y, yaw, trim, scenario_ptr=None, priority="coloring", max_num_CLs: int = 99,
+               idx_capacity: int = 0) -> dict:
+        """Coupling (reachable-set overlap > 1e-3), priorities, the level cut and computation levels of every scenario
+        (pdmpc_couple).  scenario_ptr: rows of scenario s are [ptr[s], ptr[s+1]) (default: one scenario).  Returns
+        succ_ptr / succ_idx, par_ptr / par_idx, pred_ptr / pred_idx (the relations of plan_timestep_from_states, global
+        rows), level [n] (1-based) and overlap_area (one [n_s, n_s] matrix per scenario)."""
+        x, y, yaw = (np.ascontiguousarray(a, dtype=np.float64) for a in (x, y, yaw))
+        trim = np.ascontiguousarray(trim, dtype=np.int32)
+        n = int(x.size)
+        prm, oc, rel, keep = self._couple_args(n, priority, max_num_CLs, scenario_ptr, idx_capacity)
+        self._check(self.lib.pdmpc_couple(self.h, n, _ptr(x, _p_f64), _ptr(y, _p_f64), _ptr(yaw, _p_f64), _ptr(trim, _p_i32),
+                                          C.byref(prm), C.byref(oc)))
+        return self._relations(n, rel, keep)
+
+    def plan_timestep_from_states_coupled(self, path_id, x, y, yaw, speed, trim, slot, half_length: float,
+                                          half_width: float, dt_seconds: float, checker: int, priority="coloring",
+                                          max_num_CLs: int = 99, scenario_ptr=None, idx_capacity: int = 0,
+                                          raise_on_search_error: bool = True):
+        """plan_timestep_from_states with the relations decided on the device (pdmpc_plan_timestep_from_states_coupled):
+        returns (BatchResult, relations as Planner.couple returns them)."""
+        path_id, trim, slot = (np.ascontiguousarray(a, dtype=np.int32) for a in (path_id, trim, slot))
+        x, y, yaw, speed = (np.ascontiguousarray(a, dtype=np.float64) for a in (x, y, yaw, speed))
+        n, Hp = int(x.size), int(self.lib.pdmpc_get_hp(self.h))
+        prm, oc, rel, keep = self._couple_args(n, priority, max_num_CLs, scenario_ptr, idx_capacity)
+        r = BatchResult.empty(n, Hp)
+        bo = batch_out(r)
+        st = TimestepStatesC(n=n, path_id=_ptr(path_id, _p_i32), x=_ptr(x, _p_f64), y=_ptr(y, _p_f64), yaw=_ptr(yaw, _p_f64),
+                             speed=_ptr(speed, _p_f64), trim=_ptr(trim, _p_i32), slot=_ptr(slot, _p_i32),
+                             half_length=float(half_length), half_width=float(half_width), dt_seconds=float(dt_seconds),
+                             checker=int(checker))
+        self._check(self.lib.pdmpc_plan_timestep_from_states_coupled(self.h, C.byref(st), C.byref(prm), C.byref(oc), C.byref(bo)))
+        if raise_on_search_error and n and int(r.status.max()) != PDMPC_OK:
+            bad = int(np.flatnonzero(r.status != PDMPC_OK)[0])
+            raise PdmpcError(int(r.status[bad]), f"search {bad} failed")
+        return r, self._relations(n, rel, keep)
 
     def joint_plan_batch(self, b: SearchBatch, n_vehicles: int, raise_on_search_error: bool = True) -> BatchResult:
         """Centralized (joint) searches: rows of `b` are searches x n_vehicles (pdmpc_joint_plan_batch)."""

@@ -24,6 +24,7 @@
 #include "pdmpc_inputs.cuh"
 #include "pdmpc_fallback.cuh"
 #include "pdmpc_obstacles.cuh"
+#include "pdmpc_coupling.cuh"
 
 using namespace pdmpc;
 
@@ -305,6 +306,8 @@ struct pdmpc_handle {
     ReachDev reach{};
     DBuf q_rptr, q_rx, q_ry, q_x, q_y, q_yaw, q_speed, q_trim, q_sptr, q_sidx, q_pptr, q_pidx, q_cs, q_cntp, q_cntv,
         q_slot, q_vbase, q_poly, q_vx, q_vy;
+    // coupling and priorities (pdmpc_couple)
+    DBuf c_sptr, c_pptr, c_aptr, c_x, c_y, c_yaw, c_trim, c_area, c_adj, c_rel, c_ovf;
     std::vector<int> road_bound_ptr;   // host copy (capacity checks)
     DBuf r_bptr, r_bx, r_by, r_pptr, r_px, r_py, r_lptr, r_lidx, r_pidx, r_loop, r_speed;
     DBuf i_pid, i_x, i_y, i_speed, i_refx, i_refy, i_vref, i_ridx, i_cur, i_pred, i_pre, i_cnt, i_lptr, i_lx, i_ly;
@@ -2185,6 +2188,147 @@ int pdmpc_get_stats(pdmpc_handle *h, pdmpc_stats *out) {
     if (h->timing_pending_d2h && cudaEventElapsedTime(&ms, h->ev[4], h->ev[5]) == cudaSuccess) h->stats.d2h_ms = ms;
     *out = h->stats;
     return PDMPC_OK;
+}
+
+}  // extern "C"
+
+// ---- coupling, priorities and computation levels of a time step (pdmpc_coupling.cuh) ----------------------------------
+// The relations of every row, as lists of global rows: [0] successors, [1] parallel predecessors, [2] sequential ones.
+struct HostRelations {
+    std::vector<int32_t> ptr[3], idx[3], level;
+};
+
+// Validation, both kernels and the one copy back of the per-row masks (and of the areas when `area_dst` is given).
+static int run_couple(pdmpc_handle *h, int n, const double *x, const double *y, const double *yaw, const int32_t *trim,
+                      const pdmpc_couple_params *prm, double *area_dst, HostRelations &rel) {
+    if (!h->has_mpa) return fail(h, PDMPC_ERR_NO_MPA, "couple: call pdmpc_upload_mpa first");
+    if (!prm || n < 0 || (n && (!x || !y || !yaw || !trim))) return fail(h, PDMPC_ERR_BAD_INPUT, "couple: NULL argument");
+    if (prm->prioritizer != PDMPC_PRIORITY_CONSTANT && prm->prioritizer != PDMPC_PRIORITY_COLORING)
+        return fail(h, PDMPC_ERR_BAD_INPUT, "couple: unknown prioritizer");
+    if (prm->max_num_CLs < 1) return fail(h, PDMPC_ERR_BAD_INPUT, "couple: max_num_CLs must be at least 1");
+    const int S = prm->n_scenarios;
+    if (S < 0 || (S > 0 && !prm->scenario_ptr) || (S == 0 && n != 0))
+        return fail(h, PDMPC_ERR_BAD_INPUT, "couple: scenario_ptr must cover the n rows");
+    if (S > 0 && (prm->scenario_ptr[0] != 0 || prm->scenario_ptr[S] != n))
+        return fail(h, PDMPC_ERR_BAD_INPUT, "couple: scenario_ptr must start at 0 and end at n");
+    std::vector<int> pair_ptr((size_t)S + 1, 0), area_ptr((size_t)S + 1, 0), row_base((size_t)n);
+    for (int s = 0; s < S; ++s) {
+        const int a = prm->scenario_ptr[s], b = prm->scenario_ptr[s + 1], ns = b - a;
+        if (ns < 0) return fail(h, PDMPC_ERR_BAD_INPUT, "couple: scenario_ptr not monotone");
+        if (ns > kCoupleMaxRows)
+            return fail(h, PDMPC_ERR_BAD_INPUT, "couple: a scenario has " + std::to_string(ns) + " rows, at most " +
+                                                    std::to_string(kCoupleMaxRows) + " are supported");
+        pair_ptr[s + 1] = pair_ptr[s] + ns * (ns - 1) / 2;
+        area_ptr[s + 1] = area_ptr[s] + ns * ns;
+        for (int r = a; r < b; ++r) row_base[r] = a;
+    }
+    if (!h->has_reach) return fail(h, PDMPC_ERR_BAD_INPUT, "couple: call pdmpc_upload_reachable_sets first");
+    if (h->reach.Hp != h->mpa.Hp || h->reach.nT != h->mpa.nT)
+        return fail(h, PDMPC_ERR_BAD_INPUT, "couple: the reachable sets belong to another automaton (n_trims, Hp)");
+    if (h->reach_max_pts - 1 > kCoupleMaxVerts)
+        return fail(h, PDMPC_ERR_BAD_INPUT, "couple: a reachable set has more than " + std::to_string(kCoupleMaxVerts + 1) + " points");
+    for (int i = 0; i < n; ++i)
+        if (trim[i] < 1 || trim[i] > h->mpa.nT) return fail(h, PDMPC_ERR_BAD_INPUT, "couple: trim out of range");
+    for (int k = 0; k < 3; ++k) rel.ptr[k].assign((size_t)n + 1, 0), rel.idx[k].clear();
+    rel.level.assign((size_t)n, 0);
+    if (n == 0) return PDMPC_OK;
+    CU_TRY(h, cudaSetDevice(h->device));
+    UP(h, h->c_sptr, prm->scenario_ptr, S + 1);
+    UP(h, h->c_pptr, pair_ptr.data(), S + 1);
+    UP(h, h->c_aptr, area_ptr.data(), S + 1);
+    UP(h, h->c_x, x, n);
+    UP(h, h->c_y, y, n);
+    UP(h, h->c_yaw, yaw, n);
+    UP(h, h->c_trim, trim, n);
+    const int n_pairs = pair_ptr[S], n_area = area_ptr[S];
+    CU_TRY(h, h->c_area.reserve((size_t)n_area * sizeof(double)));
+    CU_TRY(h, h->c_adj.reserve((size_t)n * sizeof(unsigned long long)));
+    CU_TRY(h, h->c_rel.reserve((size_t)n * sizeof(RelRow)));
+    CU_TRY(h, h->c_ovf.reserve(sizeof(int)));
+    CoupleDev c;
+    c.n_scen = S;
+    c.scen_ptr = h->c_sptr.as<int>(); c.pair_ptr = h->c_pptr.as<int>(); c.area_ptr = h->c_aptr.as<int>();
+    c.x = h->c_x.as<double>(); c.y = h->c_y.as<double>(); c.yaw = h->c_yaw.as<double>(); c.trim = h->c_trim.as<int>();
+    c.area = h->c_area.as<double>(); c.adj = h->c_adj.as<unsigned long long>(); c.overflow = h->c_ovf.as<int>();
+    CU_TRY(h, cudaEventRecord(h->ev[2], h->stream));
+    CU_TRY(h, cudaMemsetAsync(c.area, 0, (size_t)n_area * sizeof(double), h->stream));
+    CU_TRY(h, cudaMemsetAsync(c.adj, 0, (size_t)n * sizeof(unsigned long long), h->stream));
+    CU_TRY(h, cudaMemsetAsync(c.overflow, 0, sizeof(int), h->stream));
+    if (n_pairs > 0)
+        couple_pairs_kernel<<<(n_pairs + kCoupleWarps - 1) / kCoupleWarps, kCoupleWarps * kWarp, 0, h->stream>>>(h->reach, c, n_pairs);
+    couple_decide_kernel<<<S, kWarp, 0, h->stream>>>(c, prm->prioritizer, prm->max_num_CLs, h->c_rel.as<RelRow>());
+    CU_TRY(h, cudaGetLastError());
+    CU_TRY(h, cudaEventRecord(h->ev[3], h->stream));
+    h->timing_pending_kernel = true;
+    h->stats.kernel_launches = n_pairs > 0 ? 2 : 1;
+    std::vector<RelRow> rows((size_t)n);
+    int overflow = 0;
+    CU_TRY(h, cudaMemcpyAsync(rows.data(), h->c_rel.p, (size_t)n * sizeof(RelRow), cudaMemcpyDeviceToHost, h->stream));
+    CU_TRY(h, cudaMemcpyAsync(&overflow, h->c_ovf.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    DOWN(h, area_dst, h->c_area, (size_t)n_area);
+    CU_TRY(h, cudaStreamSynchronize(h->stream));
+    h->stats.d2h_bytes += (int64_t)(n * sizeof(RelRow));
+    if (overflow)
+        return fail(h, PDMPC_ERR_CAPACITY, "couple: a clipped polygon outgrew " + std::to_string(kCoupleListCap) + " points");
+    for (int i = 0; i < n; ++i) {
+        const unsigned long long m[3] = {rows[i].succ, rows[i].par, rows[i].pred};
+        for (int k = 0; k < 3; ++k) {
+            for (unsigned long long b = m[k]; b; b &= b - 1) rel.idx[k].push_back(row_base[i] + __builtin_ctzll(b));
+            rel.ptr[k][i + 1] = (int32_t)rel.idx[k].size();
+        }
+        rel.level[i] = rows[i].level;
+    }
+    return PDMPC_OK;
+}
+
+// Copies the relations into the caller's buffers (NULL fields are skipped).
+static int write_relations(pdmpc_handle *h, int n, const HostRelations &rel, pdmpc_couple_out *o) {
+    if (!o) return PDMPC_OK;
+    int32_t *ptr[3] = {o->succ_ptr, o->par_ptr, o->pred_ptr}, *idx[3] = {o->succ_idx, o->par_idx, o->pred_idx};
+    for (int k = 0; k < 3; ++k)
+        if (idx[k] && (int64_t)rel.idx[k].size() > (int64_t)o->idx_capacity)
+            return fail(h, PDMPC_ERR_CAPACITY, "couple: a relation has " + std::to_string(rel.idx[k].size()) +
+                                                   " entries, idx_capacity is " + std::to_string(o->idx_capacity));
+    for (int k = 0; k < 3; ++k) {
+        if (ptr[k]) std::copy(rel.ptr[k].begin(), rel.ptr[k].end(), ptr[k]);
+        if (idx[k]) std::copy(rel.idx[k].begin(), rel.idx[k].end(), idx[k]);
+    }
+    if (o->level) std::copy(rel.level.begin(), rel.level.begin() + n, o->level);
+    return PDMPC_OK;
+}
+
+extern "C" {
+
+int pdmpc_couple(pdmpc_handle *h, int32_t n, const double *x, const double *y, const double *yaw, const int32_t *trim,
+                 const pdmpc_couple_params *prm, pdmpc_couple_out *out) {
+    if (!h) return PDMPC_ERR_BAD_INPUT;
+    if (!out) return fail(h, PDMPC_ERR_BAD_INPUT, "couple: NULL output");
+    h->stats.h2d_bytes = 0;
+    h->stats.d2h_bytes = 0;
+    HostRelations rel;
+    const int rc = run_couple(h, n, x, y, yaw, trim, prm, out->overlap_area, rel);
+    if (rc != PDMPC_OK) return rc;
+    return write_relations(h, n, rel, out);
+}
+
+// pdmpc_plan_timestep_from_states with the relations of pdmpc_couple: they come back to the host once (the caller wants
+// them anyway), then the existing path validates them and orders the searches as for relations the host decided.
+int pdmpc_plan_timestep_from_states_coupled(pdmpc_handle *h, const pdmpc_timestep_states *st, const pdmpc_couple_params *prm,
+                                            pdmpc_couple_out *rel, pdmpc_batch_out *out) {
+    if (!h) return PDMPC_ERR_BAD_INPUT;
+    if (!st) return fail(h, PDMPC_ERR_BAD_INPUT, "plan_timestep_from_states_coupled: NULL states");
+    if (st->succ_ptr || st->succ_idx || st->par_ptr || st->par_idx || st->pred_ptr || st->pred_idx)
+        return fail(h, PDMPC_ERR_BAD_INPUT, "plan_timestep_from_states_coupled: the relations are decided here, pass NULL ones");
+    HostRelations r;
+    int rc = run_couple(h, st->n, st->x, st->y, st->yaw, st->trim, prm, rel ? rel->overlap_area : nullptr, r);
+    if (rc != PDMPC_OK) return rc;
+    rc = write_relations(h, st->n, r, rel);
+    if (rc != PDMPC_OK) return rc;
+    pdmpc_timestep_states s = *st;
+    s.succ_ptr = r.ptr[0].data(); s.succ_idx = r.idx[0].data();
+    s.par_ptr = r.ptr[1].data(); s.par_idx = r.idx[1].data();
+    s.pred_ptr = r.ptr[2].data(); s.pred_idx = r.idx[2].data();
+    return pdmpc_plan_timestep_from_states(h, &s, out);
 }
 
 }  // extern "C"

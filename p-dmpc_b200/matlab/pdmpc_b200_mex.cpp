@@ -45,6 +45,11 @@
 //       (assemble_obstacles_cuda.m): standing successors' occupied areas (PrioritizedController.m:508-540,
 //       get_occupied_areas.m:19-25) and parallel predecessors' reachable sets (:391-407,
 //       MotionPrimitiveAutomaton.m:649-687).
+//   [adjacency (N x N), overlap_area (N x N)] = mex(COUPLE, h, x0 [N x 3] (x, y, yaw), trims [N])
+//       ReachableSetCoupler.couple for ONE scenario (couple_cuda.m, needs UPLOAD_REACHABLE_SETS): adjacency(i, j) = 1 iff
+//       the step-Hp reachable sets of vehicles i and j overlap by more than 1e-3 (ReachableSetCoupler.m:39-42), N <= 64.
+//       The prioritizer classes stay MATLAB's.
+#include <algorithm>
 #include <cstdint>
 #include <cstring>
 #include <string>
@@ -56,7 +61,7 @@
 namespace {
 
 enum Command { CREATE = 0, DESTROY = 1, UPLOAD_MPA = 2, PLAN = 3, STATS = 4, PLAN_SAMPLED = 5, PLAN_TIMESTEP = 6, PLAN_JOINT = 7, UPLOAD_ROAD = 8,
-               SAMPLE_INPUTS = 9, UPLOAD_REACHABLE_SETS = 10, ASSEMBLE_OBSTACLES = 11 };
+               SAMPLE_INPUTS = 9, UPLOAD_REACHABLE_SETS = 10, ASSEMBLE_OBSTACLES = 11, COUPLE = 12 };
 
 std::vector<pdmpc_handle *> g_handles;   // released at `clear mex` (HighLevelController.m:284-303)
 bool g_at_exit_registered = false;
@@ -614,6 +619,40 @@ void assemble_obstacles(pdmpc_handle *h, int nlhs, mxArray *plhs[], const mxArra
     }
 }
 
+// COUPLE: the reachable-set coupling of one scenario -> pdmpc_couple; adjacency = every coupled pair in either direction
+void couple(pdmpc_handle *h, int nlhs, mxArray *plhs[], const mxArray *prhs[]) {
+    const size_t N = mxGetM(prhs[2]);
+    if (mxGetN(prhs[2]) < 3 || mxGetNumberOfElements(prhs[3]) != N) fail("pdmpc:input", "COUPLE: x0 [N x 3], trims [N]");
+    const double *x0 = mxGetDoubles(prhs[2]);
+    std::vector<int32_t> trim(N), sp = {0, static_cast<int32_t>(N)}, ptr[3], idx[3], level(N + 1);
+    for (size_t i = 0; i < N; ++i) trim[i] = static_cast<int32_t>(mxGetDoubles(prhs[3])[i]);
+    for (int k = 0; k < 3; ++k) {
+        ptr[k].resize(N + 1);
+        idx[k].resize(N * N + 1);
+    }
+    pdmpc_couple_params prm;
+    prm.n_scenarios = 1; prm.scenario_ptr = sp.data(); prm.prioritizer = PDMPC_PRIORITY_CONSTANT; prm.max_num_CLs = 1;
+    std::vector<double> area(N * N + 1);                   // symmetric: row-major == column-major
+    pdmpc_couple_out out;
+    std::memset(&out, 0, sizeof(out));
+    out.succ_ptr = ptr[0].data(); out.succ_idx = idx[0].data(); out.par_ptr = ptr[1].data(); out.par_idx = idx[1].data();
+    out.pred_ptr = ptr[2].data(); out.pred_idx = idx[2].data(); out.idx_capacity = static_cast<int32_t>(N * N + 1);
+    out.level = level.data(); out.overlap_area = area.data();
+    check(h, pdmpc_couple(h, static_cast<int32_t>(N), x0, x0 + N, x0 + 2 * N, trim.data(), &prm, &out), "pdmpc_couple");
+    plhs[0] = mxCreateDoubleMatrix(N, N, mxREAL);
+    double *adj = mxGetDoubles(plhs[0]);
+    for (int k = 0; k < 3; ++k)
+        for (size_t i = 0; i < N; ++i)
+            for (int q = ptr[k][i]; q < ptr[k][i + 1]; ++q) {
+                adj[i + N * idx[k][q]] = 1.0;
+                adj[idx[k][q] + N * i] = 1.0;
+            }
+    if (nlhs > 1) {
+        plhs[1] = mxCreateDoubleMatrix(N, N, mxREAL);
+        std::copy(area.begin(), area.end() - 1, mxGetDoubles(plhs[1]));
+    }
+}
+
 }  // namespace
 
 void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
@@ -684,6 +723,10 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
     case ASSEMBLE_OBSTACLES:
         if (nrhs < 8) fail("pdmpc:usage", "ASSEMBLE_OBSTACLES needs 8 arguments");
         assemble_obstacles(h, nlhs, plhs, prhs);
+        return;
+    case COUPLE:
+        if (nrhs < 4) fail("pdmpc:usage", "COUPLE needs 4 arguments");
+        couple(h, nlhs, plhs, prhs);
         return;
     case STATS: {
         pdmpc_stats st;

@@ -18,8 +18,9 @@ Follows (reference file:line), with documented simplifications marked [dev]:
                                      sample_reference_trajectory.m:1-103,
                                      get_arc_distance_to_endpoint.m
   * predicted lanelets / boundary .. get_predicted_lanelets.m:1-63, get_lanelets_boundary.m:1-75
-  * coupling ....................... [dev] corridor-distance proxy for ReachableSetCoupler.m:5-54
-                                     (polyshape intersection areas are not available here)
+  * coupling ....................... [dev] corridor-distance proxy for ReachableSetCoupler.m:5-54 (couple, the default),
+                                     or ReachableSetCoupler.m:5-54 with the overlap area by a convex clipping instead
+                                     of polyshape intersect (couple_reachable_sets, DESIGN.md §4.12)
   * priorities ..................... ConstantPrioritizer.m:6-18, ColoringPrioritizer.m:11-153,
                                      Prioritizer.directed_coupling_from_priorities :62-74
   * computation levels ............. utility/kahn.m:1-24
@@ -632,6 +633,89 @@ def assemble_obstacles_host(mpa: MotionPrimitiveAutomaton, x, y, yaw, speed, tri
             "vert_x": cat(vx), "vert_y": cat(vy)}
 
 
+COUPLING_AREA_THRESHOLD = 1e-3   # ReachableSetCoupler.m:39-42: coupled iff area(intersect(...)) > 1e-3
+
+
+def convex_overlap_area(P, Q) -> float:
+    """Area of the intersection of two convex polygons by the arithmetic specification of DESIGN.md §4.12, operation by
+    operation (pdmpc_coupling.cuh computes the same bits): P, Q = closed [2, m + 1] polygons (first vertex repeated last);
+    P is clipped by Q with Sutherland-Hodgman in FP64 without FMA.  [dev] stand-in for polyshape intersect + area
+    (ReachableSetCoupler.m:39-42), whose vertex arithmetic is closed source."""
+    px, py = [float(v) for v in P[0][:-1]], [float(v) for v in P[1][:-1]]
+    qx, qy = [float(v) for v in Q[0][:-1]], [float(v) for v in Q[1][:-1]]
+    mp, mq = len(px), len(qx)
+    if mp < 3 or mq < 3:
+        return 0.0
+    if max(px) < min(qx) or max(qx) < min(px) or max(py) < min(qy) or max(qy) < min(py):
+        return 0.0
+    sq = 0.0
+    for k in range(mq):
+        k1 = (k + 1) % mq
+        sq = sq + (qx[k] * qy[k1] - qx[k1] * qy[k])
+    if sq == 0.0:
+        return 0.0
+    if sq < 0.0:
+        qx.reverse()
+        qy.reverse()
+    cx, cy = px, py
+    for k in range(mq):
+        ax, ay, bx, by = qx[k], qy[k], qx[(k + 1) % mq], qy[(k + 1) % mq]
+        ex_, ey_ = bx - ax, by - ay
+        nx, ny = [], []
+        sx, sy = cx[-1], cy[-1]
+        ds = ex_ * (sy - ay) - ey_ * (sx - ax)
+        for x, y in zip(cx, cy):
+            de = ex_ * (y - ay) - ey_ * (x - ax)
+            if de >= 0.0:
+                if ds < 0.0:
+                    t = ds / (ds - de)
+                    nx.append(sx + t * (x - sx)); ny.append(sy + t * (y - sy))
+                nx.append(x); ny.append(y)
+            elif ds >= 0.0:
+                t = ds / (ds - de)
+                nx.append(sx + t * (x - sx)); ny.append(sy + t * (y - sy))
+            sx, sy, ds = x, y, de
+        if not nx:
+            return 0.0
+        cx, cy = nx, ny
+    m = len(cx)
+    if m < 3:
+        return 0.0
+    acc = 0.0
+    for k in range(m):
+        k1 = (k + 1) % m
+        acc = acc + (cx[k] * cy[k1] - cx[k1] * cy[k])
+    return 0.5 * abs(acc)
+
+
+def reachable_set_overlaps(mpa: MotionPrimitiveAutomaton, pose: np.ndarray, trim) -> np.ndarray:
+    """[n, n] overlap areas of the step-Hp reachable sets (reachable_sets{i, end}) of n vehicles at pose [n, 3] with their
+    current trims (1-based); 0.0 on the diagonal.  Set i is clipped by set j for i < j; the matrix is symmetric."""
+    n = pose.shape[0]
+    sets = [reachable_sets_at(mpa, *pose[i], int(trim[i]))[-1] for i in range(n)]
+    area = np.zeros((n, n))
+    for i in range(n):
+        for j in range(i + 1, n):
+            area[i, j] = area[j, i] = convex_overlap_area(sets[i], sets[j])
+    return area
+
+
+def couple_reachable_sets(mpa: MotionPrimitiveAutomaton, pose: np.ndarray, trim) -> np.ndarray:
+    """ReachableSetCoupler.couple (ReachableSetCoupler.m:5-54): vehicles i, j are coupled iff their step-Hp reachable sets
+    overlap by more than 1e-3 m^2.  [dev] the sets are not clipped by the predicted lanelets first
+    (HighLevelController.m:241-246).  Symmetric int64 adjacency with a zero diagonal."""
+    return (reachable_set_overlaps(mpa, pose, trim) > COUPLING_AREA_THRESHOLD).astype(np.int64)
+
+
+def decide_relations(A: np.ndarray, priority: str, max_num_CLs: int):
+    """Priorities, the level cut and the computation levels of one scenario from its adjacency:
+    D = directed coupling (row = higher priority; coloring_priorities or constant_priorities), seq = the sequential part
+    of D (limit_computation_levels, equal to D when max_num_CLs >= the depth), levels = kahn(seq) (1-based)."""
+    D = (constant_priorities(A) if priority == "constant" else coloring_priorities(A)).astype(bool)
+    seq = limit_computation_levels(D, max_num_CLs)
+    return D, seq, kahn(seq.astype(np.int64))
+
+
 def limit_computation_levels(D: np.ndarray, max_num_CLs: int) -> np.ndarray:
     """[dev] stand-in for the weigh + cut step (PrioritizedController.group :381-397, GreedyCut): the edges kept as
     SEQUENTIAL are chosen greedily in topological order so that no vehicle sits deeper than max_num_CLs
@@ -670,7 +754,8 @@ class ScenarioRunner:
     PrioritizedSequentialController.m:83-92)."""
 
     def __init__(self, sc: Scenario, plan_fn: PlanFn, max_num_CLs: int = 99, timestep_fn=None, inputs_fn=None,
-                 path_id0: int = 0, closed_loop_fn=None, obstacles_fn=None, states_fn=None):
+                 path_id0: int = 0, closed_loop_fn=None, obstacles_fn=None, states_fn=None, coupler: str = "corridor",
+                 coupled_fn=None):
         """plan_fn(batch) plans one computation level; with timestep_fn(batch, deps) the whole time
         step is ONE call and the predecessors' areas are handed over behind it (pdmpc_plan_timestep).
         inputs_fn(path_id, x, y, speed, dt) -> dict (capi.Planner.sample_inputs): reference trajectories and lanelet
@@ -690,6 +775,15 @@ class ScenarioRunner:
         # obstacle assembly, planning and fallback plans of a time step in ONE call; the host only decides coupling and
         # priorities
         self.states_fn = states_fn
+        # coupler: "corridor" (couple, the [dev] proxy) or "reachable_set" (couple_reachable_sets, ReachableSetCoupler)
+        if coupler not in ("corridor", "reachable_set"):
+            raise ValueError(f"unknown coupler {coupler!r}")
+        self.coupler = coupler
+        # coupled_fn(path_id, x, y, yaw, speed, trim, slot, half_length, half_width, dt, checker, priority, max_num_CLs)
+        # -> (BatchResult, relations) (capi.Planner.plan_timestep_from_states_coupled): states_fn with the reachable-set
+        # coupling, the priorities and the level cut decided on the device too; the relations the device returned are
+        # recorded in timestep_records as (step, None, relations, result)
+        self.coupled_fn = coupled_fn
         # closed_loop_fn(batch, deps, slot, standstill) -> BatchResult with the FINAL plan of every vehicle
         # (capi.Planner.plan_timestep_closed_loop): fallback plans are built and kept on the device, slot = path_id0 + i
         self.closed_loop_fn = closed_loop_fn
@@ -705,6 +799,11 @@ class ScenarioRunner:
         self.k = 0
         self.records: List[StepRecord] = []
         self.n_fallbacks = 0
+
+    def _adjacency(self) -> np.ndarray:
+        if self.coupler == "reachable_set":
+            return couple_reachable_sets(self.mpa, self.pose, self.trim)
+        return couple(self.sc, self.pose)
 
     def _iter_for(self, i: int) -> IterationData:
         sc, mpa = self.sc, self.mpa
@@ -757,7 +856,7 @@ class ScenarioRunner:
         sc, mpa = self.sc, self.mpa
         n = sc.amount
         iters = self._iters()
-        A = couple(sc, self.pose)
+        A = self._adjacency()
         D = constant_priorities(A) if sc.priority == "constant" else coloring_priorities(A)
         Db = D.astype(bool)
         seq = limit_computation_levels(Db, self.max_num_CLs) if self.max_num_CLs < n else Db
@@ -794,8 +893,17 @@ class ScenarioRunner:
         sc, mpa = self.sc, self.mpa
         n, Hp = sc.amount, mpa.Hp
         self.k += 1
+        if self.coupled_fn is not None:
+            speed = np.array([mpa.trim_speed[self.trim[i] - 1] for i in range(n)], dtype=np.float64)
+            ids = self.path_id0 + np.arange(n)
+            res, rel = self.coupled_fn(ids, self.pose[:, 0], self.pose[:, 1], self.pose[:, 2], speed, self.trim, ids,
+                                       VEH_LENGTH / 2 + 0.01, VEH_WIDTH / 2 + 0.01, mpa.dt_seconds, sc.checker, sc.priority,
+                                       self.max_num_CLs)
+            self.apply_final(res)
+            self.timestep_records.append((self.k, None, rel, res))
+            return res
         if self.states_fn is not None:
-            A = couple(sc, self.pose)
+            A = self._adjacency()
             D = (constant_priorities(A) if sc.priority == "constant" else coloring_priorities(A)).astype(bool)
             seq = limit_computation_levels(D, self.max_num_CLs) if self.max_num_CLs < n else D
             speed = np.array([mpa.trim_speed[self.trim[i] - 1] for i in range(n)], dtype=np.float64)
@@ -855,14 +963,15 @@ class ScenarioRunner:
         self.pose, self.trim = new_pose, new_trim
 
     def step(self) -> List[StepRecord]:
-        if self.timestep_fn is not None or self.closed_loop_fn is not None or self.states_fn is not None:
+        if (self.timestep_fn is not None or self.closed_loop_fn is not None or self.states_fn is not None
+                or self.coupled_fn is not None):
             self.step_timestep()
             return []
         sc, mpa = self.sc, self.mpa
         n, Hp = sc.amount, mpa.Hp
         self.k += 1
         iters = self._iters()
-        A = couple(sc, self.pose)
+        A = self._adjacency()
         D = constant_priorities(A) if sc.priority == "constant" else coloring_priorities(A)
         levels = kahn(D.astype(np.int64))
         shapes_now: List[Optional[List[np.ndarray]]] = [None] * n
@@ -1038,7 +1147,7 @@ class ExplorativeRunner(ScenarioRunner):
         n, Hp = sc.amount, mpa.Hp
         self.k += 1
         base = self._iters()
-        A = couple(sc, self.pose)
+        A = self._adjacency()
         D = (constant_priorities(A) if sc.priority == "constant" else coloring_priorities(A)).astype(bool)
         levels = kahn(D.astype(np.int64))
         n_cl = int(levels.max())

@@ -24,6 +24,8 @@
  *                                                            expand_node.m:15-75, are_constraints_satisfied_sat.m:37-44
  *   level loop + hand-over of predecessors' areas            hlc/controller/prioritized/PrioritizedSequentialController.m:74-92,
  *   (pdmpc_plan_timestep, optional)                          PrioritizedController.m:297-324,355-364,449-506
+ *   simultaneous prioritizations: permuted relations, costs, hlc/controller/prioritized/PrioritizedExplorativeController.m:
+ *   choice and commit (pdmpc_plan_timestep_explorative)      55-78,94-176
  *
  * Conventions
  *   - plain C, no C++ types, no exceptions cross this boundary; every call
@@ -528,6 +530,51 @@ int pdmpc_couple(pdmpc_handle *h, int32_t n, const double *x, const double *y, c
  * when they do not fit rel->idx_capacity. */
 int pdmpc_plan_timestep_from_states_coupled(pdmpc_handle *h, const pdmpc_timestep_states *st, const pdmpc_couple_params *prm,
                                             pdmpc_couple_out *rel, pdmpc_batch_out *out);
+
+/* ---- Simultaneous prioritizations (PrioritizedExplorativeController, hlc/controller/prioritized/
+ *      PrioritizedExplorativeController.m:21-176) for every scenario of the time step in ONE call (DESIGN.md §4.13):
+ *      every permutation of the computation levels is planned from the measured states as in
+ *      pdmpc_plan_timestep_from_states, the cheapest permutation per weakly connected sub-graph is chosen on the device
+ *      and its plans become the vehicles' closed-loop state.
+ *        - st: the n base rows (one per vehicle) as for pdmpc_plan_timestep_from_states; st->succ_ptr / succ_idx = the
+ *          directed coupling D (coupled rows of lower priority, pdmpc_couple's succ); st->par_* and st->pred_* must be
+ *          NULL (they are derived per permutation); base slots distinct.
+ *        - permuted relation (:55-78): lev_p(i) = perm_p[level(i) - 1]; an edge i -> j of D with lev_p(i) > lev_p(j) is
+ *          reversed.  level(i) < level(j) must hold on every edge of D, so every permuted relation is acyclic.  Per row:
+ *          standing successors from the permuted relation's row, sequential predecessors from its column, no parallel
+ *          predecessors (the controller has no level cut); fallback plans from the slot of the vehicle (read only).
+ *        - cost of a row (compute_solution_cost :94-109): g_path[Hp]; an exhausted row the squared distance of its
+ *          fallback trajectory to the reference trajectory, summed in numpy's pairwise order (DESIGN.md §4.13).
+ *        - choice (:124-176): per (permutation, sub-graph) the row costs summed in vehicle order from 0.0, rounded
+ *          sign(y) * floor(|y| + 0.5) / 1e8 with y = x * 1e8, first minimum over the permutations.
+ *        - commit: per vehicle the row of its sub-graph's chosen permutation becomes its slot's state; no other row
+ *          touches a slot.  An input error is reported before anything is launched and leaves the slots as they were.
+ *      rows_out: rows = sum_s P_s * n_s, row (s, p, v) = sum_{t<s} P_t * n_t + p * n_s + (v - scenario_ptr[s]); outputs as
+ *      pdmpc_plan_timestep_closed_loop (an exhausted row holds its fallback plan).
+ *      Errors (PDMPC_ERR_BAD_INPUT): malformed scenario_ptr / perm_ptr / perm_val_ptr, P_s < 1, a perm row that is not a
+ *      permutation of 1..L_s, a level < 1 or not increasing along an edge of D, an edge across scenarios or repeated,
+ *      repeated base slots, relations passed in, a vehicle with more predecessors in some permutation than
+ *      PDMPC_TIMESTEP_COLS allows, no pdmpc_closed_loop_reset. ---- */
+typedef struct pdmpc_explorative_in {
+    int32_t n_scenarios;            /* >= 1 */
+    const int32_t *scenario_ptr;    /* [S+1] base rows of scenario s: [ptr[s], ptr[s+1]), ptr[0] == 0, ptr[S] == n */
+    const int32_t *level;           /* [n] 1-based computation level of every base row; L_s = max level of scenario s */
+    const int32_t *perm_ptr;        /* [S+1] permutations of scenario s: [perm_ptr[s], perm_ptr[s+1]), at least one */
+    const int32_t *perm_val_ptr;    /* [S+1] values of scenario s in perm: [perm_val_ptr[s], perm_val_ptr[s+1]), P_s * L_s */
+    const int32_t *perm;            /* row-major P_s x L_s per scenario: row p = the new position (1..L_s) of level 1..L_s
+                                     * (computation_level_permutations; row 0 of the reference = identity) */
+} pdmpc_explorative_in;
+
+typedef struct pdmpc_explorative_out {   /* caller-owned host buffers; NULL fields are not copied back */
+    int32_t *belonging;      /* [n] 1-based weakly connected sub-graph of the base row within its scenario */
+    int32_t *chosen;         /* [n] 0-based permutation whose plan the base row executes */
+    int32_t *applied_row;    /* [n] row of rows_out holding that plan */
+    double *row_cost;        /* [rows] cost of every (permutation, vehicle) row, before rounding */
+    double *solution_cost;   /* [rows] per scenario a P_s x n_s block; (p, g-1) = rounded sum of sub-graph g; columns >= G_s are 0 */
+} pdmpc_explorative_out;
+
+int pdmpc_plan_timestep_explorative(pdmpc_handle *h, const pdmpc_timestep_states *st, const pdmpc_explorative_in *ex,
+                                    pdmpc_batch_out *rows_out, pdmpc_explorative_out *eo);
 
 /* Pinned host buffers for callers that want full-rate host<->device copies. */
 int pdmpc_host_alloc(void **p, size_t bytes);

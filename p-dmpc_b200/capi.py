@@ -35,7 +35,7 @@ EXPORTED_SYMBOLS = (
     "pdmpc_run_staged", "pdmpc_sync", "pdmpc_fetch_staged", "pdmpc_get_stats", "pdmpc_stream",
     "pdmpc_mcts_plan_batch", "pdmpc_mcts_run_staged", "pdmpc_set_cta_heap_smem", "pdmpc_plan_timestep",
     "pdmpc_set_pipeline_chunks", "pdmpc_measure_fp64_peak", "pdmpc_joint_plan_batch",
-    "pdmpc_couple", "pdmpc_plan_timestep_from_states_coupled",
+    "pdmpc_couple", "pdmpc_plan_timestep_from_states_coupled", "pdmpc_plan_timestep_explorative",
 )
 
 _p_u8 = C.POINTER(C.c_uint8)
@@ -123,6 +123,16 @@ class CoupleOutC(C.Structure):
     _fields_ = [("succ_ptr", _p_i32), ("succ_idx", _p_i32), ("par_ptr", _p_i32), ("par_idx", _p_i32),
                 ("pred_ptr", _p_i32), ("pred_idx", _p_i32), ("idx_capacity", C.c_int32), ("level", _p_i32),
                 ("overlap_area", _p_f64)]
+
+
+class ExplorativeInC(C.Structure):
+    _fields_ = [("n_scenarios", C.c_int32), ("scenario_ptr", _p_i32), ("level", _p_i32), ("perm_ptr", _p_i32),
+                ("perm_val_ptr", _p_i32), ("perm", _p_i32)]
+
+
+class ExplorativeOutC(C.Structure):
+    _fields_ = [("belonging", _p_i32), ("chosen", _p_i32), ("applied_row", _p_i32), ("row_cost", _p_f64),
+                ("solution_cost", _p_f64)]
 
 
 MAX_PRED_LANELETS = 8
@@ -253,6 +263,9 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
     lib.pdmpc_plan_timestep_from_states_coupled.argtypes = [H, C.POINTER(TimestepStatesC), C.POINTER(CoupleParamsC),
                                                             C.POINTER(CoupleOutC), C.POINTER(BatchOut)]
     lib.pdmpc_plan_timestep_from_states_coupled.restype = C.c_int
+    lib.pdmpc_plan_timestep_explorative.argtypes = [H, C.POINTER(TimestepStatesC), C.POINTER(ExplorativeInC),
+                                                    C.POINTER(BatchOut), C.POINTER(ExplorativeOutC)]
+    lib.pdmpc_plan_timestep_explorative.restype = C.c_int
     lib.pdmpc_closed_loop_reset.argtypes = [H, C.c_int32, C.c_double, C.c_double]
     lib.pdmpc_closed_loop_reset.restype = C.c_int
     lib.pdmpc_plan_timestep_closed_loop.argtypes = [H, C.POINTER(BatchIn), C.POINTER(TimestepDepsC), _p_i32,
@@ -635,6 +648,61 @@ class Planner:
             bad = int(np.flatnonzero(r.status != PDMPC_OK)[0])
             raise PdmpcError(int(r.status[bad]), f"search {bad} failed")
         return r, self._relations(n, rel, keep)
+
+    def plan_timestep_explorative(self, path_id, x, y, yaw, speed, trim, slot, successors, level, permutations,
+                                  half_length: float, half_width: float, dt_seconds: float, checker: int, scenario_ptr=None,
+                                  raise_on_search_error: bool = True):
+        """Simultaneous prioritizations of every scenario in one call (pdmpc_plan_timestep_explorative): every permutation
+        planned from the measured states, the cheapest per weakly connected sub-graph chosen and committed to the slots.
+        successors: per base row the coupled rows of lower priority (global rows); level [n] 1-based; permutations: one
+        [P_s, L_s] array per scenario.  Returns (BatchResult of all P_s * n_s rows per scenario, dict with belonging [n],
+        chosen [n], applied_row [n], row_cost [rows] and solution_cost = one [P_s, G_s] array per scenario)."""
+        path_id, trim, slot, level = (np.ascontiguousarray(a, dtype=np.int32) for a in (path_id, trim, slot, level))
+        x, y, yaw, speed = (np.ascontiguousarray(a, dtype=np.float64) for a in (x, y, yaw, speed))
+        n, Hp = int(x.size), int(self.lib.pdmpc_get_hp(self.h))
+        sp = np.ascontiguousarray([0, n] if scenario_ptr is None else scenario_ptr, dtype=np.int32)
+        perms = [np.atleast_2d(np.asarray(p, dtype=np.int32)) for p in permutations]
+        S = int(sp.size - 1)
+        if len(perms) != S:
+            raise PdmpcError(PDMPC_ERR_BAD_INPUT, f"{len(perms)} permutation arrays for {S} scenarios")
+        pp = np.concatenate([[0], np.cumsum([p.shape[0] for p in perms])]).astype(np.int32)
+        pv = np.concatenate([[0], np.cumsum([p.size for p in perms])]).astype(np.int32)
+        pflat = np.ascontiguousarray(np.concatenate([p.reshape(-1) for p in perms] + [np.zeros(1, np.int32)]), dtype=np.int32)
+        sizes = np.diff(sp).astype(np.int64)
+        rows = int((np.diff(pp).astype(np.int64) * sizes).sum())
+        succ_ptr = np.zeros(n + 1, dtype=np.int32)
+        for i in range(n):
+            succ_ptr[i + 1] = succ_ptr[i] + len(successors[i])
+        succ_idx = np.ascontiguousarray(np.concatenate([np.asarray(r, dtype=np.int32) for r in successors] + [np.zeros(1, np.int32)]),
+                                        dtype=np.int32)
+        r = BatchResult.empty(rows, Hp)
+        bo = batch_out(r)
+        eo = {"belonging": np.zeros(max(n, 1), dtype=np.int32), "chosen": np.zeros(max(n, 1), dtype=np.int32),
+              "applied_row": np.zeros(max(n, 1), dtype=np.int32), "row_cost": np.zeros(max(rows, 1)),
+              "solution_cost": np.zeros(max(rows, 1))}
+        oc = ExplorativeOutC(**{k: _ptr(v, _p_i32 if v.dtype == np.int32 else _p_f64) for k, v in eo.items()})
+        ex = ExplorativeInC(n_scenarios=S, scenario_ptr=_ptr(sp, _p_i32), level=_ptr(level, _p_i32), perm_ptr=_ptr(pp, _p_i32),
+                            perm_val_ptr=_ptr(pv, _p_i32), perm=_ptr(pflat, _p_i32))
+        st = TimestepStatesC(n=n, path_id=_ptr(path_id, _p_i32), x=_ptr(x, _p_f64), y=_ptr(y, _p_f64), yaw=_ptr(yaw, _p_f64),
+                             speed=_ptr(speed, _p_f64), trim=_ptr(trim, _p_i32), succ_ptr=_ptr(succ_ptr, _p_i32),
+                             succ_idx=_ptr(succ_idx, _p_i32), slot=_ptr(slot, _p_i32),
+                             half_length=float(half_length), half_width=float(half_width), dt_seconds=float(dt_seconds),
+                             checker=int(checker))
+        self._check(self.lib.pdmpc_plan_timestep_explorative(self.h, C.byref(st), C.byref(ex), C.byref(bo), C.byref(oc)))
+        if raise_on_search_error and rows and int(r.status.max()) != PDMPC_OK:
+            bad = int(np.flatnonzero(r.status != PDMPC_OK)[0])
+            raise PdmpcError(int(r.status[bad]), f"row {bad} failed")
+        for k in ("belonging", "chosen", "applied_row"):
+            eo[k] = eo[k][:n]
+        eo["row_cost"] = eo["row_cost"][:rows]
+        sol, blocks, r0 = eo["solution_cost"], [], 0
+        for s in range(S):
+            ns, P = int(sizes[s]), int(pp[s + 1] - pp[s])
+            G = int(eo["belonging"][sp[s]:sp[s + 1]].max()) if ns else 0
+            blocks.append(sol[r0:r0 + P * ns].reshape(P, ns)[:, :G].copy())
+            r0 += P * ns
+        eo["solution_cost"] = blocks
+        return r, eo
 
     def joint_plan_batch(self, b: SearchBatch, n_vehicles: int, raise_on_search_error: bool = True) -> BatchResult:
         """Centralized (joint) searches: rows of `b` are searches x n_vehicles (pdmpc_joint_plan_batch)."""

@@ -25,6 +25,7 @@
 #include "pdmpc_fallback.cuh"
 #include "pdmpc_obstacles.cuh"
 #include "pdmpc_coupling.cuh"
+#include "pdmpc_explorative.cuh"
 
 using namespace pdmpc;
 
@@ -316,6 +317,8 @@ struct pdmpc_handle {
     ClosedLoopDev cl{};
     DBuf cl_valid, cl_trims, cl_traj, cl_npts, cl_sx, cl_sy;
     DBuf cf_slot, cf_still, cf_npts, cf_x, cf_y, cf_traj, cf_trims;
+    // the choice between prioritizations (pdmpc_plan_timestep_explorative)
+    DBuf e_bptr, e_rptr, e_bel, e_cost, e_sol, e_chosen, e_applied, e_commit;
 
     // trace (debug / parity tests)
     DBuf t_ids, t_n;
@@ -1468,9 +1471,12 @@ int pdmpc_plan_batch(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc_batch_out 
 // the device (pdmpc_fallback.cuh); deps->fb_* are then ignored.
 // `dev` != NULL: the batch is in device memory already (pdmpc_plan_timestep_from_states: its input arrays but the work
 // order, dev_totals = polygons, vertices, lanelet points); `in` then only carries n_searches, checker and dt_seconds.
+// `ex` != NULL (closed loop only): the rows are permutations of the same vehicles (pdmpc_plan_timestep_explorative); the
+// choice kernels run behind the searches and only the chosen rows are committed to the slots.
 static int plan_timestep_impl(pdmpc_handle *h, const pdmpc_batch_in *in, const pdmpc_timestep_deps *deps,
                               pdmpc_batch_out *out, const int32_t *slot, const uint8_t *standstill,
-                              const void **dev = nullptr, const int *dev_totals = nullptr) {
+                              const void **dev = nullptr, const int *dev_totals = nullptr,
+                              const ExplorativeDev *ex = nullptr) {
     if (!h) return PDMPC_ERR_BAD_INPUT;
     if (!h->has_mpa) return fail(h, PDMPC_ERR_NO_MPA, "plan_timestep: call pdmpc_upload_mpa first");
     if (!in || !deps || !deps->pred_ptr) return fail(h, PDMPC_ERR_BAD_INPUT, "plan_timestep: NULL argument");
@@ -1638,6 +1644,15 @@ static int plan_timestep_impl(pdmpc_handle *h, const pdmpc_batch_in *in, const p
                                                                       TraceDev{-1, nullptr, 0, nullptr}, dp);
     CU_TRY(h, cudaGetLastError());
     h->stats.kernel_launches++;
+    if (ex) {
+        explorative_row_cost_kernel<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(n, Hp, h->out, h->batch, fbd,
+                                                                                          ex->row_cost);
+        CU_TRY(h, cudaGetLastError());
+        explorative_choose_kernel<<<(unsigned)((ex->n_scenarios + 3) / 4), 128, 0, h->stream>>>(*ex);
+        CU_TRY(h, cudaGetLastError());
+        h->stats.kernel_launches += 2;
+        fbd.commit = ex->commit;
+    }
     if (closed_loop) {
         finalize_closed_loop_kernel<<<(unsigned)((nhp + 127) / 128), 128, 0, h->stream>>>(n, h->out, h->cl, fbd);
         CU_TRY(h, cudaGetLastError());
@@ -1700,8 +1715,9 @@ static int run_assemble_obstacles(pdmpc_handle *h, const pdmpc_coupling_in *in, 
 
 // One whole time step from the vehicles' measured states: inputs (pdmpc_inputs.cuh), obstacles that do not depend on this
 // step's plans (pdmpc_obstacles.cuh), dependency-ordered searches, fallback plans (pdmpc_fallback.cuh) — nothing of the
-// batch passes through the host.
-int pdmpc_plan_timestep_from_states(pdmpc_handle *h, const pdmpc_timestep_states *st, pdmpc_batch_out *out) {
+// batch passes through the host.  `ex` != NULL: the rows of pdmpc_plan_timestep_explorative, several per slot; the
+// choice commits one row per slot (plan_timestep_impl).
+static int plan_from_states(pdmpc_handle *h, const pdmpc_timestep_states *st, pdmpc_batch_out *out, const ExplorativeDev *ex) {
     if (!h) return PDMPC_ERR_BAD_INPUT;
     if (!h->has_mpa) return fail(h, PDMPC_ERR_NO_MPA, "plan_timestep_from_states: call pdmpc_upload_mpa first");
     if (!h->has_road) return fail(h, PDMPC_ERR_BAD_INPUT, "plan_timestep_from_states: call pdmpc_upload_road first");
@@ -1723,7 +1739,7 @@ int pdmpc_plan_timestep_from_states(pdmpc_handle *h, const pdmpc_timestep_states
         for (int i = 0; i < n; ++i) {
             if (st->path_id[i] < 0 || st->path_id[i] >= h->road.n_paths)
                 return fail(h, PDMPC_ERR_BAD_INPUT, "plan_timestep_from_states: path_id out of range");
-            if (st->slot[i] < 0 || st->slot[i] >= h->cl.n_slots || seen[st->slot[i]])
+            if (st->slot[i] < 0 || st->slot[i] >= h->cl.n_slots || (seen[st->slot[i]] && !ex))
                 return fail(h, PDMPC_ERR_BAD_INPUT, "plan_timestep_from_states: slots must be distinct and below n_slots");
             seen[st->slot[i]] = 1;
             still[i] = fabs(st->speed[i]) < kStandstillSpeed ? 1 : 0;   // PrioritizedController.m:580 / :527
@@ -1758,7 +1774,11 @@ int pdmpc_plan_timestep_from_states(pdmpc_handle *h, const pdmpc_timestep_states
     pdmpc_timestep_deps deps;
     memset(&deps, 0, sizeof(deps));
     deps.pred_ptr = st->pred_ptr; deps.pred_idx = st->pred_idx;
-    return plan_timestep_impl(h, &stub, &deps, out, st->slot, still.data(), dev, totals);
+    return plan_timestep_impl(h, &stub, &deps, out, st->slot, still.data(), dev, totals, ex);
+}
+
+int pdmpc_plan_timestep_from_states(pdmpc_handle *h, const pdmpc_timestep_states *st, pdmpc_batch_out *out) {
+    return plan_from_states(h, st, out, nullptr);
 }
 
 // Centralized (joint) search: rows = searches x n_vehicles (pdmpc_joint.cuh).
@@ -2329,6 +2349,175 @@ int pdmpc_plan_timestep_from_states_coupled(pdmpc_handle *h, const pdmpc_timeste
     s.par_ptr = r.ptr[1].data(); s.par_idx = r.idx[1].data();
     s.pred_ptr = r.ptr[2].data(); s.pred_idx = r.idx[2].data();
     return pdmpc_plan_timestep_from_states(h, &s, out);
+}
+
+// Simultaneous prioritizations (DESIGN.md §4.13): the base rows are expanded into one row per (scenario, permutation,
+// vehicle), each with the relation of its permutation, and planned by the one-call time step; the choice kernels
+// (pdmpc_explorative.cuh) then pick one permutation per sub-graph and commit its rows to the slots.
+int pdmpc_plan_timestep_explorative(pdmpc_handle *h, const pdmpc_timestep_states *st, const pdmpc_explorative_in *ex,
+                                    pdmpc_batch_out *rows_out, pdmpc_explorative_out *eo) {
+    if (!h) return PDMPC_ERR_BAD_INPUT;
+    const char *who = "plan_timestep_explorative: ";
+    auto bad = [&](const std::string &m) { return fail(h, PDMPC_ERR_BAD_INPUT, who + m); };
+    if (!h->has_mpa) return fail(h, PDMPC_ERR_NO_MPA, std::string(who) + "call pdmpc_upload_mpa first");
+    if (!h->has_road) return bad("call pdmpc_upload_road first");
+    if (h->cl.n_slots < 1 || h->cl.Hp != h->mpa.Hp) return bad("call pdmpc_closed_loop_reset first (after pdmpc_upload_mpa)");
+    if (!st || !ex || !rows_out || st->n < 0) return bad("states, permutations and the row outputs are required");
+    if (st->par_ptr || st->par_idx || st->pred_ptr || st->pred_idx)
+        return bad("the parallel and sequential relations are derived per permutation, pass NULL ones");
+    const int n = st->n, S = ex->n_scenarios, Hp = h->mpa.Hp;
+    if (S < 1 || !ex->scenario_ptr || !ex->level || !ex->perm_ptr || !ex->perm_val_ptr || !ex->perm || !st->succ_ptr ||
+        !st->slot || !st->path_id || !st->x || !st->y || !st->yaw || !st->speed || !st->trim)
+        return bad("NULL argument");
+    // ---- scenarios, levels, the directed coupling D and the base slots ---------------------------------------------
+    const int32_t *sp = ex->scenario_ptr, *pp = ex->perm_ptr, *pv = ex->perm_val_ptr;
+    if (sp[0] != 0 || sp[S] != n || pp[0] != 0 || pv[0] != 0) return bad("scenario_ptr, perm_ptr and perm_val_ptr must start at 0, scenario_ptr end at n");
+    std::vector<int> scen(n), L(S, 0);
+    for (int s = 0; s < S; ++s) {
+        if (sp[s + 1] < sp[s]) return bad("scenario_ptr not monotone");
+        if (pp[s + 1] - pp[s] < 1) return bad("every scenario needs at least one permutation");
+        for (int i = sp[s]; i < sp[s + 1]; ++i) {
+            if (ex->level[i] < 1) return bad("levels are 1-based");
+            scen[i] = s;
+            L[s] = std::max(L[s], (int)ex->level[i]);
+        }
+        if ((long long)pv[s + 1] - pv[s] != (long long)(pp[s + 1] - pp[s]) * L[s])
+            return bad("perm_val_ptr: scenario " + std::to_string(s) + " needs P_s * L_s values");
+    }
+    if (st->succ_ptr[0] != 0) return bad("succ_ptr must start at 0");
+    if (n && !st->succ_idx && st->succ_ptr[n] > 0) return bad("succ_idx is NULL");
+    std::vector<int> nb_ptr(n + 1, 0), stamp(n, -1);
+    for (int i = 0; i < n; ++i) {
+        if (st->succ_ptr[i + 1] < st->succ_ptr[i]) return bad("succ_ptr not monotone");
+        for (int q = st->succ_ptr[i]; q < st->succ_ptr[i + 1]; ++q) {
+            const int j = st->succ_idx[q];
+            if (j < 0 || j >= n || j == i || stamp[j] == i) return bad("succ_idx out of range or repeated");
+            stamp[j] = i;
+            if (scen[j] != scen[i]) return bad("a coupling edge crosses scenarios");
+            if (ex->level[i] >= ex->level[j]) return bad("level must increase along every coupling edge");
+            nb_ptr[i + 1]++;
+            nb_ptr[j + 1]++;
+        }
+    }
+    {
+        std::vector<char> seen((size_t)h->cl.n_slots, 0);
+        for (int i = 0; i < n; ++i) {
+            if (st->slot[i] < 0 || st->slot[i] >= h->cl.n_slots || seen[st->slot[i]])
+                return bad("base slots must be distinct and below n_slots");
+            if (st->path_id[i] < 0 || st->path_id[i] >= h->road.n_paths) return bad("path_id out of range");
+            seen[st->slot[i]] = 1;
+        }
+    }
+    // undirected neighbours U = D | D^T, ascending per row (the host loops run over the rows of a dense matrix)
+    for (int i = 0; i < n; ++i) nb_ptr[i + 1] += nb_ptr[i];
+    std::vector<int> nb(nb_ptr[n]);
+    {
+        std::vector<int> fill(nb_ptr.begin(), nb_ptr.end() - 1);
+        for (int i = 0; i < n; ++i)
+            for (int q = st->succ_ptr[i]; q < st->succ_ptr[i + 1]; ++q) {
+                nb[fill[i]++] = st->succ_idx[q];
+                nb[fill[st->succ_idx[q]]++] = i;
+            }
+        for (int i = 0; i < n; ++i) std::sort(nb.begin() + nb_ptr[i], nb.begin() + nb_ptr[i + 1]);
+    }
+    // permutations: each row of scenario s a permutation of 1..L_s
+    for (int s = 0; s < S; ++s)
+        for (int p = 0; p < pp[s + 1] - pp[s]; ++p) {
+            std::vector<char> hit(L[s] + 1, 0);
+            for (int l = 0; l < L[s]; ++l) {
+                const int v = ex->perm[pv[s] + (size_t)p * L[s] + l];
+                if (v < 1 || v > L[s] || hit[v]) return bad("permutation " + std::to_string(p) + " of scenario " + std::to_string(s) + " is not a permutation of 1..L_s");
+                hit[v] = 1;
+            }
+        }
+    // weakly connected sub-graphs, labelled in the order of their lowest row (scenario.weak_components)
+    std::vector<int> belonging(n, 0);
+    for (int s = 0; s < S; ++s) {
+        int label = 0;
+        for (int r = sp[s]; r < sp[s + 1]; ++r) {
+            if (belonging[r]) continue;
+            belonging[r] = ++label;
+            std::vector<int> stack{r};
+            while (!stack.empty()) {
+                const int u = stack.back();
+                stack.pop_back();
+                for (int q = nb_ptr[u]; q < nb_ptr[u + 1]; ++q)
+                    if (!belonging[nb[q]]) {
+                        belonging[nb[q]] = label;
+                        stack.push_back(nb[q]);
+                    }
+            }
+        }
+    }
+    // ---- the rows: (s, p, v) -> row_ptr[s] + p * n_s + (v - sp[s]); Dp orients U from the lower permuted level -------
+    std::vector<int> row_ptr(S + 1, 0);
+    for (int s = 0; s < S; ++s) {
+        const long long r = (long long)row_ptr[s] + (long long)(pp[s + 1] - pp[s]) * (sp[s + 1] - sp[s]);
+        if (r > 0x3fffffff) return bad("too many rows");
+        row_ptr[s + 1] = (int)r;
+    }
+    const int R = row_ptr[S];
+    std::vector<int32_t> pid(R), trim(R), slot(R), succ_ptr(R + 1, 0), pred_ptr(R + 1, 0), par_ptr(R + 1, 0), succ, pred;
+    std::vector<double> x(R), y(R), yaw(R), speed(R);
+    for (int s = 0; s < S; ++s) {
+        const int ns = sp[s + 1] - sp[s];
+        for (int p = 0; p < pp[s + 1] - pp[s]; ++p) {
+            const int32_t *perm = ex->perm + pv[s] + (size_t)p * L[s];
+            const int rb = row_ptr[s] + p * ns - sp[s];   // row of base row v: rb + v
+            for (int v = sp[s]; v < sp[s + 1]; ++v) {
+                const int r = rb + v;
+                pid[r] = st->path_id[v]; trim[r] = st->trim[v]; slot[r] = st->slot[v];
+                x[r] = st->x[v]; y[r] = st->y[v]; yaw[r] = st->yaw[v]; speed[r] = st->speed[v];
+                const int lv = perm[ex->level[v] - 1];
+                int np = 0;
+                for (int q = nb_ptr[v]; q < nb_ptr[v + 1]; ++q) {
+                    const int u = nb[q], lu = perm[ex->level[u] - 1];
+                    if (lu > lv) succ.push_back(rb + u);
+                    else {
+                        pred.push_back(rb + u);
+                        ++np;
+                    }
+                }
+                if ((long long)np * Hp * PDMPC_AREA_STRIDE > PDMPC_TIMESTEP_COLS)
+                    return bad("a vehicle has too many predecessors in permutation " + std::to_string(p) + " (PDMPC_TIMESTEP_COLS)");
+                succ_ptr[r + 1] = (int)succ.size();
+                pred_ptr[r + 1] = (int)pred.size();
+            }
+        }
+    }
+    if (succ.empty()) succ.push_back(0);
+    if (pred.empty()) pred.push_back(0);
+    // ---- device buffers of the choice ----------------------------------------------------------------------------
+    CU_TRY(h, cudaSetDevice(h->device));
+    UP(h, h->e_bptr, sp, S + 1);
+    UP(h, h->e_rptr, row_ptr.data(), S + 1);
+    UP(h, h->e_bel, belonging.data(), n);
+    CU_TRY(h, h->e_cost.reserve(std::max(R, 1) * sizeof(double)));
+    CU_TRY(h, h->e_sol.reserve(std::max(R, 1) * sizeof(double)));
+    CU_TRY(h, h->e_commit.reserve(std::max(R, 1)));
+    CU_TRY(h, h->e_chosen.reserve(std::max(n, 1) * sizeof(int)));
+    CU_TRY(h, h->e_applied.reserve(std::max(n, 1) * sizeof(int)));
+    ExplorativeDev ed;
+    ed.n_scenarios = S;
+    ed.base_ptr = h->e_bptr.as<int>(); ed.row_ptr = h->e_rptr.as<int>(); ed.belonging = h->e_bel.as<int>();
+    ed.row_cost = h->e_cost.as<double>(); ed.solution_cost = h->e_sol.as<double>();
+    ed.chosen = h->e_chosen.as<int>(); ed.applied_row = h->e_applied.as<int>(); ed.commit = h->e_commit.as<unsigned char>();
+    pdmpc_timestep_states xs = *st;
+    xs.n = R;
+    xs.path_id = pid.data(); xs.x = x.data(); xs.y = y.data(); xs.yaw = yaw.data(); xs.speed = speed.data();
+    xs.trim = trim.data(); xs.slot = slot.data();
+    xs.succ_ptr = succ_ptr.data(); xs.succ_idx = succ.data();
+    xs.par_ptr = par_ptr.data(); xs.par_idx = nullptr;
+    xs.pred_ptr = pred_ptr.data(); xs.pred_idx = pred.data();
+    int rc = plan_from_states(h, &xs, rows_out, &ed);
+    if (rc != PDMPC_OK || !eo || R == 0) return rc;
+    if (eo->belonging) std::copy(belonging.begin(), belonging.end(), eo->belonging);
+    DOWN(h, eo->chosen, h->e_chosen, n);
+    DOWN(h, eo->applied_row, h->e_applied, n);
+    DOWN(h, eo->row_cost, h->e_cost, R);
+    DOWN(h, eo->solution_cost, h->e_sol, R);
+    CU_TRY(h, cudaStreamSynchronize(h->stream));
+    return PDMPC_OK;
 }
 
 }  // extern "C"

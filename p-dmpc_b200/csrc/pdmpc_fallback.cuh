@@ -35,6 +35,7 @@ struct FallbackDev {               // per row of the call
     double *fb_x, *fb_y;           // [n * Hp * kAreaStride]
     double *fb_traj;               // [n * Hp * 3]
     int *fb_trims;                 // [n * Hp]
+    const unsigned char *commit = nullptr;   // [n] finalize stores row r in its slot iff commit[r] (null: every row)
 };
 
 // one thread per (row, step)
@@ -77,7 +78,8 @@ __global__ void make_fallback_kernel(BatchDev b, ClosedLoopDev st, FallbackDev f
     }
 }
 
-// one thread per (row, step): exhausted searches take their fallback plan; every final plan becomes the slot's state
+// one thread per (row, step): exhausted searches take their fallback plan; every final plan (every committed one, when
+// fb.commit is set) becomes the slot's state
 __global__ void finalize_closed_loop_kernel(int n, OutDev o, ClosedLoopDev st, FallbackDev fb) {
     const int Hp = st.Hp;
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
@@ -93,6 +95,7 @@ __global__ void finalize_closed_loop_kernel(int n, OutDev o, ClosedLoopDev st, F
             o.shape_y[os * kAreaStride + i] = fb.fb_y[os * kAreaStride + i];
         }
     }
+    if (fb.commit && !fb.commit[row]) return;
     const size_t p = (size_t)fb.slot[row] * Hp + k;
     st.trims[p] = o.trims[(size_t)row * (Hp + 1) + k + 1];
     for (int c = 0; c < 3; ++c) st.traj[p * 3 + c] = o.y_predicted[os * 3 + c];

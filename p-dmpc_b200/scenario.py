@@ -1115,6 +1115,17 @@ def weak_components(D: np.ndarray) -> np.ndarray:
     return label
 
 
+def permuted_coupling(D: np.ndarray, levels: np.ndarray, perm: np.ndarray) -> np.ndarray:
+    """The directed coupling of one permutation of the computation levels (PrioritizedExplorativeController.m:55-78):
+    lev_p = perm[levels - 1] (i11changem), and every edge i -> j of D with lev_p(i) > lev_p(j) is reversed."""
+    lev_p = np.asarray(perm)[np.asarray(levels) - 1]
+    Dp = D.copy()
+    for i, j in zip(*np.nonzero(D)):
+        if lev_p[i] > lev_p[j]:
+            Dp[i, j], Dp[j, i] = False, True
+    return Dp
+
+
 class ExplorativeRunner(ScenarioRunner):
     """BASELINE configs[2]: simultaneous multiple prioritizations.  Every time step the n_CL computation
     levels of the base prioritisation are permuted n_CL times (Latin square), every permutation is solved
@@ -1129,26 +1140,28 @@ class ExplorativeRunner(ScenarioRunner):
     (plan_fallback :696-711); the winner does not re-seed the prioritizer (:169-173)."""
 
     def __init__(self, sc: Scenario, timestep_fn, rank: int = 0, world: int = 1, device=None, max_permutations: int = 0,
-                 fixed_permutations: int = 0, exchange=None):
+                 fixed_permutations: int = 0, exchange=None, explorative_fn=None, coupler: str = "corridor"):
         """fixed_permutations: exactly that many permutations per time step (fixed_permutation_set: BASELINE's 8).
         exchange(n_rows_local, n, fallback_rows, mine, P, belonging) -> (chosen, solution_cost, plans): replaces the
         host-side exchange below by one that starts from the plans in DEVICE memory (bench: pdmpc_pack_plan_rows +
-        one NCCL all_gather); fallback_rows [n, 2 + 21*Hp] = cost and plan a vehicle takes when its search is exhausted."""
-        super().__init__(sc, None, timestep_fn=timestep_fn)
+        one NCCL all_gather); fallback_rows [n, 2 + 21*Hp] = cost and plan a vehicle takes when its search is exhausted.
+        explorative_fn(path_id, x, y, yaw, speed, trim, slot, successors, level, permutations, half_length, half_width, dt,
+        checker) -> (BatchResult, choice) (capi.Planner.plan_timestep_explorative): the whole time step — inputs,
+        obstacles, every permutation's searches, fallback plans, the choice and the closed-loop state — in ONE call;
+        D, the levels and the permutations are still decided here; slot = path id = path_id0 + vehicle.
+        coupler: as ScenarioRunner's."""
+        super().__init__(sc, None, timestep_fn=timestep_fn, coupler=coupler)
+        self.explorative_fn = explorative_fn
         self.rank, self.world, self.device = rank, world, device
         self.max_permutations = max_permutations      # 0 = all n_CL
         self.fixed_permutations = fixed_permutations
         self.exchange = exchange
         self.explorative_records: List[dict] = []
 
-    def step(self):
-        from . import sharding
-        sc, mpa = self.sc, self.mpa
-        n, Hp = sc.amount, mpa.Hp
-        self.k += 1
-        base = self._iters()
+    def decide(self):
+        """Directed coupling D, computation levels and the permutations of this time step (self.k)."""
         A = self._adjacency()
-        D = (constant_priorities(A) if sc.priority == "constant" else coloring_priorities(A)).astype(bool)
+        D = (constant_priorities(A) if self.sc.priority == "constant" else coloring_priorities(A)).astype(bool)
         levels = kahn(D.astype(np.int64))
         n_cl = int(levels.max())
         if self.fixed_permutations:
@@ -1157,6 +1170,44 @@ class ExplorativeRunner(ScenarioRunner):
             perms = computation_level_permutations(n_cl, self.k)
         if self.max_permutations:
             perms = perms[: self.max_permutations]
+        return D, levels, perms
+
+    def explorative_args(self):
+        """(D, levels, perms) and the per-vehicle arguments of explorative_fn up to the permutations."""
+        D, levels, perms = self.decide()
+        mpa, n = self.mpa, self.sc.amount
+        speed = np.array([mpa.trim_speed[self.trim[i] - 1] for i in range(n)], dtype=np.float64)
+        ids = self.path_id0 + np.arange(n)
+        return (D, levels, perms), (ids, self.pose[:, 0], self.pose[:, 1], self.pose[:, 2], speed, self.trim, ids,
+                                    [np.flatnonzero(D[i, :]) for i in range(n)], levels)
+
+    def apply_explorative(self, res: BatchResult, choice: dict, decision) -> None:
+        """Take the winners of one explorative call (rows of res, choice of this scenario) and record the step."""
+        _D, levels, perms = decision
+        bel, chosen = np.asarray(choice["belonging"]), np.asarray(choice["chosen"])
+        rows = np.asarray(choice["applied_row"])
+        self.apply_final(dataclasses.replace(res, **{f.name: getattr(res, f.name)[rows] for f in dataclasses.fields(res)
+                                                     if isinstance(getattr(res, f.name), np.ndarray)}))
+        first = [int(np.flatnonzero(bel == g)[0]) for g in range(1, int(bel.max()) + 1)]
+        self.explorative_records.append({"step": self.k, "n_permutations": perms.shape[0], "n_levels": int(levels.max()),
+                                         "chosen": chosen[first].astype(np.int64), "solution_cost": choice["solution_cost"],
+                                         "searches_local": perms.shape[0] * self.sc.amount, "result_local": res})
+
+    def step(self):
+        from . import sharding
+        sc, mpa = self.sc, self.mpa
+        n, Hp = sc.amount, mpa.Hp
+        self.k += 1
+        if self.explorative_fn is not None:
+            decision, args = self.explorative_args()
+            res, choice = self.explorative_fn(*args, [decision[2]], VEH_LENGTH / 2 + 0.01, VEH_WIDTH / 2 + 0.01,
+                                              mpa.dt_seconds, sc.checker)
+            choice = dict(choice, solution_cost=choice["solution_cost"][0])
+            self.apply_explorative(res, choice, decision)
+            return []
+        base = self._iters()
+        D, levels, perms = self.decide()
+        n_cl = int(levels.max())
         P = perms.shape[0]
         belonging = weak_components(D)
         fallbacks = [self._fallback_plan(i) for i in range(n)]
@@ -1165,11 +1216,7 @@ class ExplorativeRunner(ScenarioRunner):
         mine = sharding.shard_block_cyclic(P, self.rank, self.world)
         batches, deps = [], []
         for p in mine:
-            lev_p = perms[p][levels - 1]                   # i11changem(levels, 1:n_CL, permutation), :55-59
-            Dp = D.copy()
-            for i, j in zip(*np.nonzero(D)):               # swap where the permuted levels invert the coupling, :66-78
-                if lev_p[i] > lev_p[j]:
-                    Dp[i, j], Dp[j, i] = False, True
+            Dp = permuted_coupling(D, levels, perms[p])
             its = []
             for i in range(n):
                 it = dataclasses.replace(base[i], obstacles=list(base[i].obstacles),
@@ -1257,6 +1304,31 @@ def lockstep_step(runners: Sequence[ScenarioRunner], timestep_fn) -> BatchResult
                                            if isinstance(getattr(res, f.name), np.ndarray)})
         r.apply_timestep(rows, fallbacks)
         off += n
+    return res
+
+
+def explorative_lockstep_step(runners: Sequence[ExplorativeRunner], explorative_fn) -> BatchResult:
+    """One time step of MANY explorative scenarios as ONE explorative_fn call (capi.Planner.plan_timestep_explorative with
+    scenario_ptr): every runner decides its coupling, levels and permutations on the host, then all permutations of all
+    scenarios are planned, chosen and committed together; each runner applies its winners."""
+    decisions, cols = [], None
+    for r in runners:
+        r.k += 1
+        d, args = r.explorative_args()
+        decisions.append(d)
+        cols = [list(a) for a in args] if cols is None else [c + list(a) for c, a in zip(cols, args)]
+    sizes = [r.sc.amount for r in runners]
+    sp = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
+    path_id, x, y, yaw, speed, trim, slot, succ, level = cols
+    succ = [np.asarray(sv) + sp[s] for s in range(len(runners)) for sv in succ[sp[s]:sp[s + 1]]]
+    r0 = runners[0]
+    res, choice = explorative_fn(np.array(path_id), np.array(x), np.array(y), np.array(yaw), np.array(speed), np.array(trim),
+                                 np.array(slot), succ, np.array(level), [d[2] for d in decisions], VEH_LENGTH / 2 + 0.01,
+                                 VEH_WIDTH / 2 + 0.01, r0.mpa.dt_seconds, r0.sc.checker, scenario_ptr=sp)
+    for s, (r, d) in enumerate(zip(runners, decisions)):
+        a, b = sp[s], sp[s + 1]
+        r.apply_explorative(res, {"belonging": choice["belonging"][a:b], "chosen": choice["chosen"][a:b],
+                                  "applied_row": choice["applied_row"][a:b], "solution_cost": choice["solution_cost"][s]}, d)
     return res
 
 

@@ -224,7 +224,8 @@ int pdmpc_set_cta_queue(pdmpc_handle *h, int32_t valid_only);
  * 8000 pops (1 in 10^5 of the road-network records) would hold a whole launch open for 40 ms.  A search that
  * reaches `pops` pops in a tile kernel is given up there and run from scratch by the CTA shape (4, or 5 after
  * pdmpc_set_cta_queue(1)) behind the tile kernel on the same stream.  0 = never; -1 (default) = by batch size:
- * 2560 pops, 3072 from 120 000 and 4096 from 300 000 searches per call (measured optima).  A list of at
+ * 2560 pops, 3072 from 120 000 and 4096 from 300 000 searches per call, fewer for the searches that start late
+ * in the work order (pdmpc_escalation_budgets; a pops > 0 is one budget for every search).  A list of at
  * most `short_list_max` searches (-1 = default, 3 per SM) runs with one master warp per CTA, all checker warps
  * serving it — the launch then ends with its longest search at 0.65 us per pop —, a longer one with several
  * masters per CTA.  Results do not depend on either; pdmpc_stats.escalated counts the searches that took this
@@ -251,6 +252,12 @@ int pdmpc_set_pipeline_chunks(pdmpc_handle *h, int32_t chunks);
  * pdmpc_set_pipeline_chunks(chunks) gives.  Chunks are of equal size, the first one half of that.
  * bounds: cap >= *n_chunks + 1 entries (PDMPC_ERR_CAPACITY otherwise, *n_chunks is still set). */
 int pdmpc_pipeline_bounds(int32_t n_searches, int32_t chunks, int32_t cap, int32_t *bounds, int32_t *n_chunks);
+
+/* The pop budgets of the throughput shapes under the default escalation threshold (pdmpc_set_escalation(-1, ..)) in a
+ * batch of n_searches (host-only, needs no device): budgets[i] = the pops after which the search at work position
+ * positions[i] (0 <= positions[i] < n_searches) is given up and run again by the CTA shape (0 = never).  A search that
+ * starts late in the work order gets fewer pops than one that starts early. */
+int pdmpc_escalation_budgets(int32_t n_searches, int32_t count, const int32_t *positions, int32_t *budgets);
 
 /* Diagnostics: the timeline of the LAST pipelined pdmpc_plan_batch call, per chunk: host_ms = host time since the start
  * of the call at which the chunk's copies and kernel had been enqueued (after its validation), in_ms / done_ms = device

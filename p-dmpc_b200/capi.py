@@ -30,7 +30,7 @@ PDMPC_ERR_ALLOC = 5
 
 EXPORTED_SYMBOLS = (
     "pdmpc_create", "pdmpc_destroy", "pdmpc_last_error", "pdmpc_abi_version",
-    "pdmpc_set_node_capacity", "pdmpc_set_variant", "pdmpc_set_tile_points", "pdmpc_set_cta_queue", "pdmpc_set_escalation", "pdmpc_get_hp", "pdmpc_pack_plan_rows", "pdmpc_upload_road", "pdmpc_sample_inputs", "pdmpc_upload_reachable_sets", "pdmpc_assemble_obstacles", "pdmpc_get_pipeline_timeline", "pdmpc_pipeline_bounds", "pdmpc_plan_timestep_from_states", "pdmpc_closed_loop_reset", "pdmpc_plan_timestep_closed_loop", "pdmpc_host_alloc", "pdmpc_host_free",
+    "pdmpc_set_node_capacity", "pdmpc_set_variant", "pdmpc_set_tile_points", "pdmpc_set_cta_queue", "pdmpc_set_escalation", "pdmpc_get_hp", "pdmpc_pack_plan_rows", "pdmpc_upload_road", "pdmpc_sample_inputs", "pdmpc_upload_reachable_sets", "pdmpc_assemble_obstacles", "pdmpc_get_pipeline_timeline", "pdmpc_pipeline_bounds", "pdmpc_escalation_budgets", "pdmpc_plan_timestep_from_states", "pdmpc_closed_loop_reset", "pdmpc_plan_timestep_closed_loop", "pdmpc_host_alloc", "pdmpc_host_free",
     "pdmpc_trace_staged", "pdmpc_upload_mpa", "pdmpc_plan_batch", "pdmpc_stage_batch",
     "pdmpc_run_staged", "pdmpc_sync", "pdmpc_fetch_staged", "pdmpc_get_stats", "pdmpc_stream",
     "pdmpc_mcts_plan_batch", "pdmpc_mcts_run_staged", "pdmpc_set_cta_heap_smem", "pdmpc_plan_timestep",
@@ -256,6 +256,8 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
     lib.pdmpc_get_pipeline_timeline.restype = C.c_int
     lib.pdmpc_pipeline_bounds.argtypes = [C.c_int32, C.c_int32, C.c_int32, _p_i32, C.POINTER(C.c_int32)]
     lib.pdmpc_pipeline_bounds.restype = C.c_int
+    lib.pdmpc_escalation_budgets.argtypes = [C.c_int32, C.c_int32, _p_i32, _p_i32]
+    lib.pdmpc_escalation_budgets.restype = C.c_int
     lib.pdmpc_plan_timestep_from_states.argtypes = [H, C.POINTER(TimestepStatesC), C.POINTER(BatchOut)]
     lib.pdmpc_plan_timestep_from_states.restype = C.c_int
     lib.pdmpc_couple.argtypes = [H, C.c_int32, _p_f64, _p_f64, _p_f64, _p_i32, C.POINTER(CoupleParamsC), C.POINTER(CoupleOutC)]
@@ -318,6 +320,18 @@ def pipeline_bounds(n_searches: int, chunks: int = 0, lib=None) -> np.ndarray:
     if rc != PDMPC_OK:
         raise PdmpcError(rc, "pdmpc_pipeline_bounds")
     return out[: n.value + 1].copy()
+
+
+def escalation_budgets(n_searches: int, positions, lib=None) -> np.ndarray:
+    """Pop budgets of the throughput shapes under the default escalation threshold for the searches at work positions
+    `positions` of a batch of n_searches (pdmpc_escalation_budgets; host-only)."""
+    lib = lib or load_library()
+    pos = np.ascontiguousarray(positions, dtype=np.int32)
+    out = np.zeros(pos.size, dtype=np.int32)
+    rc = lib.pdmpc_escalation_budgets(int(n_searches), pos.size, _ptr(pos, _p_i32), _ptr(out, _p_i32))
+    if rc != PDMPC_OK:
+        raise PdmpcError(rc, "pdmpc_escalation_budgets")
+    return out
 
 
 class PdmpcError(RuntimeError):

@@ -953,24 +953,43 @@ static int launch_warp_shape(pdmpc_handle *h, int shape, const BatchDev &bc, con
 // (profiles/r02j_escalation_threshold.txt): the larger the batch, the smaller the launch's tail is against its
 // body and the later giving up pays — 2560 pops is best at 56 k searches, 2560-3072 at 168 k, 4096 at 358 k.
 static int escalation_pops(const pdmpc_handle *h, int n) {
-    if (h->escalate_pops >= 0) return h->escalate_pops;
+    if (h && h->escalate_pops >= 0) return h->escalate_pops;
     return n >= 300000 ? 4096 : n >= 120000 ? 3072 : PDMPC_ESCALATE_POPS;
+}
+// The budget by work position under the default threshold (esc_budget: min(P_max, P_min + (n - p) / S)).  No single
+// threshold fits both ends of the work order: a search that starts late holds its SM open long after the list has run
+// dry, one that starts early has the whole launch to finish in.  P_min and S by batch size from a sweep at 358 400,
+// 168 000 and 56 000 records (profiles/r03_tail_schedule_sweep.txt): S = 64 / 96 keeps the escalation list at 136 / 232
+// / 331 searches, under the short-list gate of 3 per SM, and the tile tail shrinks more than the CTA phase grows.  An
+// explicit threshold (pdmpc_set_escalation) is one uniform budget.
+static void escalation_schedule(const pdmpc_handle *h, int n, int *p_min, int *slope) {
+    *p_min = 0;
+    *slope = 0;
+    if (h && h->escalate_pops >= 0) return;
+    *p_min = 1024;
+    *slope = n >= 120000 ? 64 : 96;
+    if (const char *e = getenv("PDMPC_ESC_MIN")) *p_min = atoi(e);     // experiments (tools/tail_anatomy.py)
+    if (const char *e = getenv("PDMPC_ESC_SLOPE")) *slope = atoi(e);   // 0: the uniform threshold
 }
 static bool escalation_on(const pdmpc_handle *h, int shape, int n) {
     return (shape == kShapeTile2 || shape == kShapeTile4) && escalation_pops(h, n) > 0 && cta_launchable(h, false) &&
            n > h->num_sms && h->batch.checker == PDMPC_CHECKER_INTERX;
 }
 
-// Resets the list (count, producers-done counter, entries = -1) on stream S and names it in the batch the tile
-// kernels get.
+// Resets the list (counts, producers-done counter, entries = -1) on stream S and names it in the batch the tile
+// kernels get (their work positions count from 0 of n; a pipeline chunk sets pos0).
 static int escalation_prepare(pdmpc_handle *h, int n, BatchDev *bt, cudaStream_t S) {
     CU_TRY(h, h->esc.reserve(((size_t)n + 4) * sizeof(int)));
     CU_TRY(h, cudaMemsetAsync(h->esc.p, 0, 4 * sizeof(int), S));
     CU_TRY(h, cudaMemsetAsync(h->esc.as<int>() + 4, 0xff, (size_t)n * sizeof(int), S));
     bt->pop_limit = escalation_pops(h, n);
+    escalation_schedule(h, n, &bt->pop_min, &bt->pop_slope);
+    bt->pos0 = 0;
+    bt->pos_n = (unsigned)n;
     bt->esc_count = h->esc.as<unsigned>();
     bt->esc_done = h->esc.as<unsigned>() + 1;
     bt->esc_list = h->esc.as<int>() + 4;
+    bt->esc_cap = (unsigned)n;
     return PDMPC_OK;
 }
 
@@ -985,11 +1004,13 @@ static int launch_escalated(pdmpc_handle *h, const ArenaDev &ar, int producers, 
     be.esc_count = h->esc.as<unsigned>();
     be.esc_done = h->esc.as<unsigned>() + 1;
     be.esc_list = h->esc.as<int>() + 4;
+    be.esc_cap = (unsigned)h->batch.n;
     be.esc_producers = (unsigned)producers;
     const int fast = h->cta_valid_only ? 1 : 0;
     unsigned *wc = h->work_counter.as<unsigned>();
     // a short list: one master per CTA, all twelve checkers serve it (0.65 us per pop: the launch then ends with
-    // its longest search, ~5 ms for 8000 pops); a long list: several masters per CTA
+    // its longest search, ~5 ms for 8000 pops); a long list: several masters per CTA.  Either way the searches given
+    // up at the full budget, the longest ones, are started first, one per SM (esc_item).
     be.esc_gate_lo = 0u; be.esc_gate_hi = (unsigned)(h->esc_short_list >= 0 ? h->esc_short_list : 3 * h->num_sms);
     KERNEL_CTA<<<h->num_sms, CtaShape<1, kCtaCheckers>::kThreads, sizeof(CtaSmemT), S>>>(
         h->mpa, be, h->out, ar, wc + 1, h->cta_heap_smem, fast, DepsDev{});
@@ -1000,6 +1021,13 @@ static int launch_escalated(pdmpc_handle *h, const ArenaDev &ar, int producers, 
     h->stats.kernel_launches += 2;
     return PDMPC_OK;
 }
+
+#ifdef PDMPC_TAIL_STAMPS
+__global__ void tail_stamps_reset_kernel() {   // minima (slots 0..2) start at the largest value, the rest at 0
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < kTailStampSlots) g_tail_stamps[i] = i < 3 ? ~0ull : 0ull;
+}
+#endif
 
 // Launches the search of the staged batch (results are identical for all shapes):
 //   the warp-level shapes see above;  kShapeCta / kShapeCtaValid are chosen for at most one search per SM
@@ -1048,6 +1076,9 @@ static int launch_search(pdmpc_handle *h, const TraceDev &tr) {
             rc = escalation_prepare(h, n, &bt, h->stream);
             if (rc != PDMPC_OK) return rc;
         }
+#ifdef PDMPC_TAIL_STAMPS
+        tail_stamps_reset_kernel<<<(kTailStampSlots + 255) / 256, 256, 0, h->stream>>>();
+#endif
         CU_TRY(h, cudaEventRecord(h->ev[2], h->stream));
         rc = launch_warp_shape(h, shape, bt, h->arena, wc, tr, h->stream);
         if (rc != PDMPC_OK) return rc;
@@ -1126,11 +1157,15 @@ struct PackDesc {
     int bytes[kNumOut], off[kNumOut];
     int row_bytes;
 };
-__global__ void pack_rows_kernel(PackDesc d, const unsigned *count, const int *list, unsigned char *rows) {
-    const unsigned n = *count;
+// The list comes out compacted (list_out[j] = search of row j).
+__global__ void pack_rows_kernel(PackDesc d, const unsigned *count, const int *list, unsigned cap, int *list_out,
+                                 unsigned char *rows) {
+    const unsigned n_full = count[0], n = n_full + count[2];
     const int lane = threadIdx.x % 32;
     for (unsigned j = blockIdx.x * (blockDim.x / 32) + threadIdx.x / 32; j < n; j += gridDim.x * (blockDim.x / 32)) {
-        const size_t si = (size_t)list[j];
+        const int si_j = *esc_item(list, cap, n_full, j);
+        if (lane == 0) list_out[j] = si_j;
+        const size_t si = (size_t)si_j;
         unsigned char *row = rows + (size_t)j * d.row_bytes;
         for (int f = 0; f < kNumOut; ++f) {
             if (!d.src[f]) continue;
@@ -1340,6 +1375,7 @@ static int plan_batch_pipelined(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc
         BatchDev bc = bproto;
         bc.n = s1 - s0;
         bc.order = b.order + s0;
+        bc.pos0 = (unsigned)s0;   // pop budgets by the position in the whole batch: only its end gets small ones
         unsigned *wc = h->wc_chunks.as<unsigned>() + c;
         if (launch_warp_shape(h, shape, bc, arena_from(h->arena, (size_t)(c % lanes) * slots), wc, tr, S) != PDMPC_OK)
             return bail(PDMPC_ERR_CUDA);
@@ -1380,9 +1416,10 @@ static int plan_batch_pipelined(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc
     CU_TRY(h, cudaEventRecord(h->ev[5], h->s_out));
     rc = pipeline_sync_all(h);
     if (rc != PDMPC_OK) return rc;
-    if (esc && *h->pin_esc.as<const unsigned>() > 0) {
-        // their output rows: packed on the device, one copy, scattered into the caller's arrays
-        const unsigned cnt = *h->pin_esc.as<const unsigned>();
+    const unsigned cnt = esc ? h->pin_esc.as<const unsigned>()[0] + h->pin_esc.as<const unsigned>()[2] : 0u;
+    if (cnt > 0) {
+        // their output rows: packed on the device behind the list of their searches, one copy, scattered into the
+        // caller's arrays
         PackDesc pd;
         int off = 0;
         for (int i = 0; i < kNumOut; ++i) {
@@ -1393,16 +1430,16 @@ static int plan_batch_pipelined(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc
         }
         pd.row_bytes = off;
         const size_t list_bytes = ((size_t)cnt * sizeof(int) + 15) / 16 * 16;
-        CU_TRY(h, h->esc_rows.reserve((size_t)cnt * off));
+        CU_TRY(h, h->esc_rows.reserve(list_bytes + (size_t)cnt * off));
         rc = ensure_pinned(h, h->pin_esc, list_bytes + (size_t)cnt * off);
         if (rc != PDMPC_OK) return rc;
+        unsigned char *rows = h->esc_rows.as<unsigned char>();
         pack_rows_kernel<<<std::min<unsigned>((cnt + 3) / 4, 256u), 128, 0, h->stream>>>(
-            pd, h->esc.as<unsigned>(), h->esc.as<int>() + 4, h->esc_rows.as<unsigned char>());
+            pd, h->esc.as<unsigned>(), h->esc.as<int>() + 4, (unsigned)n, reinterpret_cast<int *>(rows), rows + list_bytes);
         CU_TRY(h, cudaGetLastError());
         h->stats.kernel_launches++;
         unsigned char *pin = h->pin_esc.as<unsigned char>();
-        CU_TRY(h, cudaMemcpyAsync(pin, h->esc.as<int>() + 4, (size_t)cnt * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-        CU_TRY(h, cudaMemcpyAsync(pin + list_bytes, h->esc_rows.p, (size_t)cnt * off, cudaMemcpyDeviceToHost, h->stream));
+        CU_TRY(h, cudaMemcpyAsync(pin, rows, list_bytes + (size_t)cnt * off, cudaMemcpyDeviceToHost, h->stream));
         CU_TRY(h, cudaStreamSynchronize(h->stream));
         const int *list = reinterpret_cast<const int *>(pin);
         for (unsigned j = 0; j < cnt; ++j) {
@@ -1426,6 +1463,33 @@ int pdmpc_pipeline_bounds(int32_t n_searches, int32_t chunks, int32_t cap, int32
     for (size_t i = 0; i < bnd.size(); ++i) bounds[i] = bnd[i];
     return PDMPC_OK;
 }
+
+int pdmpc_escalation_budgets(int32_t n_searches, int32_t count, const int32_t *positions, int32_t *budgets) {
+    if (n_searches < 0 || count < 0 || (count && (!positions || !budgets))) return PDMPC_ERR_BAD_INPUT;
+    for (int i = 0; i < count; ++i)
+        if (positions[i] < 0 || positions[i] >= n_searches) return PDMPC_ERR_BAD_INPUT;
+    int p_min = 0, slope = 0;
+    escalation_schedule(nullptr, n_searches, &p_min, &slope);
+    const int p_max = escalation_pops(nullptr, n_searches);
+    for (int i = 0; i < count; ++i) budgets[i] = esc_budget(p_max, p_min, slope, (unsigned)n_searches, (unsigned)positions[i]);
+    return PDMPC_OK;
+}
+
+#ifdef PDMPC_TAIL_STAMPS
+// Launch anatomy of the last pdmpc_run_staged (g_tail_stamps, pdmpc_kernels.cuh); out[5] / out[6] = searches escalated
+// at the full / a reduced budget.  Built with -DPDMPC_TAIL_STAMPS only (tools/tail_anatomy.py).
+int pdmpc_get_tail_stamps(pdmpc_handle *h, int32_t cap, unsigned long long *out) {
+    if (!h || !out || cap < 8) return PDMPC_ERR_BAD_INPUT;
+    CU_TRY(h, cudaSetDevice(h->device));
+    CU_TRY(h, cudaStreamSynchronize(h->stream));
+    CU_TRY(h, cudaMemcpyFromSymbol(out, g_tail_stamps, sizeof(unsigned long long) * std::min(cap, kTailStampSlots)));
+    unsigned cnt[4] = {0, 0, 0, 0};
+    if (h->esc.p) CU_TRY(h, cudaMemcpy(cnt, h->esc.p, sizeof(cnt), cudaMemcpyDeviceToHost));
+    out[5] = cnt[0];
+    out[6] = cnt[2];
+    return PDMPC_OK;
+}
+#endif
 
 int pdmpc_get_pipeline_timeline(pdmpc_handle *h, int32_t cap, double *host_ms, double *in_ms, double *done_ms, int32_t *n_chunks) {
     if (!h || !n_chunks) return PDMPC_ERR_BAD_INPUT;

@@ -159,6 +159,7 @@ search_cta_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_co
     // with esc_gate_lo < count <= esc_gate_hi items (two instances with different NM share one list; the gate
     // is evaluated when the producers are done — until then the instance only waits).
     const bool polling = b.esc_producers > 0u;
+    if (polling && threadIdx.x == 0) TAIL_MIN(2);
     if (threadIdx.x < NC) sm.done[threadIdx.x] = 0u;
     if (threadIdx.x == 0) { sm.n_jobs = 0u; sm.rot = 0u; sm.masters_done = 0u; }
     for (int s = 0; s < NM; ++s)
@@ -411,11 +412,13 @@ search_cta_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_co
                     const int *cnt = reinterpret_cast<const int *>(b.esc_count);
                     // the gate needs the final count: wait for the producers (same stream: they are done)
                     while (ld_acquire_gpu(reinterpret_cast<const int *>(b.esc_done)) < (int)b.esc_producers) __nanosleep(2000);
-                    const int total = ld_acquire_gpu(cnt);
+                    const int n_full = ld_acquire_gpu(cnt), total = n_full + ld_acquire_gpu(cnt + 2);
                     if ((unsigned)total > b.esc_gate_lo && (unsigned)total <= b.esc_gate_hi) {
                         if (!first_item) next_item = atomicAdd(work_counter, 1u) + gridDim.x * NM;
-                        if ((int)next_item < total)
-                            while ((got = ld_acquire_gpu(b.esc_list + next_item)) < 0) __nanosleep(200);
+                        if ((int)next_item < total) {
+                            const int *e = esc_item(b.esc_list, b.esc_cap, (unsigned)n_full, next_item);
+                            while ((got = ld_acquire_gpu(e)) < 0) __nanosleep(200);
+                        }
                     }
                 }
                 first_item = false;
@@ -693,6 +696,7 @@ search_cta_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_co
     }
     // ---- the last master to run out of work releases the checkers -----------------------------------------
     unsigned fin = 0;
+    if (polling && lane == 0) TAIL_MAX(3);
     if (lane == 0) fin = atomicAdd(&sm.masters_done, 1u);
     fin = __shfl_sync(FULL, fin, 0);
     if (fin == NM - 1) {

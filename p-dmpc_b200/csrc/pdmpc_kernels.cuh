@@ -60,6 +60,31 @@
 #define PROF_FLUSH(o, lane0)
 #endif
 
+// Optional launch anatomy of the throughput launch (build with -DPDMPC_TAIL_STAMPS; tools/tail_anatomy.py):
+// %globaltimer stamps in ns, read back with pdmpc_get_tail_stamps.  Slots: [0] first tile CTA start (min),
+// [1] first fetch that found the work list empty (min), [2] first escalation CTA start (min), [3] last escalation
+// master done (max), [4] tile CTAs exited, [8 + i] exit of tile CTA i.  The default build has none of it.
+#ifdef PDMPC_TAIL_STAMPS
+constexpr int kTailStampSlots = 8 + 148 * 64;
+__device__ unsigned long long g_tail_stamps[kTailStampSlots];
+__device__ __forceinline__ unsigned long long tail_now() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+#define TAIL_MIN(i) atomicMin(g_tail_stamps + (i), tail_now())
+#define TAIL_MAX(i) atomicMax(g_tail_stamps + (i), tail_now())
+#define TAIL_EXIT(cta)                                                                     \
+    do {                                                                                   \
+        atomicAdd(g_tail_stamps + 4, 1ull);                                                \
+        if ((cta) < (unsigned)kTailStampSlots - 8u) g_tail_stamps[8 + (cta)] = tail_now(); \
+    } while (0)
+#else
+#define TAIL_MIN(i)
+#define TAIL_MAX(i)
+#define TAIL_EXIT(cta)
+#endif
+
 namespace pdmpc {
 
 constexpr int kWarp = 32;
@@ -88,13 +113,20 @@ struct BatchDev {
     const int *order;           // work item -> search index (heaviest-looking searches first), or null
     // pop_hash covers the popped nodes that passed their edge check only (pdmpc_set_cta_queue(1)); else every pop
     int hash_valid_only = 0;
-    // ESCALATION (throughput shapes -> CTA shape).  A tile kernel gives a search up after `pop_limit` pops and
-    // appends its index to esc_list[atomicAdd(esc_count)] (entries start as -1); every tile CTA counts itself in
-    // esc_done when it exits.  The CTA kernel launched behind it takes its work items from that list
-    // (esc_producers = CTAs of the tile kernel(s) > 0 selects this mode) once all producers are done.
+    // ESCALATION (throughput shapes -> CTA shape).  A tile kernel gives a search up after its pop budget
+    // (esc_budget) and appends its index to the list esc_list[0, esc_cap) (entries start as -1): a search given up
+    // at the full budget `pop_limit` at esc_list[atomicAdd(esc_count)], one given up at a reduced budget at
+    // esc_list[esc_cap - 1 - atomicAdd(esc_count + 2)].  Every tile CTA counts itself in esc_done when it exits.
+    // The CTA kernel launched behind it takes its work items from that list (esc_producers = CTAs of the tile
+    // kernel(s) > 0 selects this mode) once all producers are done: the full-budget ones first (esc_item).
     int pop_limit = 0;
+    // position schedule (pop_slope > 0): the search at work position p (of pos_n in the whole batch; a chunk's item
+    // 0 is at pos0) gets min(pop_limit, pop_min + (pos_n - p) / pop_slope) pops
+    int pop_min = 0, pop_slope = 0;
+    unsigned pos0 = 0, pos_n = 0;
     int *esc_list = nullptr;
     unsigned *esc_count = nullptr, *esc_done = nullptr;
+    unsigned esc_cap = 0;
     unsigned esc_producers = 0;
     unsigned esc_gate_lo = 0, esc_gate_hi = 0xffffffffu;   // the CTA kernel instance runs iff lo < count <= hi
     const double *x0, *y0, *yaw0;
@@ -148,6 +180,18 @@ __device__ __forceinline__ int ld_acquire_gpu(const int *p) {
 }
 __device__ __forceinline__ void st_release_gpu(int *p, int v) {
     asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+
+// Pop budget of the search at work position p < n (BatchDev::pop_min / pop_slope): the searches that start late get
+// fewer pops before they are escalated, so none of them runs on long after the work list is empty.  Host and device.
+__host__ __device__ inline int esc_budget(int p_max, int p_min, int slope, unsigned n, unsigned p) {
+    if (slope <= 0) return p_max;
+    const unsigned b = (unsigned)p_min + (n - p) / (unsigned)slope;
+    return b < (unsigned)p_max ? (int)b : p_max;
+}
+// Item i of a complete escalation list with n_full full-budget entries (BatchDev::esc_list).
+__device__ __forceinline__ const int *esc_item(const int *list, unsigned cap, unsigned n_full, unsigned i) {
+    return i < n_full ? list + i : list + (cap - 1u - (i - n_full));
 }
 
 // Node arena + heap overflow of one resident tile ("slot"), all in HBM.

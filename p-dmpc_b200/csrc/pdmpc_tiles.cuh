@@ -105,6 +105,7 @@ struct __align__(16) TileSm {
     int si, trim0, nlan, status;
     unsigned goal;
     int exhausted;
+    int budget;                             // pops before the search is escalated (esc_budget of its work position)
 };
 
 
@@ -182,13 +183,15 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
     int n_nodes = 0, n_pops = 0;
     unsigned long long hash = 0, cols = 0;
 
+    if (lane == 0) TAIL_MIN(0);
     for (;;) {
-        if (phase == RUN && b.pop_limit > 0 && n_pops >= b.pop_limit) {
+        if (phase == RUN && b.pop_limit > 0 && n_pops >= sm.budget) {
             // ---- escalation: a search this long is the tail of the launch; the CTA shape behind this kernel
             //      runs it from scratch at a fraction of the per-pop latency.  Nothing of it is written here.
             if (tl == 0) {
-                const unsigned q = atomicAdd(b.esc_count, 1u);
-                st_release_gpu(b.esc_list + q, sm.si);
+                const bool full = sm.budget >= b.pop_limit;   // the full-budget ones are the longest: run first
+                const unsigned q = atomicAdd(b.esc_count + (full ? 0 : 2), 1u);
+                st_release_gpu(b.esc_list + (full ? q : b.esc_cap - 1u - q), sm.si);
             }
             phase = IDLE;
         }
@@ -204,7 +207,11 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
             unsigned si_u = 0;
             if (tl == 0) si_u = atomicAdd(work_counter, 1u);
             si_u = __shfl_sync(tmask, si_u, shift);
-            if (si_u >= (unsigned)b.n) { phase = EXIT; break; }
+            if (si_u >= (unsigned)b.n) {
+                if (tl == 0) TAIL_MIN(1);
+                phase = EXIT;
+                break;
+            }
             const int si = b.order ? __ldg(b.order + si_u) : (int)si_u;
             __syncwarp(tmask);
             stage_reference(b, si, Hp, sm.refx, sm.refy, sm.vref, t);
@@ -226,6 +233,7 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
                 sm.op = ost ? sm.pts + (lst ? nl : 0) : b.pl_xy + pl.ob_lo;
                 sm.si = si; sm.trim0 = trim0; sm.nlan = nl;
                 sm.status = PDMPC_OK; sm.goal = 0; sm.exhausted = 0;
+                sm.budget = esc_budget(b.pop_limit, b.pop_min, b.pop_slope, b.pos_n, b.pos0 + si_u);
                 h_st(0, init_root(b, si, trim0, node(ar.a, 0), node(ar.b, 0), node(ar.cs, 0)));
             }
             len = 1;
@@ -562,6 +570,7 @@ search_tile_kernel(MpaDev m, BatchDev b, OutDev o, ArenaDev ar, unsigned *work_c
         __threadfence();
         if (lane == 0) atomicAdd(b.esc_done, 1u);
     }
+    if (lane == 0) TAIL_EXIT(blockIdx.x);
 }
 
 }  // namespace pdmpc

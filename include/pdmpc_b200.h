@@ -496,6 +496,27 @@ typedef struct pdmpc_timestep_states {
 } pdmpc_timestep_states;
 int pdmpc_plan_timestep_from_states(pdmpc_handle *h, const pdmpc_timestep_states *states, pdmpc_batch_out *out);
 
+/* ---- Time steps with the sampled optimizer (MonteCarloTreeSearch.run_optimizer as the optimizer of
+ *      PrioritizedController.plan, DESIGN.md §4.14): pdmpc_plan_timestep, pdmpc_plan_timestep_closed_loop and
+ *      pdmpc_plan_timestep_from_states with one warp per sampled search (pdmpc_mcts_plan_batch's kernel) instead of the
+ *      graph search.  prm->seed[i] is row i's RandStream seed (time_step + vehicle_index, both 1-based), the same
+ *      n_expansions_max for every row.  A row is exhausted when no valid depth-Hp leaf was found or its status is not
+ *      PDMPC_OK (PDMPC_ERR_CAPACITY: the roll-outs would read past the Hp * n_expansions_max random numbers); it then
+ *      publishes its fallback areas like an exhausted graph search, and its status is reported.  Output fields as
+ *      pdmpc_mcts_plan_batch; every one equals level-by-level pdmpc_mcts_plan_batch calls with host-side obstacle
+ *      assembly.  The relation checks, the work order, the fallback plans and the closed-loop slots are those of the
+ *      graph-search calls.  No node arena; pdmpc_set_variant has no effect and pdmpc_stats.shape reports 1.
+ *      Errors (before anything is launched): those of the graph-search call, PDMPC_ERR_BAD_INPUT for n_expansions_max
+ *      outside 1..PDMPC_MCTS_MAX_EXPANSIONS, NULL seeds with n > 0 or a branching factor above PDMPC_MCTS_MAX_BRANCH,
+ *      PDMPC_ERR_CAPACITY when the sampled tree does not fit in shared memory. ---- */
+int pdmpc_mcts_plan_timestep(pdmpc_handle *h, const pdmpc_batch_in *in, const pdmpc_timestep_deps *deps,
+                             const pdmpc_mcts_params *prm, pdmpc_batch_out *out);
+int pdmpc_mcts_plan_timestep_closed_loop(pdmpc_handle *h, const pdmpc_batch_in *in, const pdmpc_timestep_deps *deps,
+                                         const int32_t *slot, const uint8_t *standstill,
+                                         const pdmpc_mcts_params *prm, pdmpc_batch_out *out);
+int pdmpc_mcts_plan_timestep_from_states(pdmpc_handle *h, const pdmpc_timestep_states *st,
+                                         const pdmpc_mcts_params *prm, pdmpc_batch_out *out);
+
 /* ---- Coupling, priorities and computation levels of a time step on the device: what the host decides before
  *      pdmpc_plan_timestep_from_states, for every scenario of the time step in one call (DESIGN.md §4.12).
  *        - coupling (ReachableSetCoupler.m:5-54): rows i, j of one scenario are coupled iff the step-Hp reachable sets of

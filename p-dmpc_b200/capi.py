@@ -36,6 +36,7 @@ EXPORTED_SYMBOLS = (
     "pdmpc_mcts_plan_batch", "pdmpc_mcts_run_staged", "pdmpc_set_cta_heap_smem", "pdmpc_plan_timestep",
     "pdmpc_set_pipeline_chunks", "pdmpc_measure_fp64_peak", "pdmpc_joint_plan_batch",
     "pdmpc_couple", "pdmpc_plan_timestep_from_states_coupled", "pdmpc_plan_timestep_explorative",
+    "pdmpc_mcts_plan_timestep", "pdmpc_mcts_plan_timestep_closed_loop", "pdmpc_mcts_plan_timestep_from_states",
 )
 
 _p_u8 = C.POINTER(C.c_uint8)
@@ -305,6 +306,15 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
     lib.pdmpc_mcts_run_staged.restype = C.c_int
     lib.pdmpc_plan_timestep.argtypes = [H, C.POINTER(BatchIn), C.POINTER(TimestepDepsC), C.POINTER(BatchOut)]
     lib.pdmpc_plan_timestep.restype = C.c_int
+    lib.pdmpc_mcts_plan_timestep.argtypes = [H, C.POINTER(BatchIn), C.POINTER(TimestepDepsC), C.POINTER(MctsParams),
+                                             C.POINTER(BatchOut)]
+    lib.pdmpc_mcts_plan_timestep.restype = C.c_int
+    lib.pdmpc_mcts_plan_timestep_closed_loop.argtypes = [H, C.POINTER(BatchIn), C.POINTER(TimestepDepsC), _p_i32,
+                                                         C.POINTER(C.c_uint8), C.POINTER(MctsParams), C.POINTER(BatchOut)]
+    lib.pdmpc_mcts_plan_timestep_closed_loop.restype = C.c_int
+    lib.pdmpc_mcts_plan_timestep_from_states.argtypes = [H, C.POINTER(TimestepStatesC), C.POINTER(MctsParams),
+                                                         C.POINTER(BatchOut)]
+    lib.pdmpc_mcts_plan_timestep_from_states.restype = C.c_int
     lib.pdmpc_stream.argtypes = [H]
     lib.pdmpc_stream.restype = C.c_void_p
     _LIB = lib
@@ -535,13 +545,27 @@ class Planner:
     def plan_timestep(self, b: SearchBatch, deps, raise_on_search_error: bool = True) -> BatchResult:
         """All searches of one (or many) time steps in one dependency-ordered launch
         (pdmpc_plan_timestep): PrioritizedController.plan's hand-over of predecessors' areas on the device."""
+        return self._timestep(b, deps, None, raise_on_search_error)
+
+    def mcts_plan_timestep(self, b: SearchBatch, deps, seeds, n_expansions_max: int = 250,
+                           raise_on_search_error: bool = True) -> BatchResult:
+        """plan_timestep with MonteCarloTreeSearch as the optimizer (pdmpc_mcts_plan_timestep); seeds[i] = time_step +
+        vehicle_index of row i."""
+        return self._timestep(b, deps, (seeds, n_expansions_max), raise_on_search_error)
+
+    def _timestep(self, b: SearchBatch, deps, mcts, raise_on_search_error: bool) -> BatchResult:
         self._check_hp(b)
         r = BatchResult.empty(b.n, b.Hp)
         bi, bo = batch_in(b), batch_out(r)
         pidx = deps.pred_idx if deps.pred_idx.size else np.zeros(1, dtype=np.int32)
         d = TimestepDepsC(pred_ptr=_ptr(deps.pred_ptr, _p_i32), pred_idx=_ptr(pidx, _p_i32),
                           fb_npts=_ptr(deps.fb_npts, _p_i32), fb_x=_ptr(deps.fb_x, _p_f64), fb_y=_ptr(deps.fb_y, _p_f64))
-        self._check(self.lib.pdmpc_plan_timestep(self.h, C.byref(bi), C.byref(d), C.byref(bo)))
+        if mcts is None:
+            self._check(self.lib.pdmpc_plan_timestep(self.h, C.byref(bi), C.byref(d), C.byref(bo)))
+        else:
+            prm, keep = mcts_params(mcts[0], mcts[1], b.n)
+            self._check(self.lib.pdmpc_mcts_plan_timestep(self.h, C.byref(bi), C.byref(d), C.byref(prm), C.byref(bo)))
+            del keep
         if raise_on_search_error and b.n and int(r.status.max()) != PDMPC_OK:
             bad = int(np.flatnonzero(r.status != PDMPC_OK)[0])
             raise PdmpcError(int(r.status[bad]), f"search {bad} failed")
@@ -554,6 +578,14 @@ class Planner:
     def plan_timestep_closed_loop(self, b: SearchBatch, deps, slot, standstill, raise_on_search_error: bool = True) -> BatchResult:
         """pdmpc_plan_timestep_closed_loop: like plan_timestep, but the fallback plans of exhausted vehicles are built on
         the device from the previous time step's plans kept there; exhausted rows return their fallback plan."""
+        return self._closed_loop(b, deps, slot, standstill, None, raise_on_search_error)
+
+    def mcts_plan_timestep_closed_loop(self, b: SearchBatch, deps, slot, standstill, seeds, n_expansions_max: int = 250,
+                                       raise_on_search_error: bool = True) -> BatchResult:
+        """plan_timestep_closed_loop with MonteCarloTreeSearch as the optimizer (pdmpc_mcts_plan_timestep_closed_loop)."""
+        return self._closed_loop(b, deps, slot, standstill, (seeds, n_expansions_max), raise_on_search_error)
+
+    def _closed_loop(self, b: SearchBatch, deps, slot, standstill, mcts, raise_on_search_error: bool) -> BatchResult:
         self._check_hp(b)
         r = BatchResult.empty(b.n, b.Hp)
         bi, bo = batch_in(b), batch_out(r)
@@ -561,8 +593,15 @@ class Planner:
         d = TimestepDepsC(pred_ptr=_ptr(deps.pred_ptr, _p_i32), pred_idx=_ptr(pidx, _p_i32), fb_npts=None, fb_x=None, fb_y=None)
         slot = np.ascontiguousarray(slot, dtype=np.int32)
         still = np.ascontiguousarray(standstill, dtype=np.uint8)
-        self._check(self.lib.pdmpc_plan_timestep_closed_loop(self.h, C.byref(bi), C.byref(d), _ptr(slot, _p_i32),
-                                                             _ptr(still, C.POINTER(C.c_uint8)), C.byref(bo)))
+        if mcts is None:
+            self._check(self.lib.pdmpc_plan_timestep_closed_loop(self.h, C.byref(bi), C.byref(d), _ptr(slot, _p_i32),
+                                                                 _ptr(still, C.POINTER(C.c_uint8)), C.byref(bo)))
+        else:
+            prm, keep = mcts_params(mcts[0], mcts[1], b.n)
+            self._check(self.lib.pdmpc_mcts_plan_timestep_closed_loop(self.h, C.byref(bi), C.byref(d), _ptr(slot, _p_i32),
+                                                                      _ptr(still, C.POINTER(C.c_uint8)), C.byref(prm),
+                                                                      C.byref(bo)))
+            del keep
         if raise_on_search_error and b.n and int(r.status.max()) != PDMPC_OK:
             bad = int(np.flatnonzero(r.status != PDMPC_OK)[0])
             raise PdmpcError(int(r.status[bad]), f"search {bad} failed")
@@ -574,6 +613,18 @@ class Planner:
         """One whole time step from the measured states (pdmpc_plan_timestep_from_states): inputs, obstacle assembly,
         dependency-ordered searches and fallback plans chained on the device.  successors / parallel / predecessors:
         per row a sequence of row indices.  Exhausted rows return their fallback plan."""
+        return self._from_states(path_id, x, y, yaw, speed, trim, successors, parallel, predecessors, slot, half_length,
+                                 half_width, dt_seconds, checker, None, raise_on_search_error)
+
+    def mcts_plan_timestep_from_states(self, path_id, x, y, yaw, speed, trim, successors, parallel, predecessors, slot,
+                                       half_length: float, half_width: float, dt_seconds: float, checker: int, seeds,
+                                       n_expansions_max: int = 250, raise_on_search_error: bool = True) -> BatchResult:
+        """plan_timestep_from_states with MonteCarloTreeSearch as the optimizer (pdmpc_mcts_plan_timestep_from_states)."""
+        return self._from_states(path_id, x, y, yaw, speed, trim, successors, parallel, predecessors, slot, half_length,
+                                 half_width, dt_seconds, checker, (seeds, n_expansions_max), raise_on_search_error)
+
+    def _from_states(self, path_id, x, y, yaw, speed, trim, successors, parallel, predecessors, slot, half_length,
+                     half_width, dt_seconds, checker, mcts, raise_on_search_error: bool) -> BatchResult:
         path_id, trim, slot = (np.ascontiguousarray(a, dtype=np.int32) for a in (path_id, trim, slot))
         x, y, yaw, speed = (np.ascontiguousarray(a, dtype=np.float64) for a in (x, y, yaw, speed))
         n, Hp = int(x.size), int(self.lib.pdmpc_get_hp(self.h))
@@ -595,7 +646,12 @@ class Planner:
                              pred_ptr=_ptr(dp, _p_i32), pred_idx=_ptr(di, _p_i32), slot=_ptr(slot, _p_i32),
                              half_length=float(half_length), half_width=float(half_width), dt_seconds=float(dt_seconds),
                              checker=int(checker))
-        self._check(self.lib.pdmpc_plan_timestep_from_states(self.h, C.byref(st), C.byref(bo)))
+        if mcts is None:
+            self._check(self.lib.pdmpc_plan_timestep_from_states(self.h, C.byref(st), C.byref(bo)))
+        else:
+            prm, keep = mcts_params(mcts[0], mcts[1], n)
+            self._check(self.lib.pdmpc_mcts_plan_timestep_from_states(self.h, C.byref(st), C.byref(prm), C.byref(bo)))
+            del keep
         if raise_on_search_error and n and int(r.status.max()) != PDMPC_OK:
             bad = int(np.flatnonzero(r.status != PDMPC_OK)[0])
             raise PdmpcError(int(r.status[bad]), f"search {bad} failed")

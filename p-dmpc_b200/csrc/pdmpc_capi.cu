@@ -519,6 +519,33 @@ static int download(pdmpc_handle *h, T *dst, const DBuf &buf, size_t count) {
     return PDMPC_OK;
 }
 
+// The sampled optimizer's parameters for n searches (pdmpc_mcts_params): every input error before anything is launched.
+static int mcts_check(pdmpc_handle *h, const pdmpc_mcts_params *prm, int n, MctsDev *mc, size_t *smem) {
+    if (!prm || prm->n_expansions_max < 1 || prm->n_expansions_max > PDMPC_MCTS_MAX_EXPANSIONS)
+        return fail(h, PDMPC_ERR_BAD_INPUT, "mcts: n_expansions_max out of range");
+    if (n && !prm->seed) return fail(h, PDMPC_ERR_BAD_INPUT, "mcts: seed is NULL");
+    if (h->max_branch > PDMPC_MCTS_MAX_BRANCH)
+        return fail(h, PDMPC_ERR_BAD_INPUT, "mcts: branching factor of the MPA exceeds PDMPC_MCTS_MAX_BRANCH");
+    mc->n_max = prm->n_expansions_max;
+    mc->node_cap = prm->n_expansions_max + h->mpa.Hp + 1;
+    mc->seed = nullptr;   // set once the seeds are uploaded
+    *smem = mcts_smem_bytes(mc->node_cap);
+    if (*smem > kSmemLimit) return fail(h, PDMPC_ERR_CAPACITY, "mcts: sampled tree does not fit in shared memory");
+    return PDMPC_OK;
+}
+
+// Grid of the sampled kernel over n searches: at most the one-warp CTAs that are resident at once (the DEPS instance
+// relies on it: a warp waits only for searches that resident warps have taken).
+template <bool DEPS>
+static int mcts_grid(pdmpc_handle *h, size_t smem, int n, int *grid) {
+    CU_TRY(h, cudaFuncSetAttribute(mcts_kernel<DEPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int occ = 0;
+    CU_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, mcts_kernel<DEPS>, kWarp, smem));
+    if (occ < 1) return fail(h, PDMPC_ERR_CUDA, "mcts: kernel is not launchable on this device");
+    *grid = std::min(n, h->num_sms * occ);
+    return PDMPC_OK;
+}
+
 extern "C" {
 
 int pdmpc_upload_mpa(pdmpc_handle *h, const pdmpc_mpa_desc *d) {
@@ -1537,19 +1564,27 @@ int pdmpc_plan_batch(pdmpc_handle *h, const pdmpc_batch_in *in, pdmpc_batch_out 
 // order, dev_totals = polygons, vertices, lanelet points); `in` then only carries n_searches, checker and dt_seconds.
 // `ex` != NULL (closed loop only): the rows are permutations of the same vehicles (pdmpc_plan_timestep_explorative); the
 // choice kernels run behind the searches and only the chosen rows are committed to the slots.
+// `mcts` != NULL: the searches are the sampled optimizer's (pdmpc_mcts_plan_timestep*): one warp per search
+// (mcts_kernel<true>), whatever pdmpc_set_variant says.
 static int plan_timestep_impl(pdmpc_handle *h, const pdmpc_batch_in *in, const pdmpc_timestep_deps *deps,
                               pdmpc_batch_out *out, const int32_t *slot, const uint8_t *standstill,
                               const void **dev = nullptr, const int *dev_totals = nullptr,
-                              const ExplorativeDev *ex = nullptr) {
+                              const ExplorativeDev *ex = nullptr, const pdmpc_mcts_params *mcts = nullptr) {
     if (!h) return PDMPC_ERR_BAD_INPUT;
     if (!h->has_mpa) return fail(h, PDMPC_ERR_NO_MPA, "plan_timestep: call pdmpc_upload_mpa first");
     if (!in || !deps || !deps->pred_ptr) return fail(h, PDMPC_ERR_BAD_INPUT, "plan_timestep: NULL argument");
     const int n = in->n_searches, Hp = h->mpa.Hp;
     if (n < 0) return fail(h, PDMPC_ERR_BAD_INPUT, "plan_timestep: n_searches < 0");
+    MctsDev mc{};
+    size_t mcts_smem = 0;
+    if (mcts) {
+        const int rc = mcts_check(h, mcts, n, &mc, &mcts_smem);
+        if (rc != PDMPC_OK) return rc;
+    }
     // launch shape: one CTA per search (lowest latency) for up to 48 searches per SM, else — and for search
     // trees beyond what that kernel holds — one warp per search; pdmpc_set_variant 1..3 / 4..5 force either
-    bool use_cta;
-    {
+    bool use_cta = false;
+    if (!mcts) {
         const bool cta_possible = cta_launchable(h, true);
         if (h->variant_mode >= kShapeCta) use_cta = cta_possible;
         else if (h->variant_mode >= kShapeLatency) use_cta = false;
@@ -1683,8 +1718,14 @@ static int plan_timestep_impl(pdmpc_handle *h, const pdmpc_batch_in *in, const p
     CU_TRY(h, cudaMemsetAsync(h->work_counter.p, 0, sizeof(unsigned), h->stream));
     const bool cta_single = n <= h->num_sms;
     const int cta_nm = cta_single ? 1 : kCtaMastersDeps;
-    const int grid = use_cta ? std::min((n + cta_nm - 1) / cta_nm, h->num_sms) : std::min(n, h->num_sms * h->lat_ctas_per_sm);
-    rc = ensure_arena(h, use_cta ? grid * cta_nm : grid);
+    int grid = use_cta ? std::min((n + cta_nm - 1) / cta_nm, h->num_sms) : std::min(n, h->num_sms * h->lat_ctas_per_sm);
+    if (mcts) {   // the sampled tree lives in shared memory: seeds instead of a node arena
+        rc = mcts_grid<true>(h, mcts_smem, n, &grid);
+        if (rc == PDMPC_OK) rc = upload(h, h->b_seed, mcts->seed, (size_t)n);
+        mc.seed = h->b_seed.as<unsigned>();
+    } else {
+        rc = ensure_arena(h, use_cta ? grid * cta_nm : grid);
+    }
     if (rc != PDMPC_OK) return rc;
     if (!use_cta) {   // per-slot scratch for the predecessors' areas
         CU_TRY(h, h->d_depx.reserve((size_t)grid * kDepCols * sizeof(double)));
@@ -1696,7 +1737,10 @@ static int plan_timestep_impl(pdmpc_handle *h, const pdmpc_batch_in *in, const p
     h->batch.hash_valid_only = h->cta_valid_only ? 1 : 0;   // one kind of pop_hash whatever shape runs
     h->stats.shape = use_cta ? (cta_fast ? kShapeCtaValid : kShapeCta) : kShapeLatency;
     CU_TRY(h, cudaEventRecord(h->ev[2], h->stream));
-    if (use_cta && cta_single)
+    if (mcts)
+        mcts_kernel<true><<<grid, kWarp, mcts_smem, h->stream>>>(h->mpa, h->batch, h->out, mc,
+                                                                 h->work_counter.as<unsigned>(), dp);
+    else if (use_cta && cta_single)
         KERNEL_CTA_DEPS<<<grid, CtaShape<1, kCtaCheckers>::kThreads, sizeof(CtaDepsSmemT), h->stream>>>(
             h->mpa, h->batch, h->out, h->arena, h->work_counter.as<unsigned>(), h->cta_heap_smem, cta_fast ? 1 : 0, dp);
     else if (use_cta)
@@ -1754,8 +1798,10 @@ int pdmpc_closed_loop_reset(pdmpc_handle *h, int32_t n_slots, double half_length
     return PDMPC_OK;
 }
 
-int pdmpc_plan_timestep_closed_loop(pdmpc_handle *h, const pdmpc_batch_in *in, const pdmpc_timestep_deps *deps,
-                                    const int32_t *slot, const uint8_t *standstill, pdmpc_batch_out *out) {
+// Both closed-loop entry points; `mcts` as in plan_timestep_impl.
+static int plan_closed_loop(pdmpc_handle *h, const pdmpc_batch_in *in, const pdmpc_timestep_deps *deps,
+                            const int32_t *slot, const uint8_t *standstill, pdmpc_batch_out *out,
+                            const pdmpc_mcts_params *mcts) {
     if (!h) return PDMPC_ERR_BAD_INPUT;
     if (h->cl.n_slots < 1 || h->cl.Hp != h->mpa.Hp)
         return fail(h, PDMPC_ERR_BAD_INPUT, "plan_timestep_closed_loop: call pdmpc_closed_loop_reset first (after pdmpc_upload_mpa)");
@@ -1770,7 +1816,12 @@ int pdmpc_plan_timestep_closed_loop(pdmpc_handle *h, const pdmpc_batch_in *in, c
             seen[slot[i]] = 1;
         }
     }
-    return plan_timestep_impl(h, in, deps, out, slot, standstill);
+    return plan_timestep_impl(h, in, deps, out, slot, standstill, nullptr, nullptr, nullptr, mcts);
+}
+
+int pdmpc_plan_timestep_closed_loop(pdmpc_handle *h, const pdmpc_batch_in *in, const pdmpc_timestep_deps *deps,
+                                    const int32_t *slot, const uint8_t *standstill, pdmpc_batch_out *out) {
+    return plan_closed_loop(h, in, deps, slot, standstill, out, nullptr);
 }
 
 static int run_sample_inputs(pdmpc_handle *h, int n, const int32_t *path_id, const double *x, const double *y,
@@ -1780,8 +1831,9 @@ static int run_assemble_obstacles(pdmpc_handle *h, const pdmpc_coupling_in *in, 
 // One whole time step from the vehicles' measured states: inputs (pdmpc_inputs.cuh), obstacles that do not depend on this
 // step's plans (pdmpc_obstacles.cuh), dependency-ordered searches, fallback plans (pdmpc_fallback.cuh) — nothing of the
 // batch passes through the host.  `ex` != NULL: the rows of pdmpc_plan_timestep_explorative, several per slot; the
-// choice commits one row per slot (plan_timestep_impl).
-static int plan_from_states(pdmpc_handle *h, const pdmpc_timestep_states *st, pdmpc_batch_out *out, const ExplorativeDev *ex) {
+// choice commits one row per slot (plan_timestep_impl).  `mcts` as in plan_timestep_impl.
+static int plan_from_states(pdmpc_handle *h, const pdmpc_timestep_states *st, pdmpc_batch_out *out, const ExplorativeDev *ex,
+                            const pdmpc_mcts_params *mcts = nullptr) {
     if (!h) return PDMPC_ERR_BAD_INPUT;
     if (!h->has_mpa) return fail(h, PDMPC_ERR_NO_MPA, "plan_timestep_from_states: call pdmpc_upload_mpa first");
     if (!h->has_road) return fail(h, PDMPC_ERR_BAD_INPUT, "plan_timestep_from_states: call pdmpc_upload_road first");
@@ -1797,6 +1849,12 @@ static int plan_from_states(pdmpc_handle *h, const pdmpc_timestep_states *st, pd
         return fail(h, PDMPC_ERR_BAD_INPUT, "plan_timestep_from_states: NULL argument");
     if (st->checker != PDMPC_CHECKER_INTERX && st->checker != PDMPC_CHECKER_SAT)
         return fail(h, PDMPC_ERR_BAD_INPUT, "plan_timestep_from_states: unknown checker");
+    if (mcts) {   // before the inputs are sampled on the device
+        MctsDev mc;
+        size_t smem = 0;
+        const int rc = mcts_check(h, mcts, n, &mc, &smem);
+        if (rc != PDMPC_OK) return rc;
+    }
     std::vector<uint8_t> still((size_t)n);
     {
         std::vector<char> seen((size_t)h->cl.n_slots, 0);
@@ -1838,7 +1896,7 @@ static int plan_from_states(pdmpc_handle *h, const pdmpc_timestep_states *st, pd
     pdmpc_timestep_deps deps;
     memset(&deps, 0, sizeof(deps));
     deps.pred_ptr = st->pred_ptr; deps.pred_idx = st->pred_idx;
-    return plan_timestep_impl(h, &stub, &deps, out, st->slot, still.data(), dev, totals, ex);
+    return plan_timestep_impl(h, &stub, &deps, out, st->slot, still.data(), dev, totals, ex, mcts);
 }
 
 int pdmpc_plan_timestep_from_states(pdmpc_handle *h, const pdmpc_timestep_states *st, pdmpc_batch_out *out) {
@@ -1901,35 +1959,25 @@ int pdmpc_joint_plan_batch(pdmpc_handle *h, const pdmpc_batch_in *in, int32_t n_
 int pdmpc_mcts_run_staged(pdmpc_handle *h, const pdmpc_mcts_params *prm) {
     if (!h) return PDMPC_ERR_BAD_INPUT;
     if (!h->staged) return fail(h, PDMPC_ERR_BAD_INPUT, "mcts: no staged batch");
-    if (!prm || prm->n_expansions_max < 1 || prm->n_expansions_max > PDMPC_MCTS_MAX_EXPANSIONS)
-        return fail(h, PDMPC_ERR_BAD_INPUT, "mcts: n_expansions_max out of range");
     const int n = h->batch.n;
-    if (n && !prm->seed) return fail(h, PDMPC_ERR_BAD_INPUT, "mcts: seed is NULL");
-    if (h->max_branch > PDMPC_MCTS_MAX_BRANCH)
-        return fail(h, PDMPC_ERR_BAD_INPUT, "mcts: branching factor of the MPA exceeds PDMPC_MCTS_MAX_BRANCH");
+    MctsDev mc;
+    size_t smem = 0;
+    int rc = mcts_check(h, prm, n, &mc, &smem);
+    if (rc != PDMPC_OK) return rc;
     CU_TRY(h, cudaSetDevice(h->device));
     CU_TRY(h, cudaMemsetAsync(h->out.counters, 0, kCounterBytes, h->stream));
     CU_TRY(h, cudaMemsetAsync(h->work_counter.p, 0, sizeof(unsigned), h->stream));
     h->stats.kernel_launches = 0;
     if (n == 0) return PDMPC_OK;
-    {
-        int rc = upload(h, h->b_seed, prm->seed, (size_t)n);
-        if (rc != PDMPC_OK) return rc;
-        CU_TRY(h, cudaStreamSynchronize(h->stream));   // the seeds are caller-owned
-    }
-    MctsDev mc;
-    mc.n_max = prm->n_expansions_max;
-    mc.node_cap = prm->n_expansions_max + h->mpa.Hp + 1;
+    rc = upload(h, h->b_seed, prm->seed, (size_t)n);
+    if (rc != PDMPC_OK) return rc;
+    CU_TRY(h, cudaStreamSynchronize(h->stream));   // the seeds are caller-owned
     mc.seed = h->b_seed.as<unsigned>();
-    const size_t smem = mcts_smem_bytes(mc.node_cap);
-    if (smem > kSmemLimit) return fail(h, PDMPC_ERR_CAPACITY, "mcts: sampled tree does not fit in shared memory");
-    CU_TRY(h, cudaFuncSetAttribute(mcts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int occ = 0;
-    CU_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, mcts_kernel, kWarp, smem));
-    if (occ < 1) return fail(h, PDMPC_ERR_CUDA, "mcts: kernel is not launchable on this device");
-    const int grid = std::min(n, h->num_sms * occ);
+    int grid = 0;
+    rc = mcts_grid<false>(h, smem, n, &grid);
+    if (rc != PDMPC_OK) return rc;
     CU_TRY(h, cudaEventRecord(h->ev[2], h->stream));
-    mcts_kernel<<<grid, kWarp, smem, h->stream>>>(h->mpa, h->batch, h->out, mc, h->work_counter.as<unsigned>());
+    mcts_kernel<false><<<grid, kWarp, smem, h->stream>>>(h->mpa, h->batch, h->out, mc, h->work_counter.as<unsigned>());
     CU_TRY(h, cudaGetLastError());
     CU_TRY(h, cudaEventRecord(h->ev[3], h->stream));
     h->timing_pending_kernel = true;
@@ -1944,6 +1992,29 @@ int pdmpc_mcts_plan_batch(pdmpc_handle *h, const pdmpc_batch_in *in, const pdmpc
     rc = pdmpc_mcts_run_staged(h, prm);
     if (rc != PDMPC_OK) return rc;
     return pdmpc_fetch_staged(h, out);
+}
+
+// The sampled optimizer's time steps: the graph search's time-step paths with mcts_kernel<true> as the search.
+int pdmpc_mcts_plan_timestep(pdmpc_handle *h, const pdmpc_batch_in *in, const pdmpc_timestep_deps *deps,
+                             const pdmpc_mcts_params *prm, pdmpc_batch_out *out) {
+    if (!h) return PDMPC_ERR_BAD_INPUT;
+    if (!prm) return fail(h, PDMPC_ERR_BAD_INPUT, "mcts: params are NULL");
+    return plan_timestep_impl(h, in, deps, out, nullptr, nullptr, nullptr, nullptr, nullptr, prm);
+}
+
+int pdmpc_mcts_plan_timestep_closed_loop(pdmpc_handle *h, const pdmpc_batch_in *in, const pdmpc_timestep_deps *deps,
+                                         const int32_t *slot, const uint8_t *standstill, const pdmpc_mcts_params *prm,
+                                         pdmpc_batch_out *out) {
+    if (!h) return PDMPC_ERR_BAD_INPUT;
+    if (!prm) return fail(h, PDMPC_ERR_BAD_INPUT, "mcts: params are NULL");
+    return plan_closed_loop(h, in, deps, slot, standstill, out, prm);
+}
+
+int pdmpc_mcts_plan_timestep_from_states(pdmpc_handle *h, const pdmpc_timestep_states *st, const pdmpc_mcts_params *prm,
+                                         pdmpc_batch_out *out) {
+    if (!h) return PDMPC_ERR_BAD_INPUT;
+    if (!prm) return fail(h, PDMPC_ERR_BAD_INPUT, "mcts: params are NULL");
+    return plan_from_states(h, st, out, nullptr, prm);
 }
 
 int pdmpc_trace_staged(pdmpc_handle *h, int32_t search, int64_t *ids, int64_t cap, int64_t *n_out) {

@@ -82,8 +82,13 @@ __device__ __forceinline__ void mt_twist(unsigned *mt, int lane) {
 }
 
 // The sampled search.  Persistent one-warp CTAs pulling searches from a global counter.
+// DEPS (pdmpc_mcts_plan_timestep): as search_kernel<..., true> — a search waits for its predecessors' done flags,
+// copies their planned (or fallback) areas into its CTA's scratch in HBM, checks every expansion against the step-k
+// ones and releases its own flag once its areas are written.  Searches are taken in the topological work order and
+// every CTA of the grid is resident, so a warp only waits for searches that resident warps have already taken.
+template <bool DEPS = false>
 __global__ void __launch_bounds__(kWarp) mcts_kernel(MpaDev m, BatchDev b, OutDev o, MctsDev mc,
-                                                     unsigned *work_counter) {
+                                                     unsigned *work_counter, DepsDev dp = DepsDev{}) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x;
     const int nc = mc.node_cap + 1;
@@ -117,6 +122,14 @@ __global__ void __launch_bounds__(kWarp) mcts_kernel(MpaDev m, BatchDev b, OutDe
     t.shift = 0; t.lane = lane; t.mask = 0xffffffffu;
     const int Hp = m.Hp, nT = m.nT;
     const int n_rand = Hp * mc.n_max;
+    // DEPS: this CTA's scratch for the predecessors' areas; lane k - 1 keeps the real column count of step k
+    int n_pred = 0, my_dep_cols = 0;
+    double *dpx = nullptr, *dpy = nullptr;
+    int *dpn = nullptr;
+    if (DEPS) {
+        const size_t sl = blockIdx.x;
+        dpx = dp.dep_x + sl * kDepCols; dpy = dp.dep_y + sl * kDepCols; dpn = dp.dep_n + sl * (kDepCols / kAreaStride);
+    }
 
     for (;;) {
         unsigned si_u = 0;
@@ -125,6 +138,19 @@ __global__ void __launch_bounds__(kWarp) mcts_kernel(MpaDev m, BatchDev b, OutDe
         if (si_u >= (unsigned)b.n) break;
         const int si = b.order ? __ldg(b.order + si_u) : (int)si_u;
         __syncwarp();
+        if (DEPS) {   // consider_predecessors, PrioritizedController.m:449-506
+            n_pred = gather_predecessor_areas(
+                dp, o, si, Hp, 200, t, [=](int idx, double x, double y) { dpx[idx] = x; dpy[idx] = y; },
+                [=](int pk, int, int np) { dpn[pk] = np; });
+            __threadfence_block();
+            __syncwarp();
+            my_dep_cols = 0;
+            if (lane < Hp)
+                for (int r = 0; r < n_pred; ++r) {
+                    const int np = dpn[lane * n_pred + r];
+                    if (np) my_dep_cols += np + 1;
+                }
+        }
 
         // ---- per-search set-up (as in search_kernel) -------------------------------
         for (int k = lane; k < Hp; k += kWarp) {
@@ -262,7 +288,12 @@ __global__ void __launch_bounds__(kWarp) mcts_kernel(MpaDev m, BatchDev b, OutDe
                     const int st_lo = obase + rng[0], st_hi = obase + rng[1];
                     const int dy_lo = obase + rng[step], dy_hi = obase + rng[step + 1];
                     cols += (unsigned long long)((st_hi - st_lo) + (dy_hi - dy_lo) + (lhi - llo));
+                    if (DEPS) cols += (unsigned long long)__shfl_sync(0xffffffffu, my_dep_cols, step - 1);
                     if (interx_dispatch<kWarp>(ns, opx, opy, st_lo, st_hi, dy_lo, dy_hi, shx, shy, t))
+                        valid = false;
+                    else if (DEPS && n_pred > 0 &&
+                             interx_dispatch<kWarp>(ns, dpx, dpy, (step - 1) * n_pred * kAreaStride,
+                                                    step * n_pred * kAreaStride, 0, 0, shx, shy, t))
                         valid = false;
                     else if (interx_dispatch<kWarp>(nbs, lpx, lpy, llo, lhi, 0, 0, bhx, bhy, t))
                         valid = false;
@@ -274,6 +305,15 @@ __global__ void __launch_bounds__(kWarp) mcts_kernel(MpaDev m, BatchDev b, OutDe
                             const int v0 = __ldg(b.poly_ptr + p), v1 = __ldg(b.poly_ptr + p + 1);
                             cols += (unsigned long long)(v1 - v0);
                             if (sat_collide<kWarp>(shx, shy, ns, b.vert_x + v0, b.vert_y + v0, v1 - v0, t))
+                                valid = false;
+                        }
+                    }
+                    if (DEPS) {
+                        for (int r = 0; r < n_pred && valid; ++r) {
+                            const int pk = (step - 1) * n_pred + r, nv = dpn[pk];
+                            if (nv < 2) continue;
+                            cols += (unsigned long long)nv;
+                            if (sat_collide<kWarp, false>(shx, shy, ns, dpx + pk * kAreaStride, dpy + pk * kAreaStride, nv, t))
                                 valid = false;
                         }
                     }
@@ -381,6 +421,11 @@ __global__ void __launch_bounds__(kWarp) mcts_kernel(MpaDev m, BatchDev b, OutDe
                     }
                 }
             }
+        }
+        if (DEPS) {   // publish_predictions, PrioritizedController.m:355-364: the areas above are final
+            __threadfence();
+            __syncwarp();
+            if (lane == 0) st_release_gpu(dp.done + si, exhausted ? 2 : 1);
         }
         __syncwarp();
     }

@@ -24,6 +24,10 @@
 //       PrioritizedSequentialController.controller (PrioritizedSequentialController.m:74-92); vehicle i
 //       waits on the device for the vehicles j with directed_coupling_sequential(j, i) ~= 0 and takes
 //       their planned areas as dynamic obstacles (PrioritizedController.m:449-506); empty cells are skipped.
+//   [same outputs] = mex(PLAN_TIMESTEP_SAMPLED, h, <the thirteen PLAN_TIMESTEP arguments>, seeds [N], n_expansions_max)
+//       the same time step with MonteCarloTreeSearch as the optimizer (plan_timestep_cuda.m with a
+//       MonteCarloTreeSearchCuda optimizer): seeds(i) = time_step + vehicle_index of vehicle i (MonteCarloTreeSearch.m:31).
+//       A search whose roll-outs run out of random numbers is reported exhausted, like one without a valid leaf.
 //   [is_exhausted, n_expanded, trims (nV x Hp+1), y_pred (3 x Hp*nV), shapes {nV x Hp}, g_path (1 x Hp+1), h_path] =
 //       mex(PLAN_JOINT, h, x0 [nV x 3], trims [nV x 1], ref [nV x Hp x 2], v_ref [nV x Hp], obstacles {nV x S},
 //           dynamic_obstacle_area {nV x R*Hp}, left {nV x 1}, right {nV x 1}, checker (0 = SAT), dt)
@@ -61,7 +65,7 @@
 namespace {
 
 enum Command { CREATE = 0, DESTROY = 1, UPLOAD_MPA = 2, PLAN = 3, STATS = 4, PLAN_SAMPLED = 5, PLAN_TIMESTEP = 6, PLAN_JOINT = 7, UPLOAD_ROAD = 8,
-               SAMPLE_INPUTS = 9, UPLOAD_REACHABLE_SETS = 10, ASSEMBLE_OBSTACLES = 11, COUPLE = 12 };
+               SAMPLE_INPUTS = 9, UPLOAD_REACHABLE_SETS = 10, ASSEMBLE_OBSTACLES = 11, COUPLE = 12, PLAN_TIMESTEP_SAMPLED = 13 };
 
 std::vector<pdmpc_handle *> g_handles;   // released at `clear mex` (HighLevelController.m:284-303)
 bool g_at_exit_registered = false;
@@ -287,8 +291,9 @@ void plan(pdmpc_handle *h, int nlhs, mxArray *plhs[], const mxArray *prhs[], boo
 }
 
 // PLAN_TIMESTEP: N vehicles, one pdmpc_plan_timestep call.  PLAN_JOINT (joint == true): the same N rows as ONE
-// centralized search (pdmpc_joint_plan_batch), no coupling / fallback arguments.
-void plan_timestep(pdmpc_handle *h, int nlhs, mxArray *plhs[], const mxArray *prhs[], bool joint) {
+// centralized search (pdmpc_joint_plan_batch), no coupling / fallback arguments.  PLAN_TIMESTEP_SAMPLED (sampled == true):
+// pdmpc_mcts_plan_timestep with seeds and n_expansions_max after the PLAN_TIMESTEP arguments.
+void plan_timestep(pdmpc_handle *h, int nlhs, mxArray *plhs[], const mxArray *prhs[], bool joint, bool sampled = false) {
     const mxArray *x0 = prhs[2], *trim = prhs[3], *ref = prhs[4], *vref = prhs[5], *obst = prhs[6], *dyn = prhs[7];
     const mxArray *left = prhs[8], *right = prhs[9], *coupling = joint ? nullptr : prhs[12];
     const mxArray *fallback = joint ? nullptr : prhs[13];
@@ -390,9 +395,29 @@ void plan_timestep(pdmpc_handle *h, int nlhs, mxArray *plhs[], const mxArray *pr
     out.trims = out_trims.data(); out.y_predicted = ypred.data();
     out.g_path = g.data(); out.h_path = hh.data();
     out.shape_npts = shape_npts.data(); out.shape_x = sx.data(); out.shape_y = sy.data();
-    if (joint) check(h, pdmpc_joint_plan_batch(h, &in, static_cast<int32_t>(N), &out), "pdmpc_joint_plan_batch");
-    else check(h, pdmpc_plan_timestep(h, &in, &deps, &out), "pdmpc_plan_timestep");
-    for (size_t i = 0; i < N; ++i)
+    if (joint) {
+        check(h, pdmpc_joint_plan_batch(h, &in, static_cast<int32_t>(N), &out), "pdmpc_joint_plan_batch");
+    } else if (sampled) {
+        // mxGetDoubles is NULL for any class but double (e.g. uint32(time_step + (1:N)))
+        const double *ps = mxGetDoubles(prhs[14]);
+        if (!ps || mxGetNumberOfElements(prhs[14]) != N)
+            fail("pdmpc:input", "seeds must be N doubles (time_step + vehicle_index)");
+        if (mxGetNumberOfElements(prhs[15]) != 1) fail("pdmpc:input", "n_expansions_max must be a scalar");
+        std::vector<uint32_t> seeds(N);
+        for (size_t i = 0; i < N; ++i) {
+            const double v = ps[i];
+            if (!(v >= 0.0 && v <= 4294967295.0) || v != static_cast<double>(static_cast<uint32_t>(v)))
+                fail("pdmpc:input", "seeds must be integers in 0 .. 2^32 - 1");
+            seeds[i] = static_cast<uint32_t>(v);
+        }
+        pdmpc_mcts_params prm;
+        prm.n_expansions_max = static_cast<int32_t>(mxGetScalar(prhs[15]));
+        prm.seed = seeds.data();
+        check(h, pdmpc_mcts_plan_timestep(h, &in, &deps, &prm, &out), "pdmpc_mcts_plan_timestep");
+    } else {
+        check(h, pdmpc_plan_timestep(h, &in, &deps, &out), "pdmpc_plan_timestep");
+    }
+    for (size_t i = 0; i < N && !sampled; ++i)   // a sampled search out of random numbers is an exhausted row
         if (status[i] != PDMPC_OK) fail("pdmpc:search", "search " + std::to_string(i + 1) + " failed with status " + std::to_string(status[i]));
 
     plhs[0] = mxCreateDoubleMatrix(1, N, mxREAL);
@@ -703,6 +728,10 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
     case PLAN_TIMESTEP:
         if (nrhs < 14) fail("pdmpc:usage", "PLAN_TIMESTEP needs 14 arguments");
         plan_timestep(h, nlhs, plhs, prhs, false);
+        return;
+    case PLAN_TIMESTEP_SAMPLED:
+        if (nrhs < 16) fail("pdmpc:usage", "PLAN_TIMESTEP_SAMPLED needs 16 arguments");
+        plan_timestep(h, nlhs, plhs, prhs, false, true);
         return;
     case PLAN_JOINT:
         if (nrhs < 12) fail("pdmpc:usage", "PLAN_JOINT needs 12 arguments");

@@ -1,4 +1,4 @@
-function infos = plan_timestep_cuda(handle, hlcs, mpa, options)
+function infos = plan_timestep_cuda(handle, hlcs, mpa, options, time_step)
 % PLAN_TIMESTEP_CUDA  All vehicles of one time step in ONE optimizer call on the GPU.
 %
 %   Replaces the level loop of PrioritizedSequentialController.controller
@@ -17,11 +17,19 @@ function infos = plan_timestep_cuda(handle, hlcs, mpa, options)
 %   infos  : 1 x N ControlResultsInfo, built by the reference's own helper
 %            OptimizerInterface.create_control_results_info_from_mex (OptimizerInterface.m:63-101)
 %
+%   time_step : the time step PrioritizedController.plan passes to run_optimizer (:335-341); needed when
+%            hlcs(1).optimizer is a MonteCarloTreeSearchCuda
+%
 %   Vehicles planning in PARALLEL to vehicle i (other groups) and its successors enter exactly as in
 %   the reference: their reachable sets / previous trajectories / standstill areas are known
 %   before the time step and are put into iter_v by the unchanged MATLAB code below.
+%
+%   With a MonteCarloTreeSearchCuda optimizer the searches are MonteCarloTreeSearch.run_optimizer's
+%   (MEX command PLAN_TIMESTEP_SAMPLED): vehicle i's random stream has Seed = time_step + i
+%   (MonteCarloTreeSearch.m:31), and its info is rebuilt as MonteCarloTreeSearchCuda.run_optimizer does.
 
     PLAN_TIMESTEP = 6;
+    PLAN_TIMESTEP_SAMPLED = 13;
     N = numel(hlcs);
     Hp = options.Hp;
     x0 = zeros(N, 3); trims = zeros(N, 1); ref = zeros(N, Hp, 2); v_ref = zeros(N, Hp);
@@ -61,8 +69,15 @@ function infos = plan_timestep_cuda(handle, hlcs, mpa, options)
         end
     end
 
-    [is_exhausted, n_expanded, trims_out, y, shapes, g, h] = pdmpc_b200_mex(PLAN_TIMESTEP, handle, x0, trims, ref, v_ref, ...
-        obstacles, reshape(dyn, N, []), left, right, checker, options.dt_seconds, double(coupling), fallback_shapes);
+    args = {handle, x0, trims, ref, v_ref, obstacles, reshape(dyn, N, []), left, right, checker, options.dt_seconds, ...
+        double(coupling), fallback_shapes};
+    sampled = isa(hlcs(1).optimizer, 'MonteCarloTreeSearchCuda');
+    if sampled
+        [is_exhausted, n_expanded, trims_out, y, shapes, g, h] = pdmpc_b200_mex(PLAN_TIMESTEP_SAMPLED, args{:}, ...
+            time_step + (1:N), hlcs(1).optimizer.n_expansions_max);
+    else
+        [is_exhausted, n_expanded, trims_out, y, shapes, g, h] = pdmpc_b200_mex(PLAN_TIMESTEP, args{:});
+    end
     y = reshape(y, 3, Hp, N);
 
     infos = cell(1, N);
@@ -70,7 +85,25 @@ function infos = plan_timestep_cuda(handle, hlcs, mpa, options)
         info = ControlResultsInfo(1, Hp);
         info.is_exhausted = logical(is_exhausted(i));
         info.n_expanded = n_expanded(i);
-        if ~info.is_exhausted
+        if sampled && ~info.is_exhausted
+            % path-only tree, as MonteCarloTreeSearchCuda.run_optimizer builds it (MonteCarloTreeSearch.m:207-239):
+            % g = -1 except the goal leaf, h = -1
+            tree = Tree();
+            tree.trim = trims_out(i, :);
+            tree.parent = uint32(0:Hp);
+            tree.x = [x0(i, 1), y(1, :, i)];
+            tree.y = [x0(i, 2), y(2, :, i)];
+            tree.yaw = [x0(i, 3), y(3, :, i)];
+            tree.k = 1:(Hp + 1);
+            tree.g = [-1 * ones(1, Hp), g(i, end)];
+            tree.h = -1 * ones(1, Hp + 1);
+            info.tree = tree;
+            info.tree_path = 1:(Hp + 1);
+            info.y_predicted = y(:, :, i);
+            info.shapes = shapes(i, :);
+            info.predicted_trims = trims_out(i, 2:end);
+            info.needs_fallback = false;
+        elseif ~info.is_exhausted
             % next_nodes: Hp cells of 1 x 8 rows in NodeInfo order [x y yaw trim g h k exactEval]
             % (g, h: tree.get_cost(tree_path(end)) is what the explorative / optimal controllers compare,
             %  PrioritizedExplorativeController.m:100-104)

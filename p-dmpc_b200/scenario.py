@@ -755,7 +755,7 @@ class ScenarioRunner:
 
     def __init__(self, sc: Scenario, plan_fn: PlanFn, max_num_CLs: int = 99, timestep_fn=None, inputs_fn=None,
                  path_id0: int = 0, closed_loop_fn=None, obstacles_fn=None, states_fn=None, coupler: str = "corridor",
-                 coupled_fn=None):
+                 coupled_fn=None, n_expansions_max: Optional[int] = None):
         """plan_fn(batch) plans one computation level; with timestep_fn(batch, deps) the whole time
         step is ONE call and the predecessors' areas are handed over behind it (pdmpc_plan_timestep).
         inputs_fn(path_id, x, y, speed, dt) -> dict (capi.Planner.sample_inputs): reference trajectories and lanelet
@@ -787,6 +787,10 @@ class ScenarioRunner:
         # closed_loop_fn(batch, deps, slot, standstill) -> BatchResult with the FINAL plan of every vehicle
         # (capi.Planner.plan_timestep_closed_loop): fallback plans are built and kept on the device, slot = path_id0 + i
         self.closed_loop_fn = closed_loop_fn
+        # n_expansions_max: the optimizer is MonteCarloTreeSearch with this budget (the callbacks pass it on); plan_fn,
+        # timestep_fn, closed_loop_fn and states_fn then also receive the RandStream seeds of the rows they plan as their
+        # last argument: time_step + vehicle_index, both 1-based (MonteCarloTreeSearch.m:31, PrioritizedController.m:335-341)
+        self.n_expansions_max = n_expansions_max
         self.max_num_CLs = max_num_CLs              # honoured by the one-call path (timestep_inputs)
         self.timestep_records: List[tuple] = []     # (step, batch, deps, result) of the one-call path
         self.mpa = sc.mpa
@@ -799,6 +803,13 @@ class ScenarioRunner:
         self.k = 0
         self.records: List[StepRecord] = []
         self.n_fallbacks = 0
+
+    def _seeded(self, fn, *args, rows=None):
+        """fn(*args), or fn(*args, seeds of `rows` (default: all vehicles)) for the sampled optimizer."""
+        if self.n_expansions_max is None:
+            return fn(*args)
+        seeds = mcts_seeds(self.k, self.sc.amount)
+        return fn(*args, seeds if rows is None else seeds[rows])
 
     def _adjacency(self) -> np.ndarray:
         if self.coupler == "reachable_set":
@@ -908,11 +919,11 @@ class ScenarioRunner:
             seq = limit_computation_levels(D, self.max_num_CLs) if self.max_num_CLs < n else D
             speed = np.array([mpa.trim_speed[self.trim[i] - 1] for i in range(n)], dtype=np.float64)
             ids = self.path_id0 + np.arange(n)
-            res = self.states_fn(ids, self.pose[:, 0], self.pose[:, 1], self.pose[:, 2], speed, self.trim,
-                                 [np.flatnonzero(D[i, :]) for i in range(n)],
-                                 [np.flatnonzero(D[:, i] & ~seq[:, i]) for i in range(n)],
-                                 [np.flatnonzero(seq[:, i]) for i in range(n)], ids,
-                                 VEH_LENGTH / 2 + 0.01, VEH_WIDTH / 2 + 0.01, mpa.dt_seconds, sc.checker)
+            res = self._seeded(self.states_fn, ids, self.pose[:, 0], self.pose[:, 1], self.pose[:, 2], speed, self.trim,
+                               [np.flatnonzero(D[i, :]) for i in range(n)],
+                               [np.flatnonzero(D[:, i] & ~seq[:, i]) for i in range(n)],
+                               [np.flatnonzero(seq[:, i]) for i in range(n)], ids,
+                               VEH_LENGTH / 2 + 0.01, VEH_WIDTH / 2 + 0.01, mpa.dt_seconds, sc.checker)
             self.apply_final(res)
             self.timestep_records.append((self.k, None, None, res))
             return res
@@ -921,11 +932,11 @@ class ScenarioRunner:
         if self.closed_loop_fn is not None:
             deps = TimestepDeps.build(preds, [None] * n, Hp)
             still = np.array([abs(mpa.trim_speed[self.trim[i] - 1]) < 0.01 for i in range(n)], dtype=np.uint8)
-            res = self.closed_loop_fn(batch, deps, self.path_id0 + np.arange(n), still)
+            res = self._seeded(self.closed_loop_fn, batch, deps, self.path_id0 + np.arange(n), still)
             self.apply_final(res)
         else:
             deps = TimestepDeps.build(preds, [f[0] for f in fallbacks], Hp)
-            res = self.timestep_fn(batch, deps)
+            res = self._seeded(self.timestep_fn, batch, deps)
             self.apply_timestep(res, fallbacks)
         self.timestep_records.append((self.k, batch, deps, res))
         return res
@@ -992,7 +1003,7 @@ class ScenarioRunner:
                         it.obstacles.append(occupied_area(*self.pose[j]))
                 its.append(it)
             batch = SearchBatch.from_iters(its, Hp, sc.checker, mpa.dt_seconds)
-            res = self.plan_fn(batch)
+            res = self._seeded(self.plan_fn, batch, rows=members)
             for b, i in enumerate(members):
                 if not res.is_exhausted[b]:
                     shapes_now[i] = res.shapes(b)
@@ -1362,12 +1373,19 @@ def _assign_rows(dst: BatchResult, rows, src: BatchResult) -> None:
             a[rows] = getattr(src, f.name)
 
 
-def plan_timestep_by_levels(plan_fn: PlanFn, batch: SearchBatch, deps: TimestepDeps) -> BatchResult:
+def mcts_seeds(time_step: int, n: int) -> np.ndarray:
+    """RandStream seeds of vehicles 1..n at time step `time_step` (1-based): time_step + vehicle_index
+    (MonteCarloTreeSearch.m:31 with the arguments PrioritizedController.plan passes, :335-341)."""
+    return (int(time_step) + np.arange(1, n + 1)).astype(np.uint32)
+
+
+def plan_timestep_by_levels(plan_fn: PlanFn, batch: SearchBatch, deps: TimestepDeps, seeds=None) -> BatchResult:
     """The reference's way through one time step, as the specification of pdmpc_plan_timestep:
     computation levels one after the other (utility/kahn.m, PrioritizedSequentialController.m:83-92),
     each vehicle's iter_v extended on the HOST by the areas its sequential predecessors published
     (PrioritizedController.m:297-324, consider_predecessors :449-506), an exhausted predecessor
-    publishing its fallback areas (:568-621, :678-718)."""
+    publishing its fallback areas (:568-621, :678-718).  With `seeds` (the sampled optimizer, the specification of
+    pdmpc_mcts_plan_timestep) a level is planned as plan_fn(sub_batch, seeds[members])."""
     iters, Hp, checker, dt_seconds = batch.to_iters(), batch.Hp, batch.checker, batch.dt_seconds
     n = len(iters)
     level = np.zeros(n, dtype=np.int64)
@@ -1394,7 +1412,8 @@ def plan_timestep_by_levels(plan_fn: PlanFn, batch: SearchBatch, deps: TimestepD
                     continue   # nothing published (no fallback areas given)
                 it.dynamic_obstacle_area.append(published[j])
             its.append(it)
-        res = plan_fn(SearchBatch.from_iters(its, Hp, checker, dt_seconds))
+        sub = SearchBatch.from_iters(its, Hp, checker, dt_seconds)
+        res = plan_fn(sub) if seeds is None else plan_fn(sub, np.asarray(seeds)[members])
         _assign_rows(out, members, res)
         for b, i in enumerate(members):
             published[i] = deps.fallback_shapes(i) if res.is_exhausted[b] else res.shapes(b)
